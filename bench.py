@@ -2,6 +2,7 @@
 """bench.py -- streamline-steps/sec of the batched tracking step on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision fp16|tf32|bf16]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on): whole-brain synthetic
 145x174x145 1.25 mm order-8 descoteaux07 fODF, npv 20 on the mask shell (873 000 seeds per GPU),
@@ -27,6 +28,16 @@ What the JSON line carries (DESIGN.md section 6 says how every field is produced
   cpu_baseline the CPU restatement of the reference path on the host cores, same 50 000-row batch
 `--impl reference` times that CPU restatement (oracle/ttl_oracle.py + a torch-CPU fp32 actor) alone, under
 the better of OMP_NUM_THREADS in {1, cores}.
+
+`--dump-outputs DIR` writes, on rank 0, what the headline tier's timed steps left a caller after the last
+of them, as DIR/<name>.npy (float32 / float64, integers stored exactly as float64, under 64 MB in all):
+  lengths, flags        [N]                 every row (seed) of the batch
+  points, points_rows   [4096, max_pts, 3]  the streamline buffer of a fixed, seeded sample of rows
+  alive_rows            [n_alive]           the rows still tracked, ascending
+  state, state_rows     [8192, 615]         the actor's next input for a fixed, seeded sample of those rows,
+                                            in the state's column order, at the operand precision
+The inputs (volume, seeds, actor) are seeded, so two builds run with the same arguments can be compared
+array for array.
 """
 import argparse
 import json
@@ -71,6 +82,9 @@ TIER_NOTE = {
     'bf16': 'bf16 operands (8 significant bits): ~4e-3 of the output scale, OUTSIDE the 1e-3 tolerance',
 }
 NCU_SUMMARY = os.path.join(ROOT, 'profiles', 'r2_final_step_ncu_summary.json')
+DUMP_POINTS_ROWS = 4096
+DUMP_STATE_ROWS = 8192
+DUMP_MAX_BYTES = 64 << 20
 
 
 def workload_config(shape=SHAPE, voxel_mm=VOXEL_MM):
@@ -431,6 +445,46 @@ def make_env(shape, voxel_mm, dev):
     return env, sub
 
 
+def state_columns(env):
+    """Column of each state feature in the actor's operand rows: layout 1 pads every neighbourhood point's C
+    coefficients to CP columns (include/ttl_b200.h, ttl_batch.bf16_layout)."""
+    layout, C, CP, n_points = env.bf16_layout
+    S = env._batch.state_size
+    if layout == 0:
+        return np.arange(S)
+    return np.concatenate([p * CP + np.arange(C) for p in range(n_points)] + [n_points * CP + np.arange(S - n_points * C)])
+
+
+def capture_outputs(env, n_alive):
+    """Host copies of what the step path left a caller after its last step (see --dump-outputs)."""
+    import torch
+    bb = env._batch
+    n = env._n
+    rs = np.random.RandomState(2024)
+    pts_rows = np.sort(rs.choice(n, min(n, DUMP_POINTS_ROWS), replace=False))
+    alive = bb.alive[env._cur][:n_alive].long()
+    alive_sorted, ranks = torch.sort(alive)
+    pick = torch.from_numpy(np.sort(rs.choice(n_alive, min(n_alive, DUMP_STATE_ROWS), replace=False))).to(env.device)
+    st = env.current_state()
+    if st is None:        # operand-only rows: back to the state's column order
+        st = env.current_state_bf16()[:, torch.from_numpy(state_columns(env)).to(env.device)]
+    out = {'lengths': bb.lengths[:n].double(), 'flags': bb.flags[:n].double(),
+           'points': bb.points[torch.from_numpy(pts_rows).to(env.device)].float(),
+           'points_rows': torch.from_numpy(pts_rows).double(), 'alive_rows': alive_sorted.double(),
+           'state': st[ranks[pick]].float(), 'state_rows': alive_sorted[pick].double()}
+    return {k: v.cpu().numpy() for k, v in out.items()}
+
+
+def write_outputs(d, outputs):
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError('--dump-outputs: %d bytes exceeds the %d byte limit' % (total, DUMP_MAX_BYTES))
+    os.makedirs(d, exist_ok=True)
+    for name, a in outputs.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(d, name + '.npy'), a)
+
+
 def roofline_of(prec, prof, rows, pk, tf32_peak, traffic):
     """The tcgen05 launch(es) of one step against the burst peak of the operand type.  The per-launch
     time comes from CUDA events bracketing every launch of the library (ttl_prof_enable) in a separate
@@ -527,6 +581,7 @@ def run_tier(env, actor_sd, prec, args, dev, lib, barrier, sampler=None, is_main
     env.n_alive()
     units = env.streamline_steps() - steps_before
     alive_end = int(env._batch.ctrl_host[env._cur])
+    outputs = capture_outputs(env, alive_end) if args.dump_outputs and is_main else None
     # per-kernel device times (CUDA events on the launching stream), separate segment
     prof_steps = min(20, args.steps)
     lib.ttl_prof_enable(1)
@@ -564,7 +619,7 @@ def run_tier(env, actor_sd, prec, args, dev, lib, barrier, sampler=None, is_main
     sm_mhz = sampler.median_between(t_begin, t_end) if sampler is not None else None
     return alg, {'elapsed_ms': elapsed_ms, 'units': units, 'gpu_launches': gpu_launches, 'alive_end': alive_end,
                  'prof': prof, 'saturated': saturated, 'sm_mhz': sm_mhz,
-                 'sustained_ms': sustained_ms, 'sustained_units': sustained_units}
+                 'sustained_ms': sustained_ms, 'sustained_units': sustained_units, 'outputs': outputs}
 
 
 def run_e2e(env, alg, dev, world, barrier):
@@ -864,6 +919,8 @@ def main_gpu(args):
             'cpu_baseline': cpu_baseline,
             'flop_per_streamline_step': ACTOR_FLOP_PER_ROW,
         }
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, mr['outputs'])
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -885,11 +942,17 @@ if __name__ == '__main__':
     ap.add_argument('--graph', action='store_true', help='replay the kernels of a step from a CUDA graph')
     ap.add_argument('--no-e2e', action='store_true', help='skip the end-to-end leg (profiling runs)')
     ap.add_argument('--no-sharded', action='store_true', help='skip the configs[2] sharded leg')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the headline tier's outputs after its last timed step as DIR/<name>.npy")
     ap.add_argument('--cpu-worker', default=None, help=argparse.SUPPRESS)
     ap.add_argument('--torch-threads', type=int, default=os.cpu_count() or 1, help=argparse.SUPPRESS)
     a = ap.parse_args()
     if a.cpu_worker:
         sys.exit(cpu_worker(a))
+    if a.dump_outputs and a.impl == 'reference':
+        ap.error('--dump-outputs dumps the GPU step path; the reference arm has no such output')
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.warmup < 3:
         a.warmup = 3
     sys.exit(main_reference(a) if a.impl == 'reference' else main_gpu(a))
