@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """ttl_track on N GPUs of one box writes the same tractogram as on one GPU.
 
-    python benchmarks/multi_gpu_cli_check.py [N]      # needs N visible GPUs (default 2)
+    python benchmarks/multi_gpu_cli_check.py [N [ttl_track options...]]   # needs N visible GPUs (default 2)
+
+e.g. ``2 --noise 0.1 --noise_rng device`` checks noisy tracking with device-drawn noise.
 
 Builds a small synthetic subject on disk, runs the CLI in this process (1 GPU), runs it again under
 ``torch.distributed.run --nproc-per-node N`` (seeds sharded, NCCL gather to rank 0) and compares the
@@ -39,7 +41,7 @@ def main():
         common = [p('fodf.nii.gz'), p('seed.nii.gz'), p('mask.nii.gz')]
         opts = ['--agent', agent, '--hyperparameters', os.path.join(agent, 'hyperparameters.json'),
                 '--n_actor', '3000', '--npv', '3', '--min_length', '5', '--max_length', '80', '--save_seeds',
-                '--compress', '0.05', '-f']
+                '--compress', '0.05', '-f'] + sys.argv[2:]
         one = p('one.' + ext)
         cli(common + [one] + opts)
         many = p('many.' + ext)
@@ -51,7 +53,7 @@ def main():
         same = bool(np.array_equal(o1, o2) and np.array_equal(d1, d2))
         out[ext] = {'streamlines': int(len(o1) - 1), 'points': int(len(d1)), 'identical': same}
         assert same, ext
-    print(json.dumps({'gpus': n, 'result': out}))
+    print(json.dumps({'gpus': n, 'options': sys.argv[2:], 'result': out}))
 
 
 if __name__ == '__main__':

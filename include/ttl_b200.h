@@ -183,8 +183,9 @@ int ttl_env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* 
  * partial sums of the 6-wide output layer (tiles_per_256 = 256 / tile width of the launch that wrote
  * them), head_bias [6].  The sums follow the same fixed tree as the actor's own finishing pass, so this
  * entry point and ttl_actor_forward* + ttl_env_step give the same bits whatever the tile width; it
- * saves one launch and the action round trip per step.  No noise input: the noisy
- * environment with sigma > 0 goes through ttl_env_step. */
+ * saves one launch and the action round trip per step.  No noise array: the noisy
+ * environment with host-drawn noise (sigma > 0) goes through ttl_env_step; device-drawn noise
+ * through ttl_env_step_head_rng below. */
 int ttl_env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
                       const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
                       const float* head_bias, int32_t n_upper, void* stream);
@@ -203,6 +204,39 @@ int ttl_env_step_begin(const ttl_volume* vol, const ttl_params* prm, const ttl_b
 int ttl_env_step_finish(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
                         const float* scores, int32_t use_stop, int32_t min_pts_stop, int32_t min_pts_reward,
                         float bonus, int32_t n_upper, void* stream);
+
+/* Tracking noise drawn inside the step kernel (NoisyTrackingEnvironment with noise_rng = 'device').
+ * Row i of the batch, with g = row_base + i and L = its point count before the step (1 on the first
+ * step), gets noise_c = sigma * z_c for c = 0, 1, 2, where
+ *   (w0, w1, w2, w3) = Philox4x32-10(counter = (lo32(g), hi32(g), L, c), key = (lo32(seed), hi32(seed)))
+ *   u1 = (((w1 << 32 | w0) >> 12) + 0.5) * 2^-52,  u2 = (((w3 << 32 | w2) >> 12) + 0.5) * 2^-52
+ *   z_c = sqrt(-2 ln u1) * cos(2 pi u2)            (fp64; |z_c| <= 8.58)
+ * added in fp64 to the action where ttl_env_step adds its `noise` array.  Each streamline's noise
+ * depends only on (seed, g, L, c): not on the alive-list order, the slot count, refill, the tip sort or
+ * the process that tracks it, so a run sharded over GPUs (row_base = the shard's first index in the
+ * common seed list) produces what one GPU produces.  It is not the reference's RandomState stream.
+ * The struct is a host structure read at call time (like ttl_params); a CUDA graph captures its values. */
+typedef struct ttl_noise {
+  double sigma;            /* N(0, sigma) per component */
+  uint64_t seed;           /* Philox key */
+  int64_t row_base;        /* global seed index of batch row 0 */
+} ttl_noise;
+
+/* ttl_env_step, ttl_env_step_head and ttl_env_step_begin with the noise drawn on the device as
+ * described at ttl_noise: no host work, no copy and no extra launch per step.  prm->dir_f64 must be 1
+ * (the noisy environment's float64 directions), else TTL_ERR_UNSUPPORTED. */
+int ttl_env_step_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                     const float* actions, int32_t lda, const ttl_noise* nz, int32_t n_upper, void* stream);
+int ttl_env_step_head_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                          const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
+                          const float* head_bias, const ttl_noise* nz, int32_t n_upper, void* stream);
+int ttl_env_step_begin_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                           const float* actions, int32_t lda, const ttl_noise* nz, int32_t n_upper,
+                           void* stream);
+/* The standard normals the step kernels use, for tests: out [n][3] f64, out[k][c] = z_c(nz->seed, g[k],
+ * L[k]) for g [n] int64 and L [n] int32 (device arrays); nz->sigma and nz->row_base are ignored. */
+int ttl_noise_normals(const ttl_noise* nz, const int64_t* g, const int32_t* L, int32_t n, double* out,
+                      void* stream);
 
 /* Re-orders the alive list alive[cur] by the voxel raster index of every streamline's tip (radix sort of
  * the keys + one pass moving rank records, alive ids and operand rows into the cur ^ 1 buffers); the

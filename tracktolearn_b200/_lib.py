@@ -40,6 +40,11 @@ class Batch(ctypes.Structure):
                 ('operand_fmt', c_i32), ('order', c_vp)]
 
 
+class Noise(ctypes.Structure):
+    """ttl_noise: N(0, sigma) tracking noise drawn inside the step kernel (include/ttl_b200.h)."""
+    _fields_ = [('sigma', c_f64), ('seed', ctypes.c_uint64), ('row_base', c_i64)]
+
+
 class ActorWeights(ctypes.Structure):
     _fields_ = [('n_layers', c_i32), ('in_dim', c_i32 * MAX_LAYERS), ('out_dim', c_i32 * MAX_LAYERS),
                 ('w', c_vp * MAX_LAYERS), ('b', c_vp * MAX_LAYERS)]
@@ -70,6 +75,11 @@ SIGNATURES = {
     'ttl_env_step_head': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_i32, c_vp, c_i32, c_vp]),
     'ttl_env_step_begin': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_vp, c_i32, c_vp]),
     'ttl_env_step_finish': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_i32, c_i32, c_f32, c_i32, c_vp]),
+    'ttl_env_step_rng': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, P(Noise), c_i32, c_vp]),
+    'ttl_env_step_head_rng': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_i32, c_vp, P(Noise), c_i32,
+                                      c_vp]),
+    'ttl_env_step_begin_rng': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, P(Noise), c_i32, c_vp]),
+    'ttl_noise_normals': (c_i32, [P(Noise), c_vp, c_vp, c_i32, c_vp, c_vp]),
     'ttl_oracle_features_rows': (c_i32, [P(Batch), c_i32, c_i32, c_vp, c_vp]),
     'ttl_env_resort_workspace_bytes': (c_i64, [c_i32]),
     'ttl_env_resort': (c_i32, [P(Volume), P(Batch), c_i32, c_i32, c_vp, c_i64, c_vp]),

@@ -23,7 +23,9 @@ class StepRunner(object):
         self.env, self.actor, self.prob = env, actor, prob
         self.action_buf = torch.empty((env._b.n_slots, actor.action_dim), dtype=torch.float32,
                                       device=env.device)
-        noisy = getattr(env, 'noise', 0.0) > 0.0
+        # host-drawn noise arrives as an array per step: no fused head, nothing to replay.  Noise the step
+        # kernel draws itself (noise_rng = 'device') needs neither restriction.
+        noisy = getattr(env, 'noise', 0.0) > 0.0 and env._device_noise() is None
         self.use_graph = bool(use_graph) and prob == 0.0 and not noisy and not env.compute_reward \
             and env._oracle is None
         self.graphs = None
@@ -121,8 +123,10 @@ class RLAlgorithm(object):
     def _runner_for(self, env, actor, prob, use_graph):
         """The captured graphs hold raw pointers into the env's batch buffers and the actor's plan:
         keep one runner per (buffers, plan) and reuse it across episodes."""
+        nz = env._device_noise()      # a captured graph holds the noise parameters by value
         key = (id(env), id(env._batch), env._b.n_slots, env._batch.fp32_state, id(actor), id(actor._plan), prob,
-               bool(use_graph), bool(getattr(self, 'fuse_head', True)))
+               bool(use_graph), bool(getattr(self, 'fuse_head', True)),
+               None if nz is None else (nz.sigma, nz.seed, nz.row_base))
         if getattr(self, '_runner_key', None) != key or self._runner is None:
             self._runner = StepRunner(env, actor, prob, use_graph=use_graph,
                                       fuse_head=getattr(self, 'fuse_head', True))

@@ -32,6 +32,7 @@
 #include <cuda_fp16.h>
 
 #include "ttl_common.cuh"
+#include "ttl_rng.cuh"
 
 std::atomic<long long> g_ttl_launches{0};
 
@@ -383,10 +384,13 @@ struct ActionSrc {
   int n_rows;             // rows the launch covers (>= the alive count): bound for speculative loads
 };
 
-template <int MINB>
+// Where the noise comes from.  RNG = false: the optional host-drawn array `noise` [n_alive][3] per rank.
+// RNG = true (dir_f64 only): drawn here from the counter-based generator (ttl_rng.cuh) at
+// (nz.seed, nz.row_base + row, L); lanes 0-2 of the quad draw one component each and share them.
+template <int MINB, bool RNG>
 __global__ void __launch_bounds__(kK1Threads, MINB) propagate_stop_kernel(
     ttl_volume v, ttl_params prm, ttl_batch b, int cur, ActionSrc src,
-    const double* __restrict__ noise, int defer) {
+    const double* __restrict__ noise, int defer, ttl_noise nz) {
   // 4 lanes per streamline: they redo the cheap scalar work together and split the spline taps
   const int lane = threadIdx.x & 31, sub = threadIdx.x & (kLanesPerRow - 1);
   const unsigned quad_mask = 0xFu << (lane & ~(kLanesPerRow - 1));
@@ -422,7 +426,13 @@ __global__ void __launch_bounds__(kK1Threads, MINB) propagate_stop_kernel(
   if (prm.dir_f64) {
     // noisy_tracking_env.py:74-77 then env.py:493-502, all float64
     double dx = (double)ax, dy = (double)ay, dz = (double)az;
-    if (noise) {
+    const int quad_base = lane & ~(kLanesPerRow - 1);
+    if constexpr (RNG) {
+      const double za = __dmul_rn(nz.sigma, ttl_noise_normal(nz.seed, nz.row_base + i, L, min(sub, 2)));
+      dx = __dadd_rn(dx, __shfl_sync(quad_mask, za, quad_base + 0));
+      dy = __dadd_rn(dy, __shfl_sync(quad_mask, za, quad_base + 1));
+      dz = __dadd_rn(dz, __shfl_sync(quad_mask, za, quad_base + 2));
+    } else if (noise) {
       dx = __dadd_rn(dx, noise[3 * (size_t)r + 0]);
       dy = __dadd_rn(dy, noise[3 * (size_t)r + 1]);
       dz = __dadd_rn(dz, noise[3 * (size_t)r + 2]);
@@ -433,7 +443,6 @@ __global__ void __launch_bounds__(kK1Threads, MINB) propagate_stop_kernel(
     const double pa = (double)(sub == 0 ? px : (sub == 1 ? py : pz));
     const double sa = __dmul_rn(__ddiv_rn(da, nrm), prm.step_vox);
     const float qa = (float)__dadd_rn(pa, sa);
-    const int quad_base = lane & ~(kLanesPerRow - 1);
     qx = __shfl_sync(quad_mask, qa, quad_base + 0);
     qy = __shfl_sync(quad_mask, qa, quad_base + 1);
     qz = __shfl_sync(quad_mask, qa, quad_base + 2);
@@ -493,6 +502,15 @@ __global__ void __launch_bounds__(kK1Threads, MINB) propagate_stop_kernel(
   }  // r < n_alive
 
   if (!(defer & 1)) publish_stops(b, cur, stopped);
+}
+
+// ttl_noise_normals: one thread per (row, component)
+__global__ void noise_normals_kernel(unsigned long long seed, const long long* __restrict__ g,
+                                     const int32_t* __restrict__ L, int n, double* __restrict__ out) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= 3LL * n) return;
+  const int k = (int)(t / 3), c = (int)(t % 3);
+  out[t] = ttl_noise_normal(seed, g[k], L[k], c);
 }
 
 // OracleStoppingCriterion (stopping_criteria.py:113-154) and OracleReward (oracle_reward.py:45-93)
@@ -1300,19 +1318,40 @@ static int k1_min_blocks() {
   return v;
 }
 
-static void launch_propagate(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
-                             const ActionSrc& src, const double* noise, int defer, int n_upper, cudaStream_t s) {
-  const int grid = ttl_div_up(n_upper, kGroup);
+extern "C++" {   // (inside the extern "C" block)
+template <bool RNG>
+static void launch_propagate_as(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
+                                const ActionSrc& src, const double* noise, int defer, const ttl_noise& nz,
+                                int grid, cudaStream_t s) {
   switch (k1_min_blocks()) {
     case 5:
-      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<5>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer));
+      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<5, RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
       break;
     case 8:
-      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<8>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer));
+      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<8, RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
       break;
     default:
-      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<6>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer));
+      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<6, RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
   }
+}
+}  // extern "C++"
+
+// nz != NULL: the noise is drawn in the kernel (ttl_noise) and `noise` must be NULL
+static void launch_propagate(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
+                             const ActionSrc& src, const double* noise, int defer, int n_upper, cudaStream_t s,
+                             const ttl_noise* nz = nullptr) {
+  const int grid = ttl_div_up(n_upper, kGroup);
+  if (nz)
+    launch_propagate_as<true>(vol, prm, b, cur, src, nullptr, defer, *nz, grid, s);
+  else
+    launch_propagate_as<false>(vol, prm, b, cur, src, noise, defer, ttl_noise{0.0, 0, 0}, grid, s);
+}
+
+// the device-noise entry points need the float64 direction arithmetic the noise is defined in
+static int check_noise(const ttl_params* prm, const ttl_noise* nz) {
+  if (!prm || !nz || !(nz->sigma >= 0.0) || isinf(nz->sigma)) return TTL_ERR_BAD_ARG;
+  if (!prm->dir_f64) return TTL_ERR_UNSUPPORTED;
+  return 0;
 }
 
 // A/B knobs of the state kernel (TTL_STATE_OPTIONS or ttl_state_options()): bits 0-1 prefetch the
@@ -1371,50 +1410,90 @@ static int check_step_args(const ttl_volume* vol, const ttl_params* prm, const t
 
 void ttl_state_options(int32_t bits) { g_state_opts.store(bits & 15); }
 
-int ttl_env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                 const float* actions, int32_t lda, const double* noise, int32_t n_upper,
-                 void* stream) {
+static int env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                    const float* actions, int32_t lda, const double* noise, const ttl_noise* nz, int defer,
+                    int32_t n_upper, cudaStream_t s) {
   if (n_upper <= 0) return 0;   // nothing alive: no launch (and no action buffer to look at)
   if (!actions || lda < 3) return TTL_ERR_BAD_ARG;
   int rc = check_step_args(vol, prm, b, cur, &n_upper);
   if (rc) return rc;
-  cudaStream_t s = (cudaStream_t)stream;
   const ActionSrc src = {actions, lda, nullptr, 0, 1, nullptr, n_upper};
-  launch_propagate(vol, prm, b, cur, src, noise, 0, n_upper, s);
-  rc = launch_build_state(vol, prm, b, cur, n_upper, s);
-  if (rc) return rc;
+  launch_propagate(vol, prm, b, cur, src, noise, defer, n_upper, s, nz);
+  if (!defer) {
+    rc = launch_build_state(vol, prm, b, cur, n_upper, s);
+    if (rc) return rc;
+  }
   TTL_CHECK_LAST();
   return 0;
 }
 
-int ttl_env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                      const float* head_partial, int32_t n_tiles, int32_t tiles_per_256, const float* head_bias,
-                      int32_t n_upper, void* stream) {
+static int env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                         const float* head_partial, int32_t n_tiles, int32_t tiles_per_256, const float* head_bias,
+                         const ttl_noise* nz, int32_t n_upper, cudaStream_t s) {
   if (n_upper <= 0) return 0;
   if (!head_partial || !head_bias || n_tiles < 1 || (reinterpret_cast<uintptr_t>(head_partial) & 15) ||
       (tiles_per_256 != 1 && tiles_per_256 != 2 && tiles_per_256 != 4))
     return TTL_ERR_BAD_ARG;
   int rc = check_step_args(vol, prm, b, cur, &n_upper);
   if (rc) return rc;
-  cudaStream_t s = (cudaStream_t)stream;
   const ActionSrc src = {nullptr, 0, head_partial, n_tiles, tiles_per_256, head_bias, n_upper};
-  launch_propagate(vol, prm, b, cur, src, nullptr, 0, n_upper, s);
+  launch_propagate(vol, prm, b, cur, src, nullptr, 0, n_upper, s, nz);
   rc = launch_build_state(vol, prm, b, cur, n_upper, s);
   if (rc) return rc;
   TTL_CHECK_LAST();
   return 0;
 }
 
+int ttl_env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                 const float* actions, int32_t lda, const double* noise, int32_t n_upper,
+                 void* stream) {
+  return env_step(vol, prm, b, cur, actions, lda, noise, nullptr, 0, n_upper, (cudaStream_t)stream);
+}
+
+int ttl_env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                      const float* head_partial, int32_t n_tiles, int32_t tiles_per_256, const float* head_bias,
+                      int32_t n_upper, void* stream) {
+  return env_step_head(vol, prm, b, cur, head_partial, n_tiles, tiles_per_256, head_bias, nullptr, n_upper,
+                       (cudaStream_t)stream);
+}
+
 int ttl_env_step_begin(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
                        const float* actions, int32_t lda, const double* noise, int32_t n_upper,
                        void* stream) {
-  if (n_upper <= 0) return 0;
-  if (!actions || lda < 3) return TTL_ERR_BAD_ARG;
-  int rc = check_step_args(vol, prm, b, cur, &n_upper);
+  return env_step(vol, prm, b, cur, actions, lda, noise, nullptr, 1, n_upper, (cudaStream_t)stream);
+}
+
+int ttl_env_step_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                     const float* actions, int32_t lda, const ttl_noise* nz, int32_t n_upper, void* stream) {
+  int rc = check_noise(prm, nz);
   if (rc) return rc;
-  cudaStream_t s = (cudaStream_t)stream;
-  const ActionSrc src = {actions, lda, nullptr, 0, 1, nullptr, n_upper};
-  launch_propagate(vol, prm, b, cur, src, noise, 1, n_upper, s);
+  return env_step(vol, prm, b, cur, actions, lda, nullptr, nz, 0, n_upper, (cudaStream_t)stream);
+}
+
+int ttl_env_step_head_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                          const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
+                          const float* head_bias, const ttl_noise* nz, int32_t n_upper, void* stream) {
+  int rc = check_noise(prm, nz);
+  if (rc) return rc;
+  return env_step_head(vol, prm, b, cur, head_partial, n_tiles, tiles_per_256, head_bias, nz, n_upper,
+                       (cudaStream_t)stream);
+}
+
+int ttl_env_step_begin_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                           const float* actions, int32_t lda, const ttl_noise* nz, int32_t n_upper,
+                           void* stream) {
+  int rc = check_noise(prm, nz);
+  if (rc) return rc;
+  return env_step(vol, prm, b, cur, actions, lda, nullptr, nz, 1, n_upper, (cudaStream_t)stream);
+}
+
+int ttl_noise_normals(const ttl_noise* nz, const int64_t* g, const int32_t* L, int32_t n, double* out,
+                      void* stream) {
+  if (n <= 0) return 0;
+  if (!nz || !g || !L || !out) return TTL_ERR_BAD_ARG;
+  TTL_LAUNCH("noise_normals_kernel", (cudaStream_t)stream,
+             noise_normals_kernel<<<ttl_div_up((long long)n * 3, 256), 256, 0, (cudaStream_t)stream>>>(
+                 nz->seed, (const long long*)g, L, n, out));
   TTL_CHECK_LAST();
   return 0;
 }

@@ -223,6 +223,10 @@ class TrackingEnvironment(BaseEnv):
         return self._start(self.seeds[seeds])
 
     # ------------------------------------------------------------------- device protocol
+    def _device_noise(self):
+        """``_lib.Noise`` when the step kernels draw the noise themselves (ttl_env_step_rng), else None."""
+        return None
+
     def step_device(self, actions, noise=None):
         """Enqueue one step for the alive rows.  ``actions``: CUDA float32 tensor
         [>= n_alive, >= 3] (row stride taken from the tensor).  No host synchronisation."""
@@ -233,16 +237,24 @@ class TrackingEnvironment(BaseEnv):
         lda = actions.stride(0) if actions.dim() == 2 and actions.shape[0] > 1 else actions.shape[-1]
         sp = _lib.stream_ptr(self.device)
         n_up = int(self._n_alive_host)
+        nz = self._device_noise()
+        if nz is not None and noise is not None:
+            raise ValueError('the step kernels draw the noise of this environment; no noise array is taken')
+        args = (ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
+                _lib.ptr(actions), int(lda))
         if self._oracle is None:
-            _lib.check(self._lib.ttl_env_step(
-                ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
-                _lib.ptr(actions), int(lda), _lib.ptr(noise), n_up, sp), 'ttl_env_step')
+            if nz is None:
+                _lib.check(self._lib.ttl_env_step(*args, _lib.ptr(noise), n_up, sp), 'ttl_env_step')
+            else:
+                _lib.check(self._lib.ttl_env_step_rng(*args, ctypes.byref(nz), n_up, sp), 'ttl_env_step_rng')
         else:
             # propagate + geometric criteria, then score every alive streamline, then ORACLE flag /
             # bonus / compaction / state rows
-            _lib.check(self._lib.ttl_env_step_begin(
-                ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
-                _lib.ptr(actions), int(lda), _lib.ptr(noise), n_up, sp), 'ttl_env_step_begin')
+            if nz is None:
+                _lib.check(self._lib.ttl_env_step_begin(*args, _lib.ptr(noise), n_up, sp), 'ttl_env_step_begin')
+            else:
+                _lib.check(self._lib.ttl_env_step_begin_rng(*args, ctypes.byref(nz), n_up, sp),
+                           'ttl_env_step_begin_rng')
             if n_up > 0:
                 slots = self._b.n_slots
                 if getattr(self, '_oracle_dirs', None) is None or self._oracle_dirs.shape[0] < slots:
@@ -270,10 +282,15 @@ class TrackingEnvironment(BaseEnv):
         if self._oracle is not None:
             raise RuntimeError('step_device_head does not consult the oracle; use step_device')
         partial, n_tiles, tiles_per_256, bias = head
-        _lib.check(self._lib.ttl_env_step_head(
-            ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
-            partial, int(n_tiles), int(tiles_per_256), bias, int(self._n_alive_host),
-            _lib.stream_ptr(self.device)), 'ttl_env_step_head')
+        args = (ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
+                partial, int(n_tiles), int(tiles_per_256), bias)
+        nz = self._device_noise()
+        if nz is None:
+            _lib.check(self._lib.ttl_env_step_head(*args, int(self._n_alive_host), _lib.stream_ptr(self.device)),
+                       'ttl_env_step_head')
+        else:
+            _lib.check(self._lib.ttl_env_step_head_rng(*args, ctypes.byref(nz), int(self._n_alive_host),
+                                                       _lib.stream_ptr(self.device)), 'ttl_env_step_head_rng')
         self.length += 1
         self._pending_harvest = True
 

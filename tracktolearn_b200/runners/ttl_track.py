@@ -39,6 +39,7 @@ class TrackToLearnTrack(object):
         self.reference_file = track_dto['in_mask']
         self.out_tractogram = track_dto['out_tractogram']
         self.noise = track_dto['noise']
+        self.noise_rng = track_dto.get('noise_rng', 'host')
         self.binary_stopping_threshold = track_dto['binary_stopping_threshold']
         self.n_actor = track_dto['n_actor']
         self.npv = track_dto['npv']
@@ -92,7 +93,7 @@ class TrackToLearnTrack(object):
             'device': self.device, 'target_sh_order': int(self.target_sh_order),
             'in_odf': self.in_odf, 'in_seed': self.in_seed, 'in_mask': self.in_mask,
             'sh_basis': self.sh_basis, 'input_wm': self.input_wm, 'reference': self.reference_file,
-            'state_of_stopped': False,
+            'state_of_stopped': False, 'noise_rng': self.noise_rng, 'noise_seed': self.random_seed,
         }
         return NoisyTrackingEnvironment.from_files(env_dto)
 
@@ -178,6 +179,13 @@ def add_track_args(parser):
     track_g.add_argument('--noise', default=0.0, type=float, metavar='sigma',
                          help='Add noise ~ N (0, `noise`) to the agent\'s\noutput to make tracking more '
                               'probabilistic.\nShould be between 0.0 and 0.1.[%(default)s]')
+    track_g.add_argument('--noise_rng', default='host', choices=['host', 'device'],
+                         help='Where the `--noise` draws come from.\nhost: the reference\'s numpy RandomState '
+                              'stream, drawn on the CPU every step;\nthe tractogram then depends on --n_actor and '
+                              'on the number of GPUs.\ndevice: drawn inside the GPU step from --rng_seed, the seed\'s '
+                              'index and the step;\nthe tractogram is the same for every --n_actor and GPU count, and '
+                              'no host work is added per step.\nNeither reproduces the reference\'s random '
+                              'stream. [%(default)s]')
     track_g.add_argument('--fa_map', type=str, default=None,
                          help='Scale the added noise (see `--noise`) according\nto the provided FA map '
                               '(.nii.gz). Optional.')

@@ -97,7 +97,9 @@ class Tracker(object):
         ranks are gathered on rank 0 in rank order -- the order one GPU would have produced
         (tracker.py:106-145 collects batch after batch the same way).  Yields the merged Tractogram on
         rank 0 and None elsewhere; without torch.distributed it is ``track_packed``.  All ranks must make
-        the same number of passes."""
+        the same number of passes.  With device-drawn noise (``noise_rng='device'``) the caller also sets
+        ``env.seed_offset`` to the index of its first seed in the unsharded list (``parallel.shard_bounds``),
+        so that every seed gets the noise one GPU would give it."""
         from tracktolearn_b200 import parallel
         self.alg.agent.eval()
         for start, end, slots in self._passes(env):
@@ -163,6 +165,9 @@ class Tracker(object):
         world = dist.get_world_size() if dist.is_initialized() else 1
         rank = dist.get_rank() if dist.is_initialized() else 0
         if world > 1:
+            # device-drawn noise is keyed by the index in the common shuffled list: tell the env where its
+            # slice starts, so that every seed gets the noise it gets on one GPU
+            env.seed_offset = parallel.shard_bounds(len(env.seeds), rank, world)[0]
             env.seeds = parallel.shard_seeds(env.seeds, rank, world)
         vox_size = np.mean(np.abs(affine)[np.diag_indices(4)][:3])
         lo, hi = self.min_length / vox_size, self.max_length / vox_size
