@@ -2,8 +2,8 @@
 """Small end-to-end run for compute-sanitizer (scripts/sanitize.sh): reset + 20 steps of the reference
 protocol (fp32 state rows, host actions), a streaming device-mode episode in every tensor-core tier (fused
 multi-layer actor launch with its inter-layer flags, stop bookkeeping across the two env kernels, slot
-refill, the periodic tip sort), TractOracle-Net scoring, and the tractogram pack.  Sizes are tiny: the
-sanitizer slows kernels down by one to two orders of magnitude."""
+refill), TractOracle-Net scoring, and the tractogram pack.  Sizes are tiny: the sanitizer slows kernels
+down by one to two orders of magnitude."""
 import os
 import sys
 
@@ -48,12 +48,11 @@ def main():
         env.step(a)
         state, _ = env.harvest()
     n_done_api = int(env.dones.sum())
-    # device mode, every tensor-core tier, with the periodic tip sort
+    # device mode, every tensor-core tier
     counts = {}
     for prec in ('fp16', 'tf32', 'bf16'):
         alg = SACAuto(615, 3, '256-256-256', n_actors=300, device=dev, precision=prec)
         alg.agent.actor.load_state_dict(sd)
-        alg.resort_every = 4
         env.reset_streaming(0, len(seeds), 128, fp32_state=False, operand=prec)
         alg.validation_episode(None, env, 0.0)
         counts[prec] = int(env.streamline_steps())

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define TTL_ABI_VERSION 3
+#define TTL_ABI_VERSION 4
 
 /* StoppingFlags, environments/stopping_criteria.py:10-20 */
 #define TTL_STOPPING_MASK 1
@@ -212,8 +212,8 @@ int ttl_env_step_finish(const ttl_volume* vol, const ttl_params* prm, const ttl_
  *   u1 = (((w1 << 32 | w0) >> 12) + 0.5) * 2^-52,  u2 = (((w3 << 32 | w2) >> 12) + 0.5) * 2^-52
  *   z_c = sqrt(-2 ln u1) * cos(2 pi u2)            (fp64; |z_c| <= 8.58)
  * added in fp64 to the action where ttl_env_step adds its `noise` array.  Each streamline's noise
- * depends only on (seed, g, L, c): not on the alive-list order, the slot count, refill, the tip sort or
- * the process that tracks it, so a run sharded over GPUs (row_base = the shard's first index in the
+ * depends only on (seed, g, L, c): not on the alive-list order, the slot count, refill or the process
+ * that tracks it, so a run sharded over GPUs (row_base = the shard's first index in the
  * common seed list) produces what one GPU produces.  It is not the reference's RandomState stream.
  * The struct is a host structure read at call time (like ttl_params); a CUDA graph captures its values. */
 typedef struct ttl_noise {
@@ -237,17 +237,6 @@ int ttl_env_step_begin_rng(const ttl_volume* vol, const ttl_params* prm, const t
  * L[k]) for g [n] int64 and L [n] int32 (device arrays); nz->sigma and nz->row_base are ignored. */
 int ttl_noise_normals(const ttl_noise* nz, const int64_t* g, const int32_t* L, int32_t n, double* out,
                       void* stream);
-
-/* Re-orders the alive list alive[cur] by the voxel raster index of every streamline's tip (radix sort of
- * the keys + one pass moving rank records, alive ids and operand rows into the cur ^ 1 buffers); the
- * caller flips cur afterwards, as after a step.  Operand-only device mode only (bf16_layout 1): there the
- * position of a streamline in the list is free, rows keep their identity and every per-row result is
- * unchanged.  No counterpart in the reference; it restores the gather locality of env.py:538-541 after
- * streamlines that were seeded together have drifted apart.  workspace: device,
- * ttl_env_resort_workspace_bytes(n_slots) bytes. */
-int64_t ttl_env_resort_workspace_bytes(int32_t n_slots);
-int ttl_env_resort(const ttl_volume* vol, const ttl_batch* b, int32_t cur, int32_t n_upper, void* workspace,
-                   int64_t workspace_bytes, void* stream);
 
 /* state[cur^1][dest[r]] -> out[r] for r < n_rows: the `self.state[self.continue_idx]` that
  * step() returns, in the order of the pre-harvest alive list (tracking_env.py:217-218). */
@@ -424,10 +413,6 @@ void ttl_prof_enable(int32_t on);
  * (every one of them waits for its predecessor's completion before its first global access).
  * On by default; 0 switches back to plain stream-ordered launches. */
 void ttl_pdl_enable(int32_t on);
-/* A/B switches of the device-mode state kernel (default 0): bits 0-1 prefetch the row's cache lines
- * into L1 (1) / L2 (2) before gathering, bit 3 recompute the previous-direction block from the fp32
- * points instead of shifting the previous row's.  Results are identical in every combination. */
-void ttl_state_options(int32_t bits);
 int32_t ttl_prof_report(char* buf_host, int32_t buflen);
 
 #ifdef __cplusplus

@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, 'include', 'ttl_b200.h')
 
 
-def test_library_builds_and_exports_declared_symbols():
+def test_library_builds_and_exports_the_abi_v4_symbols():
     build.build()
     lib = _lib.load()
     text = open(HEADER).read()
@@ -24,7 +24,7 @@ def test_library_builds_and_exports_declared_symbols():
     for name in declared:
         assert hasattr(lib, name), name
     assert declared == set(_lib.SIGNATURES), declared ^ set(_lib.SIGNATURES)
-    assert lib.ttl_abi_version() == _lib.ABI_VERSION == 3
+    assert lib.ttl_abi_version() == _lib.ABI_VERSION == 4
     assert lib.ttl_launch_count() >= 0
 
 

@@ -35,7 +35,6 @@ def test_no_kernel_writes_outside_its_buffers(guarded, n_seeds, slots):
         alg = SACAuto(615, 3, '128-128-128', n_actors=slots, device=torch.device('cuda:0'), precision=prec)
         alg.agent.actor.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
         for fp32_state in (True, False):
-            alg.resort_every = 0 if fp32_state else 3
             env._batch = None            # exact-size buffers: the guards border what the kernels may touch
             st = env.reset_streaming(0, n, slots, fp32_state=fp32_state, operand=prec)
             assert env._batch.GUARD and len(env._batch._guarded) > 15

@@ -59,12 +59,12 @@ def test_philox_normals_shape_and_dependence():
     assert not np.array_equal(big, N.philox_normals(3, np.asarray([7]), 5))
 
 
-def test_noise_entry_points_are_exported_and_bound():
+def test_noise_entry_points_are_exported_and_bound_in_abi_v4():
     build.build()
     lib = _lib.load()
     for name in ('ttl_env_step_rng', 'ttl_env_step_head_rng', 'ttl_env_step_begin_rng', 'ttl_noise_normals'):
         assert hasattr(lib, name) and name in _lib.SIGNATURES, name
-    assert lib.ttl_abi_version() == _lib.ABI_VERSION == 3
+    assert lib.ttl_abi_version() == _lib.ABI_VERSION == 4
 
 
 def test_noise_struct_layout_matches_header():
@@ -87,8 +87,8 @@ int main(void) {
                    _lib.Noise.row_base.offset]
 
 
-def test_rng_step_kernel_adds_no_stack_at_default_occupancy():
-    """The RNG instantiation of propagate_stop_kernel at 6 CTAs per SM (the default) fits the 80 registers
+def test_rng_step_kernel_adds_no_stack_at_six_ctas_per_sm():
+    """The RNG instantiation of propagate_stop_kernel, built for 6 CTAs per SM, fits the 80 registers
     that occupancy leaves without spilling: its stack frame is the plain instantiation's (a 40-byte local
     array both have), no larger."""
     tool = shutil.which('cuobjdump') or '/usr/local/cuda/bin/cuobjdump'
@@ -97,11 +97,11 @@ def test_rng_step_kernel_adds_no_stack_at_default_occupancy():
     build.build()
     out = subprocess.run([tool, '-res-usage', _lib.LIB_PATH], stdout=subprocess.PIPE, stderr=subprocess.STDOUT,
                          check=True).stdout.decode()
-    found = {(int(m), b): (int(reg), int(stack)) for m, b, reg, stack in re.findall(
-        r'Function \S*propagate_stop_kernelILi(\d)ELb([01])E\S*:\s*\n\s*REG:(\d+) STACK:(\d+)', out)}
-    assert set(found) == {(m, b) for m in (5, 6, 8) for b in '01'}, found
-    reg, stack = found[(6, '1')]
-    assert reg <= 80 and stack == found[(6, '0')][1], found
+    found = {b: (int(reg), int(stack)) for b, reg, stack in re.findall(
+        r'Function \S*propagate_stop_kernelILb([01])E\S*:\s*\n\s*REG:(\d+) STACK:(\d+)', out)}
+    assert set(found) == {'0', '1'}, found
+    reg, stack = found['1']
+    assert reg <= 80 and stack == found['0'][1], found
 
 
 def test_ttl_track_help_lists_noise_rng():

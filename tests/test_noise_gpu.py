@@ -196,11 +196,8 @@ def test_device_noise_tractogram_does_not_depend_on_scheduling():
         alg.use_cuda_graph = True
         _assert_same(ref, _episode(env, alg, 0, n, slots=256), 'graph replay')
         assert alg._runner.graphs is not None and alg._runner.replays > 10
-        alg.use_cuda_graph = False
-        alg.resort_every = 4
-        _assert_same(ref, _episode(env, alg, 0, n, slots=256), 'tip sort every 4 steps')
     finally:
-        alg.fuse_head, alg.use_cuda_graph, alg.resort_every = True, False, 0
+        alg.fuse_head, alg.use_cuda_graph = True, False
     # two shards of the same list, tracked one after the other, concatenated
     k = 377
     env.seeds, env.seed_offset = seeds[:k], 0

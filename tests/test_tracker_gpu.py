@@ -219,38 +219,6 @@ def test_bf16_direction_block_is_the_rounded_point_differences(prec):
 
 
 @pytest.mark.parametrize('prec', TC)
-def test_state_kernel_variants_write_identical_rows(prec):
-    """The shifted direction block (default) and the recomputed one (bit 3), with and without the L2
-    prefetch (bit 1), produce bit-identical operand rows, hence bit-identical streamlines."""
-    from tracktolearn_b200 import _lib
-    lib = _lib.load()
-    env, alg, sub, seeds, sd = _setup(precision=prec)
-    n = len(seeds)
-    out, rows = [], []
-    try:
-        for opts in (0, 8, 2, 8 | 1):
-            lib.ttl_state_options(opts)
-            st = env.reset_streaming(0, n, 256, fp32_state=False)
-            from tracktolearn_b200.algorithms.rl import StepRunner
-            runner = StepRunner(env, alg.agent.actor, 0.0, use_graph=False)
-            for _ in range(12):
-                runner.step()
-            torch.cuda.synchronize()
-            rows.append(env._batch.state_bf16[env._cur][:256].clone())
-            st = env.reset_streaming(0, n, 256, fp32_state=False)
-            alg.validation_episode(st, env, 0.0)
-            out.append(env.get_streamlines())
-    finally:
-        lib.ttl_state_options(0)
-    bits = torch.int32 if prec == 'tf32' else torch.int16
-    for r in rows[1:]:
-        assert torch.equal(rows[0].view(bits), r.view(bits))
-    for b in out[1:]:
-        np.testing.assert_array_equal(out[0].lengths, b.lengths)
-        np.testing.assert_array_equal(out[0].data, b.data)
-
-
-@pytest.mark.parametrize('prec', TC)
 def test_cuda_graph_replay_equals_plain_launches(prec):
     """validation_episode with the step replayed from two captured CUDA graphs (one per ping-pong
     parity; programmatic-dependent-launch edges inside) vs plain launches: same streamlines."""
@@ -297,44 +265,6 @@ def test_locality_order_does_not_change_any_streamline(prec):
     np.testing.assert_array_equal(a.data, b.data)
     np.testing.assert_array_equal(a.data_per_streamline['flags'], b.data_per_streamline['flags'])
     np.testing.assert_array_equal(a.data_per_streamline['seeds'], b.data_per_streamline['seeds'])
-
-
-@pytest.mark.parametrize('prec', TC)
-def test_periodic_tip_sort_does_not_change_any_streamline(prec):
-    """Streaming tracker with the alive list re-sorted by tip voxel every 5 steps (ttl_env_resort) vs never:
-    every row holds the same streamline, bit for bit; and the list really is in voxel order after a sort."""
-    env, alg, sub, seeds, sd = _setup(precision=prec)
-    n = len(seeds)
-    out = []
-    for every in (0, 5):
-        alg.resort_every = every
-        st = env.reset_streaming(0, n, 256, fp32_state=False)
-        alg.validation_episode(st, env, 0.0)
-        out.append(env.get_streamlines())
-        assert env.streamline_steps() == int((env.lengths - 1).sum())
-    alg.resort_every = 0
-    a, b = out
-    np.testing.assert_array_equal(a.lengths, b.lengths)
-    np.testing.assert_array_equal(a.data, b.data)
-    np.testing.assert_array_equal(a.data_per_streamline['flags'], b.data_per_streamline['flags'])
-    # the order itself: a few steps, one sort, keys ascending
-    from tracktolearn_b200.algorithms.rl import StepRunner
-    env.reset_streaming(0, n, 256, fp32_state=False)
-    runner = StepRunner(env, alg.agent.actor, 0.0, use_graph=False)
-    for _ in range(9):
-        runner.step()
-    before = env.n_alive()
-    env.resort_device()
-    assert env.n_alive() == before
-    rec = env._batch.rank_rec[env._cur][:before].cpu().numpy()
-    tips = rec[:, 2:5]
-    X, Y, Z = int(env._volume.X), int(env._volume.Y), int(env._volume.Z)
-    vox = np.clip(np.floor(tips).astype(np.int64), 0, [X - 1, Y - 1, Z - 1])
-    key = (vox[:, 0] * Y + vox[:, 1]) * Z + vox[:, 2]
-    assert (np.diff(key) >= 0).all()
-    rows = rec[:, 0].view(np.int32)
-    np.testing.assert_array_equal(np.sort(rows), np.sort(env._batch.alive[env._cur][:before].cpu().numpy()))
-    np.testing.assert_array_equal(rows, env._batch.alive[env._cur][:before].cpu().numpy())
 
 
 def test_training_episode_rollout_replay_and_update():

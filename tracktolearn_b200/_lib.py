@@ -15,7 +15,7 @@ PRECISION_BF16, PRECISION_FP32, PRECISION_FP16, PRECISION_TF32 = 0, 1, 2, 3
 PRECISIONS = {'bf16': PRECISION_BF16, 'fp32': PRECISION_FP32, 'fp16': PRECISION_FP16, 'tf32': PRECISION_TF32}
 OPERAND_BF16, OPERAND_FP16, OPERAND_TF32 = 0, 1, 2
 OPERAND_OF_PRECISION = {'bf16': OPERAND_BF16, 'fp16': OPERAND_FP16, 'tf32': OPERAND_TF32}
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 
 class Volume(ctypes.Structure):
@@ -65,7 +65,6 @@ SIGNATURES = {
     'ttl_launch_count': (c_i64, []),
     'ttl_prof_enable': (None, [c_i32]),
     'ttl_pdl_enable': (None, [c_i32]),
-    'ttl_state_options': (None, [c_i32]),
     'ttl_prof_report': (c_i32, [ctypes.c_char_p, c_i32]),
     'ttl_pad_channels': (c_i32, [c_vp, c_vp, c_i64, c_i32, c_i32, c_vp]),
     'ttl_peaks_from_sh': (c_i32, [c_vp, c_i64, c_i32, c_i32, c_vp, c_vp, c_vp, c_i32, c_i32, c_f64, c_f64, c_f64,
@@ -81,8 +80,6 @@ SIGNATURES = {
     'ttl_env_step_begin_rng': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, P(Noise), c_i32, c_vp]),
     'ttl_noise_normals': (c_i32, [P(Noise), c_vp, c_vp, c_i32, c_vp, c_vp]),
     'ttl_oracle_features_rows': (c_i32, [P(Batch), c_i32, c_i32, c_vp, c_vp]),
-    'ttl_env_resort_workspace_bytes': (c_i64, [c_i32]),
-    'ttl_env_resort': (c_i32, [P(Volume), P(Batch), c_i32, c_i32, c_vp, c_i64, c_vp]),
     'ttl_env_gather_step_state': (c_i32, [P(Batch), c_i32, c_i32, c_vp, c_i32, c_vp]),
     'ttl_format_state': (c_i32, [P(Volume), P(Params), c_vp, c_i32, c_i32, c_vp, c_i32, c_vp]),
     'ttl_stopping_flags': (c_i32, [P(Volume), P(Params), c_vp, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp]),

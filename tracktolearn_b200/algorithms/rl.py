@@ -112,10 +112,6 @@ class RLAlgorithm(object):
         self.use_cuda_graph = False
         # deterministic episodes read tanh(mu) straight from the actor's fused output layer
         self.fuse_head = True
-        # streaming device mode: re-sort the alive list by tip voxel every this many steps (0 = never);
-        # TTL_RESORT_EVERY overrides.  Measured on B200 (DESIGN.md section 4)
-        import os as _os
-        self.resort_every = int(_os.environ.get('TTL_RESORT_EVERY', '0'))
         self._snap_ring = None
         self._runner = None
         self._runner_key = None
@@ -160,9 +156,6 @@ class RLAlgorithm(object):
         done = False
         while not done and it < limit:
             rows = env._n_alive_host
-            if self.resort_every and streaming and it and it % self.resort_every == 0 and not env._batch.fp32_state \
-                    and runner.graphs is None:
-                env.resort_device()
             runner.step()
             if env.compute_reward:
                 # ctrl[3] = alive count the step just processed; rows beyond it hold stale rewards

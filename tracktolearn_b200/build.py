@@ -12,8 +12,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 LIB_DIR = os.path.join(HERE, 'lib')
 LIB_PATH = os.path.join(LIB_DIR, 'libttl_b200.so')
-SOURCES = ['ttl_env.cu', 'ttl_actor.cu', 'ttl_oracle_net.cu', 'ttl_tractogram.cu', 'ttl_sh.cu', 'ttl_prof.cu',
-           'ttl_resort.cu']
+SOURCES = ['ttl_env.cu', 'ttl_actor.cu', 'ttl_oracle_net.cu', 'ttl_tractogram.cu', 'ttl_sh.cu', 'ttl_prof.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC']
 

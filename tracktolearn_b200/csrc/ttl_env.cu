@@ -387,8 +387,8 @@ struct ActionSrc {
 // Where the noise comes from.  RNG = false: the optional host-drawn array `noise` [n_alive][3] per rank.
 // RNG = true (dir_f64 only): drawn here from the counter-based generator (ttl_rng.cuh) at
 // (nz.seed, nz.row_base + row, L); lanes 0-2 of the quad draw one component each and share them.
-template <int MINB, bool RNG>
-__global__ void __launch_bounds__(kK1Threads, MINB) propagate_stop_kernel(
+template <bool RNG>
+__global__ void __launch_bounds__(kK1Threads, 6) propagate_stop_kernel(
     ttl_volume v, ttl_params prm, ttl_batch b, int cur, ActionSrc src,
     const double* __restrict__ noise, int defer, ttl_noise nz) {
   // 4 lanes per streamline: they redo the cheap scalar work together and split the spline taps
@@ -627,27 +627,6 @@ __device__ __forceinline__ void corner_table(const ttl_volume& v, const ttl_para
   }
 }
 
-// Lane i (and i+32) asks the memory system for the two 128-byte lines of its corner voxel (a
-// 192-byte voxel always straddles exactly two lines): all ~52 distinct lines of a row are in
-// flight at once without holding a register each, and the LDG.128 gathers that follow wait one
-// latency instead of one per batch of loads.  level 1: into L1, 2: into L2.
-__device__ __forceinline__ void prefetch_corners(const ttl_volume& v, const int* s_vox, int lane, int level) {
-#pragma unroll
-  for (int rep = 0; rep < 2; ++rep) {
-    const int i = lane + 32 * rep;
-    if (i < 56) {
-      const char* a = reinterpret_cast<const char*>(v.sh) + (size_t)s_vox[i] * v.CP * 4;
-      if (level == 1) {
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(a));
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(a + 128));
-      } else {
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(a + 128));
-      }
-    }
-  }
-}
-
 // Builds one state row for the streamline whose points start at P (L points) and writes
 //   out_f32 [0, n_f32)   fp32: 7*C SH values | 3*n_dirs previous directions | zero padding
 //   out_bf16 [0, n_bf16) the same values rounded to bf16 (actor operand), zero padded
@@ -839,7 +818,7 @@ __device__ __forceinline__ void write_dirs_shifted(const uint8_t* __restrict__ o
 // once per volume instead of every kernel checking every value (tracking_env.py, _start).
 template <int FMT>
 __device__ void build_state_row_c45_op(const ttl_volume& v, const ttl_params& prm, const float* P, int L, float3 tip,
-                                       void* __restrict__ out_v, int n_op, float* smem_f, int lane, int pf = 0,
+                                       void* __restrict__ out_v, int n_op, float* smem_f, int lane,
                                        const uint8_t* __restrict__ old_dirs = nullptr,
                                        float3 prev_tip = make_float3(0.f, 0.f, 0.f)) {
   constexpr int CP = 48, CP4 = 12, S = 7 * CP;
@@ -848,7 +827,6 @@ __device__ void build_state_row_c45_op(const ttl_volume& v, const ttl_params& pr
   float* s_w = smem_f;
   int* s_vox = reinterpret_cast<int*>(smem_f + 64);
   corner_table(v, prm, tip, s_w, s_vox, lane);
-  if (pf & 3) prefetch_corners(v, s_vox, lane, pf & 3);   // own entries: no __syncwarp needed first
   __syncwarp();
   const float4* vol4 = reinterpret_cast<const float4*>(v.sh);
   // all 24 gathers of this lane's three work items are issued before the first is consumed
@@ -988,13 +966,15 @@ __device__ __forceinline__ Compaction survivors_before(const ttl_batch& b, const
   return c;
 }
 
-// FAST = 1: the operand-only device mode (ttl_batch.bf16_layout == 1) compiled on its own with a register
-// budget (85) that lets one lane keep all 24 of its LDG.128 gathers in flight; in the general kernel
-// ptxas keeps 4 in flight to stay at 47 registers.  FMT: element type of the operand rows in that mode.
-template <int FAST, int MINB, int FMT>
-__global__ void __launch_bounds__(kStateWarps * 32, MINB) build_state_kernel(ttl_volume v, ttl_params prm,
+// FAST = 1: the operand-only device mode (ttl_batch.bf16_layout == 1) compiled on its own for 6 CTAs per
+// SM, which caps it at 40 registers: ptxas spills a few dozen bytes per thread to fit (`-Xptxas -v`), and
+// launch_state_fmt records why 6 is still the fastest.  FAST = 0: every other layout, without a register
+// cap.  FMT: element type of the operand rows in the operand-only mode.  early_release: release the
+// dependent launch before this kernel's work (PDL on), see below.
+template <int FAST, int FMT>
+__global__ void __launch_bounds__(kStateWarps * 32, FAST ? 6 : 1) build_state_kernel(ttl_volume v, ttl_params prm,
                                                                                      ttl_batch b, int cur, int warp_smem,
-                                                                                     int pf) {
+                                                                                     int early_release) {
   extern __shared__ __align__(128) uint8_t smem_dyn[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* smem_f = reinterpret_cast<float*>(smem_dyn + (size_t)warp * warp_smem);
@@ -1005,7 +985,7 @@ __global__ void __launch_bounds__(kStateWarps * 32, MINB) build_state_kernel(ttl
   // Measured on B200 (50 000 rows): 316 -> 312 us per step.  The same early release in the dense
   // kernels and in propagate_stop was measured slower (up to +38 us with all of them on), so those
   // release at exit.
-  if (pf & 4) ttl_grid_dep_launch();
+  if (early_release) ttl_grid_dep_launch();
   // independent loads first, all of them addressed by r alone (buffers are padded past n_slots): alive count
   // and cursor, stop counts / flags, this rank's record and new point
   const int n_old = b.ctrl[cur];
@@ -1079,8 +1059,7 @@ __global__ void __launch_bounds__(kStateWarps * 32, MINB) build_state_kernel(ttl
     const uint8_t* old_dirs = static_cast<const uint8_t*>(b.state_bf16[cur]) +
                               ((size_t)r * b.ld_bf16 + 7 * 48) * (FMT == TTL_OPERAND_TF32 ? 4 : 2);
     const float3 prev_tip = make_float3(rec.tx, rec.ty, rec.tz);
-    build_state_row_c45_op<FMT>(v, prm, P, L, tip, o16, b.ld_bf16, smem_f, lane, pf, (pf & 8) ? nullptr : old_dirs,
-                                prev_tip);
+    build_state_row_c45_op<FMT>(v, prm, P, L, tip, o16, b.ld_bf16, smem_f, lane, old_dirs, prev_tip);
   }
   else
     build_state_row(v, prm, P, L, tip, o32, b.ld_state, o16, b.ld_bf16, smem_f, lane, b.bf16_layout, b.operand_fmt);
@@ -1202,21 +1181,22 @@ constexpr int kStateSmem = kStateWarps * kWarpSmemBytes;
 // flight) and 8 (32 registers) were measured at 70.0 and 74.7 us against 68.8 us for 50 000 rows.
 template <int FMT>
 cudaError_t launch_state_fmt(int grid, int smem, cudaStream_t s, const ttl_volume& vol, const ttl_params& prm,
-                             const ttl_batch& b, int cur, int warp_smem, int pf) {
+                             const ttl_batch& b, int cur, int warp_smem, int early_release) {
   static bool ready = false;
   if (!ready) {
-    cudaError_t e = cudaFuncSetAttribute(build_state_kernel<1, 6, FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(build_state_kernel<1, FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          kStateSmem);
     if (e != cudaSuccess) return e;
     ready = true;
   }
-  return ttl_launch_chain(build_state_kernel<1, 6, FMT>, grid, kStateWarps * 32, smem, s, vol, prm, b, cur, warp_smem, pf);
+  return ttl_launch_chain(build_state_kernel<1, FMT>, grid, kStateWarps * 32, smem, s, vol, prm, b, cur, warp_smem,
+                          early_release);
 }
 
 int state_kernels_ready() {
   static bool done = false;
   if (done) return 0;
-  cudaError_t e = cudaFuncSetAttribute(build_state_kernel<0, 1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStateSmem);
+  cudaError_t e = cudaFuncSetAttribute(build_state_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStateSmem);
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(reset_state_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStateSmem);
   if (e == cudaSuccess)
@@ -1306,33 +1286,14 @@ int ttl_env_reset(const ttl_volume* vol, const ttl_params* prm, const ttl_batch*
 
 // propagate_stop_kernel is latency-bound (a short dependent chain per streamline and ~90 registers
 // of fp64 spline state): how many 128-thread CTAs share an SM decides how many waves 50 000 rows
-// take.  Instantiations for 5 (94 registers, what ptxas picks unconstrained), 6 (80) and 8 (64, a
-// few spilled doubles) CTAs per SM; TTL_K1_MINB selects one for experiments, default below.
-static int k1_min_blocks() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TTL_K1_MINB");
-    v = e ? atoi(e) : 6;
-    if (v != 5 && v != 6 && v != 8) v = 6;
-  }
-  return v;
-}
-
+// take.  It is built for 6 CTAs per SM (80 registers); 5 (94 registers, what ptxas picks
+// unconstrained) and 8 (64, a few spilled doubles) were measured and not adopted.
 extern "C++" {   // (inside the extern "C" block)
 template <bool RNG>
 static void launch_propagate_as(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
                                 const ActionSrc& src, const double* noise, int defer, const ttl_noise& nz,
                                 int grid, cudaStream_t s) {
-  switch (k1_min_blocks()) {
-    case 5:
-      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<5, RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
-      break;
-    case 8:
-      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<8, RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
-      break;
-    default:
-      TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<6, RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
-  }
+  TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
 }
 }  // extern "C++"
 
@@ -1354,22 +1315,6 @@ static int check_noise(const ttl_params* prm, const ttl_noise* nz) {
   return 0;
 }
 
-// A/B knobs of the state kernel (TTL_STATE_OPTIONS or ttl_state_options()): bits 0-1 prefetch the
-// row's lines into L1 (1) / L2 (2) ahead of the gathers, bit 3 recompute the direction block from the
-// fp32 points instead of shifting the previous row's.  Default 0: every alternative was measured
-// slower or equal (DESIGN.md section 4).
-static std::atomic<int> g_state_opts{-1};
-static int state_prefetch_level() {
-  int v = g_state_opts.load(std::memory_order_relaxed);
-  if (v < 0) {
-    const char* e = getenv("TTL_STATE_OPTIONS");
-    v = e ? atoi(e) : 0;
-    if (v < 0 || v > 15) v = 0;
-    g_state_opts.store(v);
-  }
-  return v & 11;
-}
-
 static int launch_build_state(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
                               int n_upper, cudaStream_t s) {
   int rc = state_kernels_ready();
@@ -1378,17 +1323,20 @@ static int launch_build_state(const ttl_volume* vol, const ttl_params* prm, cons
   // the SM's 228 KB to L1, which is what dedupes the overlapping trilinear corners
   const int warp_smem = b->bf16_layout == 1 ? kWarpSmemSmall : kWarpSmemBytes;
   const int grid = ttl_div_up(n_upper, kStateWarps), smem = kStateWarps * warp_smem;
-  const int pf = state_prefetch_level() | (g_ttl_pdl.load() ? 4 : 0);
+  const int early_release = g_ttl_pdl.load() ? 1 : 0;
   if (b->bf16_layout == 1 && b->operand_fmt == TTL_OPERAND_TF32)
-    TTL_LAUNCH("build_state_kernel", s, launch_state_fmt<TTL_OPERAND_TF32>(grid, smem, s, *vol, *prm, *b, cur, warp_smem, pf));
+    TTL_LAUNCH("build_state_kernel", s,
+               launch_state_fmt<TTL_OPERAND_TF32>(grid, smem, s, *vol, *prm, *b, cur, warp_smem, early_release));
   else if (b->bf16_layout == 1 && b->operand_fmt == TTL_OPERAND_FP16)
-    TTL_LAUNCH("build_state_kernel", s, launch_state_fmt<TTL_OPERAND_FP16>(grid, smem, s, *vol, *prm, *b, cur, warp_smem, pf));
+    TTL_LAUNCH("build_state_kernel", s,
+               launch_state_fmt<TTL_OPERAND_FP16>(grid, smem, s, *vol, *prm, *b, cur, warp_smem, early_release));
   else if (b->bf16_layout == 1)
-    TTL_LAUNCH("build_state_kernel", s, launch_state_fmt<TTL_OPERAND_BF16>(grid, smem, s, *vol, *prm, *b, cur, warp_smem, pf));
+    TTL_LAUNCH("build_state_kernel", s,
+               launch_state_fmt<TTL_OPERAND_BF16>(grid, smem, s, *vol, *prm, *b, cur, warp_smem, early_release));
   else
     TTL_LAUNCH("build_state_kernel", s,
-               ttl_launch_chain(build_state_kernel<0, 1, 0>, grid, kStateWarps * 32, smem, s, *vol, *prm, *b, cur,
-                                warp_smem, (g_ttl_pdl.load() == 1 ? 4 : 0)));
+               ttl_launch_chain(build_state_kernel<0, 0>, grid, kStateWarps * 32, smem, s, *vol, *prm, *b, cur,
+                                warp_smem, early_release));
   return 0;
 }
 
@@ -1407,8 +1355,6 @@ static int check_step_args(const ttl_volume* vol, const ttl_params* prm, const t
     return TTL_ERR_BAD_ARG;
   return 0;
 }
-
-void ttl_state_options(int32_t bits) { g_state_opts.store(bits & 15); }
 
 static int env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
                     const float* actions, int32_t lda, const double* noise, const ttl_noise* nz, int defer,

@@ -10,7 +10,7 @@ Where the noise comes from (``env_dto['noise_rng']``):
   * ``'device'``: the step kernel draws it from a counter-based generator keyed by
     ``env_dto['noise_seed']`` (ttl_noise in include/ttl_b200.h): a streamline's noise at each step is a
     function of (seed, its index in the seed list, its point count) only, so the tractogram does not
-    depend on ``n_actor``, refill, the slot order, the tip sort, CUDA-graph replay or the number of GPUs.
+    depend on ``n_actor``, refill, the slot order, CUDA-graph replay or the number of GPUs.
     No host work per step, and the fused actor head and graph replay stay available.
 Neither is the reference's random stream: at noise > 0 no tractogram matches the reference's bit for bit.
 """

@@ -302,26 +302,6 @@ class TrackingEnvironment(BaseEnv):
             self._continue_idx_cache = None
         return self._batch.state[self._cur]
 
-    def resort_device(self):
-        """Re-order the alive list by tip voxel (``ttl_env_resort``) between two steps: a step without a
-        step -- the sorted list lands in the other ping-pong buffers and becomes current.  Device
-        (operand-only) mode only; per-row results are unchanged."""
-        if self._pending_harvest:
-            raise RuntimeError('resort_device() between step and harvest')
-        if self._batch.fp32_state:
-            raise _lib.TTLError('the tip sort needs the operand-only device mode (reset_streaming(fp32_state=False))')
-        n_slots = int(self._b.n_slots)
-        ws = getattr(self, '_resort_ws', None)
-        need = self._lib.ttl_env_resort_workspace_bytes(n_slots)
-        if ws is None or ws.numel() < need:
-            ws = torch.empty((need,), dtype=torch.uint8, device=self.device)
-            self._resort_ws = ws
-        _lib.check(self._lib.ttl_env_resort(ctypes.byref(self._volume), ctypes.byref(self._b), self._cur,
-                                            int(self._n_alive_host), _lib.ptr(ws), int(ws.numel()),
-                                            _lib.stream_ptr(self.device)), 'ttl_env_resort')
-        self._cur ^= 1
-        self._continue_idx_cache = None
-
     def n_alive(self):
         """Alive count after the last harvest (one 32-byte D2H copy + stream sync)."""
         bb = self._batch
