@@ -238,6 +238,40 @@ int ttl_env_step_begin_rng(const ttl_volume* vol, const ttl_params* prm, const t
 int ttl_noise_normals(const ttl_noise* nz, const int64_t* g, const int32_t* L, int32_t n, double* out,
                       void* stream);
 
+/* Stochastic policy sampled on the device (Tracker / validation_episode with prob > 0 and a policy seed).
+ * Row i of the batch, with g = row_base + i (row_base as for ttl_noise: seed_offset + start after
+ * reset / reset_streaming, 0 after nreset) and L = its point count before the step, takes for c = 0, 1, 2
+ *   eps_c = fp32_rn(z(seed, g, L, 3 + c))        z = the ttl_noise normal above, counter words 3..5
+ *   mu_c  = head output c     + bias[c]          the actor's fixed summation tree (ttl_env_step_head)
+ *   ls_c  = head output 3 + c + bias[3 + c]
+ *   std_c = expf(fminf(fmaxf(ls_c, -20.f), 2.f)) * prob
+ *   a_c   = tanhf(fmaf(std_c, eps_c, mu_c))
+ * which is the actor's own head arithmetic (MaxEntropyActor.forward, offpolicy.py:94-140) with eps_c in
+ * place of torch.randn: the fused route (ttl_env_step_head_policy) and the actor-then-step route fed by
+ * ttl_policy_eps give the same bits.  Counter words 3..5 keep eps independent of the tracking noise
+ * (words 0..2) under one seed.  At prob = 0 the action is tanh(mu) bit for bit.  Each streamline's sample
+ * depends only on (seed, g, L): not on the slot count, the alive-list order or the GPU count.  It is not
+ * torch's random stream.  Host struct read at call time; a CUDA graph captures its values. */
+typedef struct ttl_policy {
+  uint64_t seed;           /* Philox key */
+  int64_t row_base;        /* global seed index of batch row 0 */
+  float prob;              /* std scale (Tracker's prob), >= 0 */
+  int32_t pad;
+} ttl_policy;
+
+/* ttl_env_step_head with the policy sampled inside the propagate kernel: head_partial must hold all six
+ * outputs (ttl_actor_forward*_policy_partial).  nz == NULL: no device noise; non-NULL: device-drawn
+ * tracking noise added to a as ttl_env_step_head_rng does (prm->dir_f64 must be 1). */
+int ttl_env_step_head_policy(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                             const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
+                             const float* head_bias, const ttl_policy* pol, const ttl_noise* nz,
+                             int32_t n_upper, void* stream);
+/* eps [rank][ld] fp32 (ld >= 3) for every rank of alive[cur], in rank order: the draws the fused route
+ * makes, for the routes that run the actor's head on its own (ttl_actor_forward* with eps).  (row, L) come
+ * from rank_rec[cur], the alive count from ctrl[cur]; ranks beyond it are not written. */
+int ttl_policy_eps(const ttl_policy* pol, const ttl_batch* b, int32_t cur, int32_t n_upper, float* eps,
+                   int32_t ld, void* stream);
+
 /* state[cur^1][dest[r]] -> out[r] for r < n_rows: the `self.state[self.continue_idx]` that
  * step() returns, in the order of the pre-harvest alive list (tracking_env.py:217-218). */
 int ttl_env_gather_step_state(const ttl_batch* b, int32_t cur, int32_t n_rows, float* out,
@@ -336,6 +370,15 @@ int ttl_actor_forward_packed(ttl_actor_plan* plan, const void* state_op, int32_t
  * TTL_ERR_UNSUPPORTED when the plan's output layer is not fused. */
 int ttl_actor_head_partial(const ttl_actor_plan* plan, const float** partial, int32_t* n_tiles,
                            int32_t* tiles_per_256, const float** bias);
+/* ttl_actor_forward / ttl_actor_forward_packed with action == NULL for the stochastic policy: the
+ * partial sums of all six outputs (mu and log_std) stay in the plan's scratch, for
+ * ttl_env_step_head_policy.  The mu partials are the bits the deterministic call leaves.  Tensor-core
+ * tiers with the output layer fused only (else TTL_ERR_BAD_ARG / TTL_ERR_UNSUPPORTED). */
+int ttl_actor_forward_policy_partial(ttl_actor_plan* plan, const float* state, int32_t ld_state,
+                                     const int32_t* n_rows_dev, int32_t n_rows_max, void* stream);
+int ttl_actor_forward_packed_policy_partial(ttl_actor_plan* plan, const void* state_op, int32_t ld,
+                                            int32_t rows_alloc, const int32_t* n_rows_dev, int32_t n_rows_max,
+                                            int32_t layout, void* stream);
 /* fp16 tier: 1 when a state or activation value was outside +-65504 and was saturated since the last
  * clearing call (synchronises `stream`).  The caller should then re-run in tf32. */
 int ttl_actor_overflow(ttl_actor_plan* plan, int32_t* out_host, int32_t clear, void* stream);

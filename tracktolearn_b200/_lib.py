@@ -45,6 +45,11 @@ class Noise(ctypes.Structure):
     _fields_ = [('sigma', c_f64), ('seed', ctypes.c_uint64), ('row_base', c_i64)]
 
 
+class Policy(ctypes.Structure):
+    """ttl_policy: the stochastic policy sampled with counter-based draws (include/ttl_b200.h)."""
+    _fields_ = [('seed', ctypes.c_uint64), ('row_base', c_i64), ('prob', c_f32), ('pad', c_i32)]
+
+
 class ActorWeights(ctypes.Structure):
     _fields_ = [('n_layers', c_i32), ('in_dim', c_i32 * MAX_LAYERS), ('out_dim', c_i32 * MAX_LAYERS),
                 ('w', c_vp * MAX_LAYERS), ('b', c_vp * MAX_LAYERS)]
@@ -79,6 +84,9 @@ SIGNATURES = {
                                       c_vp]),
     'ttl_env_step_begin_rng': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, P(Noise), c_i32, c_vp]),
     'ttl_noise_normals': (c_i32, [P(Noise), c_vp, c_vp, c_i32, c_vp, c_vp]),
+    'ttl_env_step_head_policy': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_i32, c_vp, P(Policy),
+                                         P(Noise), c_i32, c_vp]),
+    'ttl_policy_eps': (c_i32, [P(Policy), P(Batch), c_i32, c_i32, c_vp, c_i32, c_vp]),
     'ttl_oracle_features_rows': (c_i32, [P(Batch), c_i32, c_i32, c_vp, c_vp]),
     'ttl_env_gather_step_state': (c_i32, [P(Batch), c_i32, c_i32, c_vp, c_i32, c_vp]),
     'ttl_format_state': (c_i32, [P(Volume), P(Params), c_vp, c_i32, c_i32, c_vp, c_i32, c_vp]),
@@ -96,6 +104,8 @@ SIGNATURES = {
     'ttl_actor_forward': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'ttl_actor_forward_packed': (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_i32, c_f32, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp]),
     'ttl_actor_head_partial': (c_i32, [c_vp, P(c_vp), P(c_i32), P(c_i32), P(c_vp)]),
+    'ttl_actor_forward_policy_partial': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_vp]),
+    'ttl_actor_forward_packed_policy_partial': (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_i32, c_i32, c_vp]),
     'ttl_actor_overflow': (c_i32, [c_vp, P(c_i32), c_i32, c_vp]),
     'ttl_actor_plan_set_layout': (c_i32, [c_vp, c_i32, c_i32, c_i32, c_vp]),
     'ttl_gemm_tc': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp, c_i32, c_i32, c_vp]),

@@ -19,14 +19,20 @@ class StepRunner(object):
     early.  Capturing does not execute anything: the two captures flip the env's host-side
     parity twice, so host and device stay consistent."""
 
-    def __init__(self, env, actor, prob=0.0, use_graph=True, fuse_head=True):
+    def __init__(self, env, actor, prob=0.0, use_graph=True, fuse_head=True, policy_seed=None):
         self.env, self.actor, self.prob = env, actor, prob
         self.action_buf = torch.empty((env._b.n_slots, actor.action_dim), dtype=torch.float32,
                                       device=env.device)
         # host-drawn noise arrives as an array per step: no fused head, nothing to replay.  Noise the step
         # kernel draws itself (noise_rng = 'device') needs neither restriction.
         noisy = getattr(env, 'noise', 0.0) > 0.0 and env._device_noise() is None
-        self.use_graph = bool(use_graph) and prob == 0.0 and not noisy and not env.compute_reward \
+        # prob > 0 with a policy seed: eps is a counter-based draw per (seed, seed index, point count)
+        # (ttl_policy), made inside the step kernel on the fused route and by ttl_policy_eps otherwise; no
+        # host input either way.  Without a seed: torch.randn per step, as the reference does.
+        self.policy_seed = policy_seed if prob != 0.0 else None
+        self.eps_buf = None
+        keyed = prob == 0.0 or self.policy_seed is not None
+        self.use_graph = bool(use_graph) and keyed and not noisy and not env.compute_reward \
             and env._oracle is None
         self.graphs = None
         self.warm = 0
@@ -35,22 +41,33 @@ class StepRunner(object):
         self._lib = __import__('tracktolearn_b200._lib', fromlist=['load']).load()
         # deterministic tracking: the env step reads tanh(mu) straight from the actor's fused output
         # layer (one launch and one HBM round trip less per step; same bits)
-        self.fuse_head = prob == 0.0 and not noisy and env._oracle is None and fuse_head \
+        self.fuse_head = keyed and not noisy and env._oracle is None and fuse_head \
             and hasattr(actor, 'forward_head_partial')
 
     def _one(self, rows):
         env = self.env
+        sampled = self.policy_seed is not None
+        # the batch's row_base is read when the launch is made (a captured graph holds it by value)
+        pol = env.policy(self.policy_seed, self.prob) if sampled else None
         if self.fuse_head:
             head = self.actor.forward_head_partial(env.current_state_bf16(), rows,
                                                    n_rows_dev=env.alive_count_tensor(), layout=env.bf16_layout,
-                                                   state=env.current_state())
+                                                   state=env.current_state(), policy=sampled)
             if head is not None:
-                env.step_device_head(head)
+                if sampled:
+                    env.step_device_head_policy(head, pol)
+                else:
+                    env.step_device_head(head)
                 env.harvest_device()
                 return
             self.fuse_head = False
+        eps = None
+        if sampled:
+            if self.eps_buf is None:
+                self.eps_buf = torch.empty_like(self.action_buf)
+            eps = env.policy_eps(pol, self.eps_buf)
         self.actor.forward_device(env.current_state(), self.prob, n_rows_dev=env.alive_count_tensor(),
-                                  n_rows=rows, want_logp=False, out_action=self.action_buf,
+                                  n_rows=rows, eps=eps, want_logp=False, out_action=self.action_buf,
                                   state_bf16=env.current_state_bf16(), layout=env.bf16_layout)
         env.step_device(self.action_buf)
         env.harvest_device()
@@ -116,28 +133,35 @@ class RLAlgorithm(object):
         self._runner = None
         self._runner_key = None
 
-    def _runner_for(self, env, actor, prob, use_graph):
+    def _runner_for(self, env, actor, prob, use_graph, policy_seed=None):
         """The captured graphs hold raw pointers into the env's batch buffers and the actor's plan:
         keep one runner per (buffers, plan) and reuse it across episodes."""
-        nz = env._device_noise()      # a captured graph holds the noise parameters by value
+        nz = env._device_noise()      # a captured graph holds the noise and policy parameters by value
+        sampled = prob != 0.0 and policy_seed is not None
         key = (id(env), id(env._batch), env._b.n_slots, env._batch.fp32_state, id(actor), id(actor._plan), prob,
                bool(use_graph), bool(getattr(self, 'fuse_head', True)),
-               None if nz is None else (nz.sigma, nz.seed, nz.row_base))
+               None if nz is None else (nz.sigma, nz.seed, nz.row_base),
+               (int(policy_seed), int(env._row_base)) if sampled else None)
         if getattr(self, '_runner_key', None) != key or self._runner is None:
             self._runner = StepRunner(env, actor, prob, use_graph=use_graph,
-                                      fuse_head=getattr(self, 'fuse_head', True))
+                                      fuse_head=getattr(self, 'fuse_head', True),
+                                      policy_seed=policy_seed if sampled else None)
             self._runner_key = key
         elif self._runner.graphs is not None:
             env_cur = env._cur          # graphs were captured for both parities; nothing to redo
             assert env_cur in self._runner.graphs
         return self._runner
 
-    def validation_episode(self, initial_state, env, prob=1., max_steps=None):
+    def validation_episode(self, initial_state, env, prob=1., max_steps=None, policy_seed=None):
         """Run the agent until every streamline of the env's current batch is done.
 
         Reference: algorithms/rl.py:58-106.  ``initial_state`` is accepted for signature
         compatibility; the state rows are read from the env's device buffers.  Returns the
-        cumulative reward (0 when the env does not compute rewards)."""
+        cumulative reward (0 when the env does not compute rewards).
+        ``policy_seed`` (prob > 0): eps of the stochastic policy is a counter-based draw per (seed, seed
+        index, point count) made on the device (ttl_policy) instead of torch.randn, so each streamline's
+        samples do not depend on how the episode is scheduled and the fused head and graph replay stay
+        available."""
         actor = self.agent.actor
         running_reward = 0
         reward_acc = None
@@ -146,7 +170,7 @@ class RLAlgorithm(object):
             return running_reward
         # graphs pay off when the launch shapes are stable: the streaming tracker
         streaming = bool(env._params.refill)
-        runner = self._runner_for(env, actor, prob, self.use_cuda_graph and streaming)
+        runner = self._runner_for(env, actor, prob, self.use_cuda_graph and streaming, policy_seed)
         bb = env._batch
         stream = torch.cuda.current_stream(env.device)
         pending = []          # (event, pinned ctrl snapshot, parity the snapshot describes)

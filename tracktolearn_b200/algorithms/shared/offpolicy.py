@@ -214,12 +214,14 @@ class MaxEntropyActor(object):
         self._keep = (state, eps)
         return action, logp, pre
 
-    def forward_head_partial(self, state_bf16, n_rows, n_rows_dev=None, layout=None, state=None):
+    def forward_head_partial(self, state_bf16, n_rows, n_rows_dev=None, layout=None, state=None, policy=False):
         """Deterministic policy (prob = 0) for the device loop: runs the tensor-core layers over the
         env's operand rows (or, when their element type is not this actor's, over ``state``: the fp32 rows,
         packed first) and leaves the 6-wide output layer as per-tile partial sums in the plan's scratch.
         Returns (partial_ptr, n_tiles, tiles_per_256, bias_ptr) for ``env.step_device_head``, or None when
-        this actor cannot do it (fp32 tier, output layer not fused, no usable rows)."""
+        this actor cannot do it (fp32 tier, output layer not fused, no usable rows).
+        ``policy=True``: the partials of all six outputs (mu and log_std) for the stochastic policy that
+        ``env.step_device_head_policy`` samples; the mu partials are the same bits."""
         packed = self._operand_matches(state_bf16)
         if self.precision not in self._OPERAND_DTYPES or (not packed and state is None):
             return None
@@ -241,16 +243,27 @@ class MaxEntropyActor(object):
                         self._plan, int(layout[1]), int(layout[2]), int(layout[3]),
                         _lib.stream_ptr(self.device)), 'ttl_actor_plan_set_layout')
                     self._plan_layout = tuple(layout)
-            _lib.check(self._lib.ttl_actor_forward_packed(
-                self._plan, _lib.ptr(state_bf16), int(state_bf16.stride(0)), int(state_bf16.shape[0]),
-                _lib.ptr(n_rows_dev), rows, 0.0, None, None, None, None, lay,
-                _lib.stream_ptr(self.device)), 'ttl_actor_forward_packed')
+            if policy:
+                _lib.check(self._lib.ttl_actor_forward_packed_policy_partial(
+                    self._plan, _lib.ptr(state_bf16), int(state_bf16.stride(0)), int(state_bf16.shape[0]),
+                    _lib.ptr(n_rows_dev), rows, lay, _lib.stream_ptr(self.device)),
+                    'ttl_actor_forward_packed_policy_partial')
+            else:
+                _lib.check(self._lib.ttl_actor_forward_packed(
+                    self._plan, _lib.ptr(state_bf16), int(state_bf16.stride(0)), int(state_bf16.shape[0]),
+                    _lib.ptr(n_rows_dev), rows, 0.0, None, None, None, None, lay,
+                    _lib.stream_ptr(self.device)), 'ttl_actor_forward_packed')
             self._keep = (state_bf16, None)
         elif rows > 0:
             ld = state.stride(0) if state.shape[0] > 1 else state.shape[1]
-            _lib.check(self._lib.ttl_actor_forward(
-                self._plan, _lib.ptr(state), int(ld), _lib.ptr(n_rows_dev), rows, 0.0, None, None, None, None,
-                _lib.stream_ptr(self.device)), 'ttl_actor_forward')
+            if policy:
+                _lib.check(self._lib.ttl_actor_forward_policy_partial(
+                    self._plan, _lib.ptr(state), int(ld), _lib.ptr(n_rows_dev), rows,
+                    _lib.stream_ptr(self.device)), 'ttl_actor_forward_policy_partial')
+            else:
+                _lib.check(self._lib.ttl_actor_forward(
+                    self._plan, _lib.ptr(state), int(ld), _lib.ptr(n_rows_dev), rows, 0.0, None, None, None, None,
+                    _lib.stream_ptr(self.device)), 'ttl_actor_forward')
             self._keep = (state, None)
         query()                   # the geometry of the partials depends on the launch just made
         return partial.value, int(n_tiles.value), int(per256.value), bias.value

@@ -511,7 +511,7 @@ void pack_weights(ttl_actor_plan* p, cudaStream_t s) {
 // map_a0: TMA map of the first layer's operand rows [rows][k_pad[0]].
 int run_tc_layers(ttl_actor_plan* p, const CUtensorMap& map_a0, const int32_t* n_rows_dev, int32_t n_rows_max,
                   float probabilistic, const float* eps, float* action, float* logp, float* pre, cudaStream_t s,
-                  bool alt_w0 = false) {
+                  bool alt_w0 = false, bool policy_partial = false) {
   const ttl_actor_weights& w = p->w;
   const int nl = w.n_layers, nh = nl - 1;     // nh tensor-core layers
   const int n_out = w.out_dim[nl - 1], k_last = w.in_dim[nl - 1];
@@ -519,8 +519,9 @@ int run_tc_layers(ttl_actor_plan* p, const CUtensorMap& map_a0, const int32_t* n
   for (int i = 0; i < nh; ++i) max_np = p->n_pad[i] > max_np ? p->n_pad[i] : max_np;
   const int bn = choose_bn(n_rows_max, max_np);
   const int bi = bn_index(bn);
-  // only mu is needed when nothing reads log_std: deterministic policy, no log-prob, no raw output
-  const int head_n = (p->fuse_head && probabilistic == 0.f && !logp && !pre) ? n_out / 2 : n_out;
+  // only mu is needed when nothing reads log_std: deterministic policy, no log-prob, no raw output, no
+  // sampling in the env step (policy_partial)
+  const int head_n = (p->fuse_head && probabilistic == 0.f && !logp && !pre && !policy_partial) ? n_out / 2 : n_out;
 
   auto fill_layer = [&](MlpMaps& maps, MlpArgs& a, int slot, int i) {
     maps.a[slot] = i == 0 ? map_a0 : p->map_a[i];
@@ -602,6 +603,38 @@ int run_tc_layers(ttl_actor_plan* p, const CUtensorMap& map_a0, const int32_t* n
           n_rows_max, probabilistic, eps, action, logp, pre));
   }
   TTL_CHECK_LAST();
+  return 0;
+}
+
+// fp32 state rows -> the plan's first-layer operand rows (ttl_actor_forward on the tensor-core tiers)
+void pack_state(ttl_actor_plan* p, const float* state, int ld_state, const int32_t* n_rows_dev, int n_rows_max,
+                cudaStream_t s) {
+  const long long tot = (long long)n_rows_max * (p->k_pad[0] >> 2);
+  const int grid = ttl_div_up(tot, 256);
+  const int width = p->w.in_dim[0];
+  if (p->kind == KIND_BF16)
+    TTL_LAUNCH("pack_state_kernel", s, pack_state_kernel<KIND_BF16><<<grid, 256, 0, s>>>(
+        state, ld_state, width, n_rows_dev, n_rows_max, p->act_in, p->k_pad[0], p->overflow));
+  else if (p->kind == KIND_F16)
+    TTL_LAUNCH("pack_state_kernel", s, pack_state_kernel<KIND_F16><<<grid, 256, 0, s>>>(
+        state, ld_state, width, n_rows_dev, n_rows_max, p->act_in, p->k_pad[0], p->overflow));
+  else
+    TTL_LAUNCH("pack_state_kernel", s, pack_state_kernel<KIND_TF32><<<grid, 256, 0, s>>>(
+        state, ld_state, width, n_rows_dev, n_rows_max, p->act_in, p->k_pad[0], p->overflow));
+}
+
+// TMA map of caller-owned operand rows (ttl_actor_forward_packed), cached per (pointer, rows)
+int ext_map(ttl_actor_plan* p, const void* state_op, int ld, int rows_alloc, const CUtensorMap** out) {
+  for (auto& e : p->ext_maps)
+    if (e.ptr == state_op && e.rows == rows_alloc) { *out = &e.map; return 0; }
+  if (p->ext_maps.size() >= 16) p->ext_maps.clear();
+  ttl_actor_plan::ExtMap e;
+  e.ptr = state_op;
+  e.rows = rows_alloc;
+  int rc = make_tmap(&e.map, p->kind, state_op, (uint64_t)rows_alloc, (uint64_t)ld, MLP_BM);
+  if (rc) return rc;
+  p->ext_maps.push_back(e);
+  *out = &p->ext_maps.back().map;
   return 0;
 }
 }  // namespace
@@ -688,17 +721,7 @@ int ttl_actor_forward(ttl_actor_plan* p, const float* state, int32_t ld_state, c
   const int n_out = w.out_dim[nl - 1], k_last = w.in_dim[nl - 1];
 
   if (p->kind >= 0) {
-    const long long tot = (long long)n_rows_max * (p->k_pad[0] >> 2);
-    const int grid = ttl_div_up(tot, 256);
-    if (p->kind == KIND_BF16)
-      TTL_LAUNCH("pack_state_kernel", s, pack_state_kernel<KIND_BF16><<<grid, 256, 0, s>>>(
-          state, ld_state, w.in_dim[0], n_rows_dev, n_rows_max, p->act_in, p->k_pad[0], p->overflow));
-    else if (p->kind == KIND_F16)
-      TTL_LAUNCH("pack_state_kernel", s, pack_state_kernel<KIND_F16><<<grid, 256, 0, s>>>(
-          state, ld_state, w.in_dim[0], n_rows_dev, n_rows_max, p->act_in, p->k_pad[0], p->overflow));
-    else
-      TTL_LAUNCH("pack_state_kernel", s, pack_state_kernel<KIND_TF32><<<grid, 256, 0, s>>>(
-          state, ld_state, w.in_dim[0], n_rows_dev, n_rows_max, p->act_in, p->k_pad[0], p->overflow));
+    pack_state(p, state, ld_state, n_rows_dev, n_rows_max, s);
     return run_tc_layers(p, p->map_a[0], n_rows_dev, n_rows_max, probabilistic, eps, action, logp, pre, s);
   }
   // Reference-precision tier; needs the row count on the host.
@@ -750,20 +773,36 @@ int ttl_actor_forward_packed(ttl_actor_plan* p, const void* state_op, int32_t ld
   if (probabilistic != 0.f && !eps) return TTL_ERR_BAD_ARG;
   if (n_rows_max <= 0) return 0;
   const CUtensorMap* map = nullptr;
-  for (auto& e : p->ext_maps)
-    if (e.ptr == state_op && e.rows == rows_alloc) map = &e.map;
-  if (!map) {
-    if (p->ext_maps.size() >= 16) p->ext_maps.clear();
-    ttl_actor_plan::ExtMap e;
-    e.ptr = state_op;
-    e.rows = rows_alloc;
-    int rc = make_tmap(&e.map, p->kind, state_op, (uint64_t)rows_alloc, (uint64_t)ld, MLP_BM);
-    if (rc) return rc;
-    p->ext_maps.push_back(e);
-    map = &p->ext_maps.back().map;
-  }
+  int rc = ext_map(p, state_op, ld, rows_alloc, &map);
+  if (rc) return rc;
   return run_tc_layers(p, *map, n_rows_dev, n_rows_max, probabilistic, eps, action, logp, pre,
                        (cudaStream_t)stream, layout == 1);
+}
+
+int ttl_actor_forward_policy_partial(ttl_actor_plan* p, const float* state, int32_t ld_state,
+                                     const int32_t* n_rows_dev, int32_t n_rows_max, void* stream) {
+  if (!p || !state || p->kind < 0 || n_rows_max > p->max_rows) return TTL_ERR_BAD_ARG;
+  if (!p->fuse_head) return TTL_ERR_UNSUPPORTED;
+  if (n_rows_max <= 0) return 0;
+  cudaStream_t s = (cudaStream_t)stream;
+  pack_state(p, state, ld_state, n_rows_dev, n_rows_max, s);
+  return run_tc_layers(p, p->map_a[0], n_rows_dev, n_rows_max, 0.f, nullptr, nullptr, nullptr, nullptr, s,
+                       false, true);
+}
+
+int ttl_actor_forward_packed_policy_partial(ttl_actor_plan* p, const void* state_op, int32_t ld,
+                                            int32_t rows_alloc, const int32_t* n_rows_dev, int32_t n_rows_max,
+                                            int32_t layout, void* stream) {
+  if (!p || !state_op || p->kind < 0 || n_rows_max > p->max_rows || n_rows_max > rows_alloc) return TTL_ERR_BAD_ARG;
+  if (!p->fuse_head) return TTL_ERR_UNSUPPORTED;
+  if (layout != 0 && !(layout == 1 && p->has_alt)) return TTL_ERR_BAD_ARG;
+  if (ld != p->k_pad[0] || (reinterpret_cast<uintptr_t>(state_op) & 15)) return TTL_ERR_BAD_ARG;
+  if (n_rows_max <= 0) return 0;
+  const CUtensorMap* map = nullptr;
+  int rc = ext_map(p, state_op, ld, rows_alloc, &map);
+  if (rc) return rc;
+  return run_tc_layers(p, *map, n_rows_dev, n_rows_max, 0.f, nullptr, nullptr, nullptr, nullptr,
+                       (cudaStream_t)stream, layout == 1, true);
 }
 
 int ttl_actor_head_partial(const ttl_actor_plan* p, const float** partial, int32_t* n_tiles,

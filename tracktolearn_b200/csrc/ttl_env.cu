@@ -387,10 +387,14 @@ struct ActionSrc {
 // Where the noise comes from.  RNG = false: the optional host-drawn array `noise` [n_alive][3] per rank.
 // RNG = true (dir_f64 only): drawn here from the counter-based generator (ttl_rng.cuh) at
 // (nz.seed, nz.row_base + row, L); lanes 0-2 of the quad draw one component each and share them.
-template <bool RNG>
-__global__ void __launch_bounds__(kK1Threads, 6) propagate_stop_kernel(
+// POLICY = true (head partials only): the stochastic policy is sampled here (ttl_policy): lane c < 3 of
+// the quad sums its own mu_c and log_std_c, draws eps_c at (pol.seed, pol.row_base + row, L) and forms
+// a_c with head_finish_kernel's arithmetic; the quad shares the three components.  (The arguments are taken
+// by value: with references the RNG build of propagate_stop_kernel allocated its registers differently.)
+template <bool RNG, bool POLICY>
+__device__ __forceinline__ void propagate_stop_body(
     ttl_volume v, ttl_params prm, ttl_batch b, int cur, ActionSrc src,
-    const double* __restrict__ noise, int defer, ttl_noise nz) {
+    const double* __restrict__ noise, int defer, ttl_noise nz, ttl_policy pol) {
   // 4 lanes per streamline: they redo the cheap scalar work together and split the spline taps
   const int lane = threadIdx.x & 31, sub = threadIdx.x & (kLanesPerRow - 1);
   const unsigned quad_mask = 0xFu << (lane & ~(kLanesPerRow - 1));
@@ -402,7 +406,12 @@ __global__ void __launch_bounds__(kK1Threads, 6) propagate_stop_kernel(
   const int r_ld = min(r, src.n_rows - 1);
   const RankRec rec = read_rank_rec(b.rank_rec[cur], r_ld);
   float ax = 0.f, ay = 0.f, az = 0.f;
-  if (src.partial) {
+  float pmu = 0.f, pls = 0.f;   // POLICY: this lane's partial sums of mu_c and log_std_c
+  if constexpr (POLICY) {
+    const float* prow = src.partial + (size_t)r_ld * src.n_tiles * 8;
+    pmu = ttl_head_tree_sum(prow, src.n_tiles, src.tiles_per_256, min(sub, 2));
+    pls = ttl_head_tree_sum(prow, src.n_tiles, src.tiles_per_256, 3 + min(sub, 2));
+  } else if (src.partial) {
     ttl_head_tree_sum3(src.partial + (size_t)r_ld * src.n_tiles * 8, src.n_tiles, src.tiles_per_256, ax, ay, az);
   } else {
     ax = src.actions[(size_t)r_ld * src.lda + 0];
@@ -412,13 +421,25 @@ __global__ void __launch_bounds__(kK1Threads, 6) propagate_stop_kernel(
   const int n_alive = b.ctrl[cur];
   int stopped = 0;
   if (r < n_alive) {
-  if (src.partial) {
+  if (!POLICY && src.partial) {
     ax = tanhf(ax + __ldg(src.bias + 0));
     ay = tanhf(ay + __ldg(src.bias + 1));
     az = tanhf(az + __ldg(src.bias + 2));
   }
   const int i = rec.row;
   const int L = rec.L;  // points so far in this row
+  if constexpr (POLICY) {
+    // head_finish_kernel (ttl_actor.cu), operation for operation, with eps_c drawn here
+    const int c = min(sub, 2);
+    const float mu = pmu + __ldg(src.bias + c);
+    const float ls = pls + __ldg(src.bias + 3 + c);
+    const float sd = expf(fminf(fmaxf(ls, -20.f), 2.f)) * pol.prob;
+    const float a = tanhf(fmaf(sd, ttl_policy_eps(pol.seed, pol.row_base + i, L, c), mu));
+    const int qb = lane & ~(kLanesPerRow - 1);
+    ax = __shfl_sync(quad_mask, a, qb + 0);
+    ay = __shfl_sync(quad_mask, a, qb + 1);
+    az = __shfl_sync(quad_mask, a, qb + 2);
+  }
   float* P = b.points + (size_t)i * b.max_pts * 3;
   const float px = rec.tx, py = rec.ty, pz = rec.tz;
 
@@ -502,6 +523,32 @@ __global__ void __launch_bounds__(kK1Threads, 6) propagate_stop_kernel(
   }  // r < n_alive
 
   if (!(defer & 1)) publish_stops(b, cur, stopped);
+}
+
+template <bool RNG>
+__global__ void __launch_bounds__(kK1Threads, 6) propagate_stop_kernel(
+    ttl_volume v, ttl_params prm, ttl_batch b, int cur, ActionSrc src,
+    const double* __restrict__ noise, int defer, ttl_noise nz) {
+  propagate_stop_body<RNG, false>(v, prm, b, cur, src, noise, defer, nz, ttl_policy{0, 0, 0.f, 0});
+}
+
+// The fused-head step with the stochastic policy sampled in the kernel (ttl_env_step_head_policy);
+// NOISE: device-drawn tracking noise on top (dir_f64 only).  Never deferred: no oracle on this route.
+template <bool NOISE>
+__global__ void __launch_bounds__(kK1Threads, 6) propagate_policy_kernel(
+    ttl_volume v, ttl_params prm, ttl_batch b, int cur, ActionSrc src, ttl_noise nz, ttl_policy pol) {
+  propagate_stop_body<NOISE, true>(v, prm, b, cur, src, nullptr, 0, nz, pol);
+}
+
+// ttl_policy_eps: one thread per (rank, component) of alive[cur]
+__global__ void policy_eps_kernel(ttl_policy pol, ttl_batch b, int cur, int n_upper, float* __restrict__ eps,
+                                  int ld) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= 3LL * n_upper) return;
+  const int r = (int)(t / 3), c = (int)(t % 3);
+  if (r >= b.ctrl[cur]) return;
+  const RankRec rec = read_rank_rec(b.rank_rec[cur], r);
+  eps[(size_t)r * ld + c] = ttl_policy_eps(pol.seed, pol.row_base + rec.row, rec.L, c);
 }
 
 // ttl_noise_normals: one thread per (row, component)
@@ -1295,6 +1342,12 @@ static void launch_propagate_as(const ttl_volume* vol, const ttl_params* prm, co
                                 int grid, cudaStream_t s) {
   TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
 }
+template <bool NOISE>
+static void launch_policy_as(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
+                             const ActionSrc& src, const ttl_noise& nz, const ttl_policy& pol, int grid,
+                             cudaStream_t s) {
+  TTL_LAUNCH("propagate_policy_kernel", s, ttl_launch_chain(propagate_policy_kernel<NOISE>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, nz, pol));
+}
 }  // extern "C++"
 
 // nz != NULL: the noise is drawn in the kernel (ttl_noise) and `noise` must be NULL
@@ -1306,6 +1359,22 @@ static void launch_propagate(const ttl_volume* vol, const ttl_params* prm, const
     launch_propagate_as<true>(vol, prm, b, cur, src, nullptr, defer, *nz, grid, s);
   else
     launch_propagate_as<false>(vol, prm, b, cur, src, noise, defer, ttl_noise{0.0, 0, 0}, grid, s);
+}
+
+// nz != NULL: device-drawn noise on top of the sampled policy
+static void launch_propagate_policy(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
+                                    const ActionSrc& src, const ttl_policy& pol, const ttl_noise* nz,
+                                    int n_upper, cudaStream_t s) {
+  const int grid = ttl_div_up(n_upper, kGroup);
+  if (nz)
+    launch_policy_as<true>(vol, prm, b, cur, src, *nz, pol, grid, s);
+  else
+    launch_policy_as<false>(vol, prm, b, cur, src, ttl_noise{0.0, 0, 0}, pol, grid, s);
+}
+
+static int check_policy(const ttl_policy* pol) {
+  if (!pol || !(pol->prob >= 0.f) || isinf(pol->prob)) return TTL_ERR_BAD_ARG;
+  return 0;
 }
 
 // the device-noise entry points need the float64 direction arithmetic the noise is defined in
@@ -1373,9 +1442,10 @@ static int env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batc
   return 0;
 }
 
+// pol != NULL: the stochastic policy is sampled in the propagate kernel (propagate_policy_kernel)
 static int env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
                          const float* head_partial, int32_t n_tiles, int32_t tiles_per_256, const float* head_bias,
-                         const ttl_noise* nz, int32_t n_upper, cudaStream_t s) {
+                         const ttl_noise* nz, int32_t n_upper, cudaStream_t s, const ttl_policy* pol = nullptr) {
   if (n_upper <= 0) return 0;
   if (!head_partial || !head_bias || n_tiles < 1 || (reinterpret_cast<uintptr_t>(head_partial) & 15) ||
       (tiles_per_256 != 1 && tiles_per_256 != 2 && tiles_per_256 != 4))
@@ -1383,7 +1453,10 @@ static int env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl
   int rc = check_step_args(vol, prm, b, cur, &n_upper);
   if (rc) return rc;
   const ActionSrc src = {nullptr, 0, head_partial, n_tiles, tiles_per_256, head_bias, n_upper};
-  launch_propagate(vol, prm, b, cur, src, nullptr, 0, n_upper, s, nz);
+  if (pol)
+    launch_propagate_policy(vol, prm, b, cur, src, *pol, nz, n_upper, s);
+  else
+    launch_propagate(vol, prm, b, cur, src, nullptr, 0, n_upper, s, nz);
   rc = launch_build_state(vol, prm, b, cur, n_upper, s);
   if (rc) return rc;
   TTL_CHECK_LAST();
@@ -1431,6 +1504,33 @@ int ttl_env_step_begin_rng(const ttl_volume* vol, const ttl_params* prm, const t
   int rc = check_noise(prm, nz);
   if (rc) return rc;
   return env_step(vol, prm, b, cur, actions, lda, nullptr, nz, 1, n_upper, (cudaStream_t)stream);
+}
+
+int ttl_env_step_head_policy(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                             const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
+                             const float* head_bias, const ttl_policy* pol, const ttl_noise* nz, int32_t n_upper,
+                             void* stream) {
+  int rc = check_policy(pol);
+  if (rc) return rc;
+  if (nz) {
+    rc = check_noise(prm, nz);
+    if (rc) return rc;
+  }
+  return env_step_head(vol, prm, b, cur, head_partial, n_tiles, tiles_per_256, head_bias, nz, n_upper,
+                       (cudaStream_t)stream, pol);
+}
+
+int ttl_policy_eps(const ttl_policy* pol, const ttl_batch* b, int32_t cur, int32_t n_upper, float* eps, int32_t ld,
+                   void* stream) {
+  if (!pol || !b || (cur != 0 && cur != 1) || !b->ctrl || !b->rank_rec[cur]) return TTL_ERR_BAD_ARG;
+  if (n_upper > b->n_slots) n_upper = b->n_slots;
+  if (n_upper <= 0) return 0;
+  if (!eps || ld < 3) return TTL_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  TTL_LAUNCH("policy_eps_kernel", s,
+             policy_eps_kernel<<<ttl_div_up((long long)n_upper * 3, 256), 256, 0, s>>>(*pol, *b, cur, n_upper, eps, ld));
+  TTL_CHECK_LAST();
+  return 0;
 }
 
 int ttl_noise_normals(const ttl_noise* nz, const int64_t* g, const int32_t* L, int32_t n, double* out,

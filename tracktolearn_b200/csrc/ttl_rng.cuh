@@ -39,3 +39,9 @@ __device__ __forceinline__ double ttl_noise_normal(unsigned long long seed, long
   const double u1 = ttl_open_unit(w.x, w.y), u2 = ttl_open_unit(w.z, w.w);
   return __dmul_rn(__dsqrt_rn(__dmul_rn(-2.0, log(u1))), cospi(__dmul_rn(2.0, u2)));
 }
+
+// eps_c of the stochastic policy (ttl_policy, include/ttl_b200.h): counter words 3..5, so that it is
+// independent of the tracking noise (words 0..2) under the same seed; rounded once to fp32
+__device__ __forceinline__ float ttl_policy_eps(unsigned long long seed, long long g, int L, int c) {
+  return (float)ttl_noise_normal(seed, g, L, 3 + c);
+}

@@ -42,10 +42,6 @@ class NoisyTrackingEnvironment(TrackingEnvironment):
             self.noise_seed = int(self.noise_seed)
             if not 0 <= self.noise_seed < 1 << 64:
                 raise ValueError('noise_seed must be in [0, 2**64), not %d' % self.noise_seed)
-        # Device noise: global index of seeds[0] in the seed list the whole run shares.  Tracker.track_to_file
-        # sets it when it shards the seeds over processes; 0 otherwise.
-        self.seed_offset = 0
-        self._row_base = 0
         self.max_action = 1.
         self._float64_directions = True
         super().__init__(dataset_file, split_id, env_dto)
@@ -54,22 +50,8 @@ class NoisyTrackingEnvironment(TrackingEnvironment):
         super().load_subject()
         self._params.dir_f64 = 1
 
-    # Device noise is keyed by g = row_base + batch row: reset / reset_streaming(start, end) use
-    # row_base = seed_offset + start, so a seed keeps its index whichever pass or shard tracks it.
-    def reset(self, start, end):
-        self._row_base = int(self.seed_offset) + int(start)
-        return super().reset(start, end)
-
-    def reset_streaming(self, start, end, n_slots, fp32_state=True, locality=True, operand=None):
-        self._row_base = int(self.seed_offset) + int(start)
-        return super().reset_streaming(start, end, n_slots, fp32_state=fp32_state, locality=locality,
-                                       operand=operand)
-
-    def nreset(self, n_seeds):
-        """Random seeds with replacement: the rows are not seed-list indices, so device noise uses
-        row_base = 0 (row i of the batch is g = i)."""
-        self._row_base = 0
-        return super().nreset(n_seeds)
+    # Device noise is keyed by g = row_base + batch row, with seed_offset / row_base kept by
+    # TrackingEnvironment (reset, reset_streaming, nreset), which keys the stochastic policy the same way.
 
     def _device_noise(self):
         if self.noise_rng != 'device':

@@ -135,6 +135,14 @@ class _BatchBuffers(object):
 class TrackingEnvironment(BaseEnv):
     """Reference: environments/tracking_env.py:13."""
 
+    # Counter-based draws made on the device (the stochastic policy, ttl_policy; device tracking noise,
+    # ttl_noise) are keyed by g = row_base + batch row.  ``seed_offset``: global index of seeds[0] in the seed
+    # list the whole run shares (Tracker.track_to_file sets it when it shards the seeds over processes).
+    # reset / reset_streaming(start, end) use row_base = seed_offset + start, so a seed keeps its index
+    # whichever pass or shard tracks it; nreset uses 0.
+    seed_offset = 0
+    _row_base = 0
+
     # ------------------------------------------------------------------------------ reset
     def _ensure_buffers(self, rows, slots, fp32_state=True, operand='bf16'):
         need_pts = self.max_nb_steps + 1
@@ -202,6 +210,7 @@ class TrackingEnvironment(BaseEnv):
 
     def reset(self, start, end):
         """Reference: tracking_env.py:91-133."""
+        self._row_base = int(self.seed_offset) + int(start)
         return self._start(self.seeds[start:end])
 
     def reset_streaming(self, start, end, n_slots, fp32_state=True, locality=True, operand=None):
@@ -213,11 +222,14 @@ class TrackingEnvironment(BaseEnv):
         neighbours in the alive list start in the same or adjacent voxels and their trilinear
         gathers share cache lines (the reference shuffles the seeds, tracker.py:94; the rows -- and
         with them every per-seed result and the output order -- stay in the shuffled order)."""
+        self._row_base = int(self.seed_offset) + int(start)
         return self._start(self.seeds[start:end], n_slots=n_slots, fp32_state=fp32_state,
                            locality=locality and os.environ.get('TTL_LOCALITY', '1') != '0', operand=operand)
 
     def nreset(self, n_seeds):
-        """Reference: tracking_env.py:47-89."""
+        """Reference: tracking_env.py:47-89.  Random seeds with replacement: the rows are not seed-list
+        indices, so device draws use row_base = 0 (row i of the batch is g = i)."""
+        self._row_base = 0
         replace = n_seeds > len(self.seeds)
         seeds = np.random.choice(np.arange(len(self.seeds)), size=n_seeds, replace=replace)
         return self._start(self.seeds[seeds])
@@ -293,6 +305,41 @@ class TrackingEnvironment(BaseEnv):
                                                        _lib.stream_ptr(self.device)), 'ttl_env_step_head_rng')
         self.length += 1
         self._pending_harvest = True
+
+    def policy(self, seed, prob):
+        """``_lib.Policy`` for the current batch: the stochastic policy with std scaled by ``prob``, its eps
+        drawn from ``seed`` at (row_base + batch row, point count) -- ttl_policy in include/ttl_b200.h."""
+        return _lib.Policy(seed=int(seed), row_base=int(self._row_base), prob=float(prob))
+
+    def step_device_head_policy(self, head, policy):
+        """``step_device_head`` with the policy sampled inside the step kernel (ttl_env_step_head_policy):
+        ``head`` must hold all six outputs (``actor.forward_head_partial(..., policy=True)``); device-drawn
+        tracking noise, if any, is added on top.  Same bits as ``policy_eps`` + the actor's head + step."""
+        if self._pending_harvest:
+            raise RuntimeError('step() called twice without harvest()')
+        if self._oracle is not None:
+            raise RuntimeError('step_device_head_policy does not consult the oracle; use step_device')
+        if getattr(self, 'noise', 0.0) > 0.0 and self._device_noise() is None:
+            raise RuntimeError('host-drawn noise arrives as an array: use policy_eps and step_device')
+        partial, n_tiles, tiles_per_256, bias = head
+        nz = self._device_noise()
+        _lib.check(self._lib.ttl_env_step_head_policy(
+            ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur, partial,
+            int(n_tiles), int(tiles_per_256), bias, ctypes.byref(policy), None if nz is None else ctypes.byref(nz),
+            int(self._n_alive_host), _lib.stream_ptr(self.device)), 'ttl_env_step_head_policy')
+        self.length += 1
+        self._pending_harvest = True
+
+    def policy_eps(self, policy, out):
+        """Enqueue ttl_policy_eps: ``out`` (CUDA float32 [>= n_alive, >= 3], row stride from the tensor)
+        gets, rank by rank of the current alive list, the eps the fused route would draw -- for
+        ``actor.forward_device(..., eps=out)``."""
+        if out.dtype != torch.float32 or out.device != self.device or out.stride(-1) != 1 or out.dim() != 2:
+            raise ValueError('policy_eps writes a CUDA float32 [rows, >= 3] tensor on the env device')
+        _lib.check(self._lib.ttl_policy_eps(ctypes.byref(policy), ctypes.byref(self._b), self._cur,
+                                            int(self._n_alive_host), _lib.ptr(out), int(out.stride(0)),
+                                            _lib.stream_ptr(self.device)), 'ttl_policy_eps')
+        return out
 
     def harvest_device(self):
         """The flip that makes the compacted alive list / state rows current (harvest)."""

@@ -40,6 +40,7 @@ class TrackToLearnTrack(object):
         self.out_tractogram = track_dto['out_tractogram']
         self.noise = track_dto['noise']
         self.noise_rng = track_dto.get('noise_rng', 'host')
+        self.policy_prob = float(track_dto.get('policy_prob') or 0.0)
         self.binary_stopping_threshold = track_dto['binary_stopping_threshold']
         self.n_actor = track_dto['n_actor']
         self.npv = track_dto['npv']
@@ -115,8 +116,10 @@ class TrackToLearnTrack(object):
         alg = algs[self.algorithm](self.input_size, self.action_size, self.hidden_dims, n_actors=self.n_actor,
                                    rng=self.rng, device=self.device, precision=self.precision)
         alg.agent.load(self.agent, 'last_model_state')
-        tracker = Tracker(alg, self.n_actor, compress=self.compress, min_length=self.min_length,
-                          max_length=self.max_length, save_seeds=self.save_seeds)
+        # --policy_prob > 0: the agent's stochastic policy, its draws keyed by --rng_seed (ttl_policy)
+        tracker = Tracker(alg, self.n_actor, prob=self.policy_prob, compress=self.compress,
+                          min_length=self.min_length, max_length=self.max_length, save_seeds=self.save_seeds,
+                          policy_seed=self.random_seed if self.policy_prob > 0 else None)
         n = tracker.track_to_file(env, self.out_tractogram, ref_img.shape[:3], ref_img.zooms[:3])
         if int(os.environ.get('RANK', '0')) == 0:
             print('Wrote {} streamlines to {}.'.format(n, self.out_tractogram))
@@ -186,6 +189,11 @@ def add_track_args(parser):
                               'index and the step;\nthe tractogram is the same for every --n_actor and GPU count, and '
                               'no host work is added per step.\nNeither reproduces the reference\'s random '
                               'stream. [%(default)s]')
+    track_g.add_argument('--policy_prob', default=0.0, type=float, metavar='P',
+                         help='Sample the agent\'s stochastic policy, its std scaled by P:\n'
+                              'a = tanh(mu + P * std * eps).  0 tracks with the mean action.\n'
+                              'eps is drawn on the GPU from --rng_seed, the seed\'s index and the step, so the\n'
+                              'tractogram is the same for every --n_actor and GPU count. [%(default)s]')
     track_g.add_argument('--fa_map', type=str, default=None,
                          help='Scale the added noise (see `--noise`) according\nto the provided FA map '
                               '(.nii.gz). Optional.')
@@ -212,6 +220,8 @@ def parse_args(argv=None):
     parser = argparse.ArgumentParser(description=parse_args.__doc__, formatter_class=RawTextHelpFormatter)
     add_track_args(parser)
     args = parser.parse_args(argv)
+    if not 0 <= args.policy_prob < float('inf'):
+        parser.error('--policy_prob must be a finite number >= 0, not %r' % args.policy_prob)
     for f in (args.in_odf, args.in_seed, args.in_mask):
         if not os.path.isfile(f):
             parser.error('Input file {} does not exist'.format(f))

@@ -6,7 +6,9 @@ space, yield ``TractogramItem`` -- but by default it drives the env as a *stream
 ``n_actor`` streamlines are alive at once and slots freed by stopped streamlines take the next
 seeds on the device, so the GPU stays full while the tail of long streamlines finishes.
 At ``prob = 0`` every streamline depends only on its own seed, so the output is the same as
-batch-by-batch tracking (tests/test_tracker_gpu.py).
+batch-by-batch tracking (tests/test_tracker_gpu.py).  At ``prob > 0`` that holds with a
+``policy_seed``: the policy's eps is then drawn per (seed, seed index, point count) on the device
+(ttl_policy); without one, eps comes from torch.randn in alive-list order and tracking goes batch by batch.
 """
 import numpy as np
 import torch
@@ -32,10 +34,11 @@ def streamline_lengths(data, offsets):
 class Tracker(object):
 
     def __init__(self, alg, n_actor, prob=0., compress=0.0, min_length=20, max_length=200,
-                 save_seeds=False, streaming=True, rows_per_pass=None):
+                 save_seeds=False, streaming=True, rows_per_pass=None, policy_seed=None):
         self.alg = alg
         self.n_actor = n_actor
         self.prob = prob
+        self.policy_seed = policy_seed
         self.compress = compress
         self.min_length = min_length
         self.max_length = max_length
@@ -46,7 +49,7 @@ class Tracker(object):
     # ----------------------------------------------------------------------------------
     def _passes(self, env):
         n_seeds = len(env.seeds)
-        if not self.streaming or self.prob != 0.:
+        if not self.streaming or (self.prob != 0. and self.policy_seed is None):
             for start in range(0, n_seeds, self.n_actor):
                 yield start, min(start + self.n_actor, n_seeds), None
             return
@@ -79,7 +82,7 @@ class Tracker(object):
             tc_actor = prec in ('bf16', 'fp16', 'tf32')
             state = env.reset_streaming(start, end, slots, fp32_state=not tc_actor,
                                         operand=prec if tc_actor else None)
-        self.alg.validation_episode(state, env, self.prob)
+        self.alg.validation_episode(state, env, self.prob, policy_seed=self.policy_seed)
         self._check_range(env)
 
     def track_packed(self, env, copy=True):
@@ -165,8 +168,8 @@ class Tracker(object):
         world = dist.get_world_size() if dist.is_initialized() else 1
         rank = dist.get_rank() if dist.is_initialized() else 0
         if world > 1:
-            # device-drawn noise is keyed by the index in the common shuffled list: tell the env where its
-            # slice starts, so that every seed gets the noise it gets on one GPU
+            # device-drawn noise and policy samples are keyed by the index in the common shuffled list: tell
+            # the env where its slice starts, so that every seed gets the draws it gets on one GPU
             env.seed_offset = parallel.shard_bounds(len(env.seeds), rank, world)[0]
             env.seeds = parallel.shard_seeds(env.seeds, rank, world)
         vox_size = np.mean(np.abs(affine)[np.diag_indices(4)][:3])
@@ -259,7 +262,7 @@ class Tracker(object):
         for start in range(0, len(env.seeds), self.n_actor):
             end = min(start + self.n_actor, len(env.seeds))
             state = env.reset(start, end)
-            reward = self.alg.validation_episode(state, env, self.prob)
+            reward = self.alg.validation_episode(state, env, self.prob, policy_seed=self.policy_seed)
             t = env.get_streamlines()
             if tractogram is None and len(t) > 0:
                 tractogram = t
