@@ -305,6 +305,20 @@ int ttl_streamline_lengths(const float* points, const int64_t* offsets, int32_t 
  * per-point keep mask [total] and per-streamline kept-point counts [n]; the caller compacts. */
 int ttl_compress_mask(const float* points, const int64_t* offsets, int32_t n, double tol_error,
                       double max_segment_length, uint8_t* keep, int32_t* count, void* stream);
+/* Ordered compaction of n packed streamlines (offsets [n+1]): row i is kept when
+ * (keep_in == NULL || keep_in[i] != 0) && (scores == NULL || scores[i] >= threshold), compared in
+ * fp32; a NaN score is never kept.  Writes, in source order, out_offsets [m+1], out_index [m] (the
+ * source row of every kept streamline) and result [2] = {m, out_offsets[m]} on the device, so one
+ * small copy tells the host both sizes.  workspace: device, 256-byte aligned,
+ * ttl_select_workspace_bytes(n) bytes (0 for n == 0). */
+int64_t ttl_select_workspace_bytes(int32_t n);
+int ttl_select_streamlines(const int64_t* offsets, int32_t n, const uint8_t* keep_in, const float* scores,
+                           float threshold, void* workspace, int64_t workspace_bytes, int64_t* out_offsets,
+                           int64_t* out_index, int64_t* result, void* stream);
+/* out_points[out_offsets[k] ..] = points[offsets[index[k]] ..] for the m kept streamlines of
+ * ttl_select_streamlines: the points copied bit for bit, one warp per streamline. */
+int ttl_gather_streamlines(const float* points, const int64_t* offsets, const int64_t* index,
+                           const int64_t* out_offsets, int32_t m, float* out_points, void* stream);
 
 /* ---- SAC actor (algorithms/shared/offpolicy.py:61-140, shared/utils.py:41-51) -------------- */
 

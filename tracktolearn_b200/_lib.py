@@ -94,6 +94,9 @@ SIGNATURES = {
     'ttl_streamline_offsets': (c_i32, [P(Batch), c_vp, c_vp]),
     'ttl_streamline_lengths': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_vp]),
     'ttl_compress_mask': (c_i32, [c_vp, c_vp, c_i32, c_f64, c_f64, c_vp, c_vp, c_vp]),
+    'ttl_select_workspace_bytes': (c_i64, [c_i32]),
+    'ttl_select_streamlines': (c_i32, [c_vp, c_i32, c_vp, c_vp, c_f32, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp]),
+    'ttl_gather_streamlines': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_vp]),
     'ttl_pack_streamlines': (c_i32, [P(Batch), c_vp, c_vp, c_vp]),
     'ttl_actor_workspace_bytes': (c_i64, [P(ActorWeights), c_i32, c_i32]),
     'ttl_actor_plan_create': (c_i32, [P(c_vp), P(ActorWeights), c_i32, c_i32, c_vp, c_i64, c_vp]),

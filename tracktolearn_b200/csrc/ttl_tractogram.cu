@@ -1,8 +1,11 @@
 // Tractogram output path on the device (SURVEY.md section 8(f) rows 1 and 4): what the reference does
 // per streamline in Python after tracking (tracking/tracker.py:118-125) -- dipy `length` for the
 // min/max length filter and dipy `compress_streamlines` for --compress -- on packed ragged arrays
-// [total][3] fp32 + int64 offsets [n+1], one warp per streamline.
+// [total][3] fp32 + int64 offsets [n+1], one warp per streamline -- and the ordered selection that
+// keeps the streamlines passing the length filter and, optionally, the TractOracle-Net score threshold.
 #include <math.h>
+
+#include <cub/device/device_scan.cuh>
 
 #include "ttl_common.cuh"
 
@@ -94,6 +97,64 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) compress_mask_kernel(
   if (lane == 0) count[i] = nb;
 }
 
+// Ordered selection of packed streamlines.  Row i contributes (1, its point count) when it is kept and
+// (0, 0) otherwise; an exclusive scan of these pairs gives every kept row its output position and its
+// first output point.  A NaN score fails `>=` and is never kept.
+struct PairSum {
+  __device__ __forceinline__ longlong2 operator()(const longlong2& a, const longlong2& b) const {
+    return make_longlong2(a.x + b.x, a.y + b.y);
+  }
+};
+
+constexpr int kSelectThreads = 256;
+
+__global__ void __launch_bounds__(kSelectThreads) select_flag_kernel(
+    const long long* __restrict__ offsets, int n, const uint8_t* __restrict__ keep_in,
+    const float* __restrict__ scores, float threshold, longlong2* __restrict__ vals) {
+  const int i = blockIdx.x * kSelectThreads + threadIdx.x;
+  if (i >= n) return;
+  const bool keep = (keep_in == nullptr || keep_in[i] != 0) && (scores == nullptr || scores[i] >= threshold);
+  vals[i] = keep ? make_longlong2(1, offsets[i + 1] - offsets[i]) : make_longlong2(0, 0);
+}
+
+__global__ void __launch_bounds__(kSelectThreads) select_scatter_kernel(
+    const longlong2* __restrict__ vals, const longlong2* __restrict__ pre, int n, long long* __restrict__ out_offsets,
+    long long* __restrict__ out_index, long long* __restrict__ result) {
+  const int i = blockIdx.x * kSelectThreads + threadIdx.x;
+  if (i >= n) return;
+  const longlong2 v = vals[i], p = pre[i];
+  if (v.x) {
+    out_index[p.x] = i;
+    out_offsets[p.x + 1] = p.y + v.y;
+  }
+  if (i == n - 1) {
+    out_offsets[0] = 0;
+    result[0] = p.x + v.x;
+    result[1] = p.y + v.y;
+  }
+}
+
+// out_points[out_offsets[k]..] = points[offsets[index[k]]..], one warp per kept streamline.
+__global__ void __launch_bounds__(kWarpsPerBlock * 32) gather_streamlines_kernel(
+    const float* __restrict__ points, const long long* __restrict__ offsets, const long long* __restrict__ index,
+    const long long* __restrict__ out_offsets, int m, float* __restrict__ out_points) {
+  const int k = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (k >= m) return;
+  const float* src = points + offsets[index[k]] * 3;
+  float* dst = out_points + out_offsets[k] * 3;
+  const long long cnt = (out_offsets[k + 1] - out_offsets[k]) * 3;
+  for (long long j = lane; j < cnt; j += 32) dst[j] = src[j];
+}
+
+size_t select_pairs_bytes(int n) { return ((size_t)n * sizeof(longlong2) + 255) / 256 * 256; }
+
+size_t select_scan_bytes(int n) {
+  size_t tmp = 0;
+  cub::DeviceScan::ExclusiveScan(nullptr, tmp, (const longlong2*)nullptr, (longlong2*)nullptr, PairSum(),
+                                 make_longlong2(0, 0), n);
+  return tmp;
+}
+
 }  // namespace
 
 extern "C" {
@@ -118,6 +179,58 @@ int ttl_compress_mask(const float* points, const int64_t* offsets, int32_t n, do
   TTL_LAUNCH("compress_mask_kernel", s,
              compress_mask_kernel<<<ttl_div_up(n, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
                  points, (const long long*)offsets, n, tol_error, max_segment_length, keep, count));
+  TTL_CHECK_LAST();
+  return 0;
+}
+
+int64_t ttl_select_workspace_bytes(int32_t n) {
+  if (n < 0) return TTL_ERR_BAD_ARG;
+  if (n == 0) return 0;
+  return (int64_t)(2 * select_pairs_bytes(n) + select_scan_bytes(n));
+}
+
+int ttl_select_streamlines(const int64_t* offsets, int32_t n, const uint8_t* keep_in, const float* scores,
+                           float threshold, void* workspace, int64_t workspace_bytes, int64_t* out_offsets,
+                           int64_t* out_index, int64_t* result, void* stream) {
+  if (n < 0 || !out_offsets || !result) return TTL_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (n == 0) {
+    if (cudaMemsetAsync(out_offsets, 0, sizeof(int64_t), s) != cudaSuccess ||
+        cudaMemsetAsync(result, 0, 2 * sizeof(int64_t), s) != cudaSuccess)
+      return TTL_ERR_DRIVER;
+    return 0;
+  }
+  if (!offsets || !out_index || !workspace || workspace_bytes < ttl_select_workspace_bytes(n)) return TTL_ERR_BAD_ARG;
+  longlong2* vals = (longlong2*)workspace;
+  longlong2* pre = (longlong2*)((char*)workspace + select_pairs_bytes(n));
+  void* tmp = (char*)workspace + 2 * select_pairs_bytes(n);
+  size_t tmp_bytes = select_scan_bytes(n);
+  const int blocks = ttl_div_up(n, kSelectThreads);
+  TTL_LAUNCH("select_flag_kernel", s,
+             select_flag_kernel<<<blocks, kSelectThreads, 0, s>>>((const long long*)offsets, n, keep_in, scores,
+                                                                   threshold, vals));
+  TTL_CHECK_LAST();
+  cudaError_t e = cudaSuccess;
+  TTL_LAUNCH("select_scan", s,
+             e = cub::DeviceScan::ExclusiveScan(tmp, tmp_bytes, (const longlong2*)vals, pre, PairSum(), make_longlong2(0, 0), n, s));
+  if (e != cudaSuccess) return (int)e;
+  TTL_LAUNCH("select_scatter_kernel", s,
+             select_scatter_kernel<<<blocks, kSelectThreads, 0, s>>>(vals, pre, n, (long long*)out_offsets,
+                                                                      (long long*)out_index, (long long*)result));
+  TTL_CHECK_LAST();
+  return 0;
+}
+
+int ttl_gather_streamlines(const float* points, const int64_t* offsets, const int64_t* index,
+                           const int64_t* out_offsets, int32_t m, float* out_points, void* stream) {
+  if (m < 0) return TTL_ERR_BAD_ARG;
+  if (m == 0) return 0;
+  if (!points || !offsets || !index || !out_offsets || !out_points) return TTL_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  TTL_LAUNCH("gather_streamlines_kernel", s,
+             gather_streamlines_kernel<<<ttl_div_up(m, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
+                 points, (const long long*)offsets, (const long long*)index, (const long long*)out_offsets, m,
+                 out_points));
   TTL_CHECK_LAST();
   return 0;
 }

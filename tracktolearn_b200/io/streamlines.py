@@ -31,22 +31,24 @@ def _voxel_order(affine):
 
 
 class TrkWriter(object):
-    """Streams (data, offsets) batches to a .trk file; the streamline count is patched on close."""
+    """Streams (data, offsets) batches to a .trk file; the streamline count is patched on close.
+    Per-streamline properties: ``seeds_x/y/z`` (``save_seeds``), then ``oracle_score`` (``save_scores``)."""
 
-    def __init__(self, path, dims, voxel_sizes, affine, save_seeds=False):
+    def __init__(self, path, dims, voxel_sizes, affine, save_seeds=False, save_scores=False):
         self.f = open(path, 'wb')
         self.n = 0
         self.save_seeds = save_seeds
+        self.save_scores = save_scores
+        names = ((b'seeds_x', b'seeds_y', b'seeds_z') if save_seeds else ()) + ((b'oracle_score',) if save_scores else ())
         hdr = bytearray(1000)
         hdr[0:6] = b'TRACK\x00'
         struct.pack_into('<3h', hdr, 6, *[int(d) for d in dims])
         struct.pack_into('<3f', hdr, 12, *[float(v) for v in voxel_sizes])
         struct.pack_into('<3f', hdr, 24, 0.0, 0.0, 0.0)
         struct.pack_into('<h', hdr, 36, 0)                                   # n_scalars
-        struct.pack_into('<h', hdr, 238, 3 if save_seeds else 0)             # n_properties
-        if save_seeds:
-            for i, name in enumerate((b'seeds_x', b'seeds_y', b'seeds_z')):
-                hdr[240 + 20 * i:240 + 20 * i + len(name)] = name
+        struct.pack_into('<h', hdr, 238, len(names))                         # n_properties
+        for i, name in enumerate(names):
+            hdr[240 + 20 * i:240 + 20 * i + len(name)] = name
         struct.pack_into('<16f', hdr, 440, *np.asarray(affine, dtype=np.float32).reshape(-1))
         vo = _voxel_order(affine).encode()
         hdr[948:948 + len(vo)] = vo
@@ -55,12 +57,12 @@ class TrkWriter(object):
         struct.pack_into('<i', hdr, 996, 1000)                               # hdr_size
         self.f.write(bytes(hdr))
 
-    def write(self, data, offsets, seeds=None):
+    def write(self, data, offsets, seeds=None, scores=None):
         n = len(offsets) - 1
         if n <= 0:
             return
         lens = np.diff(offsets).astype(np.int64)
-        n_prop = 3 if self.save_seeds else 0
+        n_prop = (3 if self.save_seeds else 0) + (1 if self.save_scores else 0)
         total = int(lens.sum()) * 3 + n * (1 + n_prop)
         out = np.empty(total, dtype='<f4')
         # positions of the int32 counts inside the float buffer
@@ -72,6 +74,8 @@ class TrkWriter(object):
             ps = starts + 1 + lens * 3
             for c in range(3):
                 out[ps + c] = np.asarray(seeds, dtype=np.float32)[:, c]
+        if self.save_scores:
+            out[starts + lens * 3 + n_prop] = np.asarray(scores, dtype=np.float32).reshape(-1)
         self.f.write(out.tobytes())
         self.n += n
 
@@ -97,7 +101,8 @@ class TckWriter(object):
         self.f.write(text.encode())
         self.offset = offset
 
-    def write(self, data, offsets, seeds=None):
+    def write(self, data, offsets, seeds=None, scores=None):
+        """``seeds`` and ``scores`` are accepted for TrkWriter's signature: .tck has no per-streamline data."""
         n = len(offsets) - 1
         if n <= 0:
             return
@@ -118,8 +123,9 @@ class TckWriter(object):
         self.f.close()
 
 
-def read_trk(path):
-    """-> (data [sum L,3] float32 in voxmm, offsets, header dict).  For tests."""
+def read_trk(path, spans=False):
+    """-> (data [sum L,3] float32 in voxmm, offsets, header dict).  ``spans=True``: also the byte span
+    [start, end) of every record in the file, as a fourth item (int64 arrays (start, end))."""
     with open(path, 'rb') as f:
         raw = f.read()
     n_scalars = struct.unpack('<h', raw[36:38])[0]
@@ -127,22 +133,37 @@ def read_trk(path):
     n_count = struct.unpack('<i', raw[988:992])[0]
     hdr = {'dims': struct.unpack('<3h', raw[6:12]), 'voxel_sizes': struct.unpack('<3f', raw[12:24]),
            'affine': np.array(struct.unpack('<16f', raw[440:504])).reshape(4, 4), 'n_count': n_count,
-           'voxel_order': raw[948:951].decode(), 'n_properties': n_prop}
+           'voxel_order': raw[948:951].decode(), 'n_properties': n_prop, 'n_scalars': n_scalars,
+           'property_names': [raw[240 + 20 * i:260 + 20 * i].split(b'\x00')[0].decode() for i in range(n_prop)]}
     body = np.frombuffer(raw, dtype='<f4', offset=1000)
-    ints = body.view('<i4')
-    pos, pts, lens, props = 0, [], [], []
-    for _ in range(n_count):
-        L = int(ints[pos])
-        pts.append(body[pos + 1:pos + 1 + L * (3 + n_scalars)].reshape(L, 3 + n_scalars)[:, :3])
-        props.append(body[pos + 1 + L * (3 + n_scalars):pos + 1 + L * (3 + n_scalars) + n_prop])
-        lens.append(L)
-        pos += 1 + L * (3 + n_scalars) + n_prop
+    # the records are found by walking their counts (each position depends on the previous count); the
+    # points are then what is left once the count and property words are masked out
+    ints = memoryview(raw)[1000:1000 + (len(raw) - 1000) // 4 * 4].cast('i')
+    w = 3 + n_scalars
+    starts, lens = [0] * n_count, [0] * n_count
+    pos = 0
+    for i in range(n_count):
+        L = ints[pos]
+        starts[i] = pos
+        lens[i] = L
+        pos += 1 + L * w + n_prop
+    starts, lens = np.asarray(starts, dtype=np.int64), np.asarray(lens, dtype=np.int64)
     offsets = np.concatenate(([0], np.cumsum(lens))).astype(np.int64)
-    hdr['properties'] = np.asarray(props)
-    return (np.concatenate(pts) if pts else np.zeros((0, 3), np.float32)), offsets, hdr
+    prop_at = starts + 1 + lens * w
+    is_point = np.ones((pos,), dtype=bool)
+    is_point[starts] = False
+    for k in range(n_prop):
+        is_point[prop_at + k] = False
+    data = np.ascontiguousarray(body[:pos][is_point].reshape(-1, w)[:, :3])
+    hdr['properties'] = body[prop_at[:, None] + np.arange(n_prop)] if n_count else np.asarray([])
+    if spans:
+        return data, offsets, hdr, (1000 + 4 * starts, 1000 + 4 * (prop_at + n_prop))
+    return data, offsets, hdr
 
 
-def read_tck(path):
+def read_tck(path, spans=False):
+    """-> (data [sum L,3] float32, offsets, header dict).  ``spans=True``: also the byte span [start, end)
+    of every record, its NaN delimiter included, as a fourth item."""
     with open(path, 'rb') as f:
         raw = f.read()
     head = raw[:raw.index(b'END\n')].decode()
@@ -156,4 +177,6 @@ def read_tck(path):
     data = body[~(is_nan | is_inf)]
     offsets = np.concatenate(([0], np.cumsum(lens))).astype(np.int64)
     assert len(lens) == count
+    if spans:
+        return data, offsets, {'count': count}, (offset + 12 * (ends - lens), offset + 12 * (ends + 1))
     return data, offsets, {'count': count}

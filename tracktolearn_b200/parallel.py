@@ -212,7 +212,7 @@ def _gather_via_arena(parts, dst, copy):
     return out
 
 
-def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto'):
+def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', scores=None):
     """Gather packed streamlines on rank `dst` in rank order.
 
     ``via``: 'nccl' -- the data travels through NCCL to `dst`'s GPU and over its PCIe link (below);
@@ -226,7 +226,9 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto'):
     sizes, then every rank sends exactly its rows into its slice of `dst`'s buffers (batched
     point-to-point: device-to-device over NVLink under NCCL) and `dst` makes one D2H copy per array
     into grow-only pinned memory.  With ``copy=False`` the returned arrays are views of that pinned
-    memory, valid until the next gather.  Returns a Tractogram on `dst`, None elsewhere."""
+    memory, valid until the next gather.  ``scores`` [n] float32 (optional): per-streamline oracle scores,
+    carried along and returned as ``data_per_streamline['oracle_score']``.  Returns a Tractogram on `dst`,
+    None elsewhere."""
     world, rank = dist.get_world_size(), dist.get_rank()
     dev = _device_for_backend()
     if via == 'auto':
@@ -239,18 +241,20 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto'):
                  (lengths.to(dtype=torch.int64).reshape(-1, 1), 1, torch.int64, 'len'),
                  (seeds.to(dtype=torch.float64).reshape(-1, 3), 3, torch.float64, 'seeds'),
                  (flags.to(dtype=torch.int64).reshape(-1, 1), 1, torch.int64, 'flags')]
+        if scores is not None:
+            parts.append((scores.to(dtype=torch.float32).reshape(-1, 1), 1, torch.float32, 'scores'))
         arrs = _gather_via_arena(parts, dst, copy)
         if arrs is None:
             return None
         if not isinstance(arrs, str):
-            data, lens, gseeds, gflags = arrs
-            offsets = np.concatenate(([0], np.cumsum(lens[:, 0]))).astype(np.int64)
-            return Tractogram(data=data, offsets=offsets, data_per_streamline={'seeds': gseeds, 'flags': gflags[:, 0]})
+            return _packed_tractogram(arrs)
         # the arena could not be set up on some rank (every rank knows): the NCCL route below
     parts = [(points.to(dev, dtype=torch.float32).reshape(-1, 3).contiguous(), 3, torch.float32, 'pts'),
              (lengths.to(dev, dtype=torch.int64).reshape(-1, 1).contiguous(), 1, torch.int64, 'len'),
              (seeds.to(dev, dtype=torch.float64).reshape(-1, 3).contiguous(), 3, torch.float64, 'seeds'),
              (flags.to(dev, dtype=torch.int64).reshape(-1, 1).contiguous(), 1, torch.int64, 'flags')]
+    if scores is not None:
+        parts.append((scores.to(dev, dtype=torch.float32).reshape(-1, 1).contiguous(), 1, torch.float32, 'scores'))
     n_sl, n_pts = int(parts[1][0].shape[0]), int(parts[0][0].shape[0])
     sizes = torch.tensor([n_sl, n_pts], dtype=torch.int64, device=dev)
     all_sizes = [torch.zeros_like(sizes) for _ in range(world)]
@@ -289,10 +293,17 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto'):
             host.append(buf)
     if bufs and bufs[0].is_cuda:
         torch.cuda.current_stream(bufs[0].device).synchronize()
-    arrs = [h.numpy().copy() if copy else h.numpy() for h in host]
-    data, lens, gseeds, gflags = arrs
+    return _packed_tractogram([h.numpy().copy() if copy else h.numpy() for h in host])
+
+
+def _packed_tractogram(arrs):
+    """[points, lengths, seeds, flags(, scores)] host arrays in gather_packed's part order -> Tractogram."""
+    data, lens, gseeds, gflags = arrs[:4]
     offsets = np.concatenate(([0], np.cumsum(lens[:, 0]))).astype(np.int64)
-    return Tractogram(data=data, offsets=offsets, data_per_streamline={'seeds': gseeds, 'flags': gflags[:, 0]})
+    per = {'seeds': gseeds, 'flags': gflags[:, 0]}
+    if len(arrs) > 4:
+        per['oracle_score'] = arrs[4][:, 0]
+    return Tractogram(data=data, offsets=offsets, data_per_streamline=per)
 
 
 def gather_tractogram(local, dst=0, copy=True, via='auto'):

@@ -49,6 +49,10 @@ class TrackToLearnTrack(object):
         self.compress = track_dto['compress'] or 0.0
         self.sh_basis = track_dto['sh_basis']
         self.save_seeds = track_dto['save_seeds']
+        self.oracle_checkpoint = track_dto.get('oracle_checkpoint')
+        self.oracle_threshold = float(track_dto.get('oracle_threshold', 0.5))
+        self.oracle_precision = track_dto.get('oracle_precision', 'fp16')
+        self.save_oracle_scores = bool(track_dto.get('save_oracle_scores', False))
         self.compute_reward = False
         if not torch.cuda.is_available():
             raise SystemExit('ttl_track (tracktolearn_b200) needs a CUDA device; there is no CPU path')
@@ -120,7 +124,13 @@ class TrackToLearnTrack(object):
         tracker = Tracker(alg, self.n_actor, prob=self.policy_prob, compress=self.compress,
                           min_length=self.min_length, max_length=self.max_length, save_seeds=self.save_seeds,
                           policy_seed=self.random_seed if self.policy_prob > 0 else None)
-        n = tracker.track_to_file(env, self.out_tractogram, ref_img.shape[:3], ref_img.zooms[:3])
+        oracle = None
+        if self.oracle_checkpoint:
+            from tracktolearn_b200.oracles.oracle import OracleSingleton
+            OracleSingleton.clear()
+            oracle = OracleSingleton(self.oracle_checkpoint, self.device, precision=self.oracle_precision)
+        n = tracker.track_to_file(env, self.out_tractogram, ref_img.shape[:3], ref_img.zooms[:3], oracle=oracle,
+                                  oracle_threshold=self.oracle_threshold, save_scores=self.save_oracle_scores)
         if int(os.environ.get('RANK', '0')) == 0:
             print('Wrote {} streamlines to {}.'.format(n, self.out_tractogram))
         return n
@@ -201,6 +211,19 @@ def add_track_args(parser):
                          help='Lower limit for interpolation of tracking mask value.\nTracking will stop '
                               'below this threshold.')
     parser.add_argument('--rng_seed', default=1337, type=int, help='Random number generator seed [%(default)s].')
+    oracle_g = parser.add_argument_group('Oracle filtering')
+    oracle_g.add_argument('--oracle_checkpoint', type=str, default=None, metavar='CKPT',
+                          help='TractOracle-Net checkpoint.  If set, every streamline that passes the length\n'
+                               'filter is scored on the GPU and kept only when its score is\n'
+                               '>= --oracle_threshold.  Scores are taken before --compress.')
+    oracle_g.add_argument('--oracle_threshold', type=float, default=0.5, metavar='T',
+                          help='Keep streamlines whose oracle score is >= T, in [0, 1]. [%(default)s]')
+    oracle_g.add_argument('--oracle_precision', default='fp16', choices=['fp16', 'fp32'],
+                          help='Oracle arithmetic.  fp16: tcgen05 tensor cores, the reference\'s autocast\n'
+                               'arithmetic; fp32: CUDA cores. [%(default)s]')
+    oracle_g.add_argument('--save_oracle_scores', action='store_true',
+                          help='Save each kept streamline\'s score as the per-streamline\nproperty '
+                               '"oracle_score" (.trk only).')
 
 
 def verify_agent_option(parser, args):
@@ -235,6 +258,14 @@ def parse_args(argv=None):
         parser.error('Invalid streamline length options')
     if args.compress is not None and args.compress < 0.001:
         parser.error('--compress should be at least 0.001')
+    if not 0.0 <= args.oracle_threshold <= 1.0:
+        parser.error('--oracle_threshold must be in [0, 1], not %r' % args.oracle_threshold)
+    if args.save_oracle_scores and not args.oracle_checkpoint:
+        parser.error('--save_oracle_scores needs --oracle_checkpoint')
+    if args.save_oracle_scores and detect_format(args.out_tractogram) != 'trk':
+        parser.error('--save_oracle_scores needs a .trk output: .tck files cannot hold per-streamline data')
+    if args.oracle_checkpoint and not os.path.isfile(args.oracle_checkpoint):
+        parser.error('Oracle checkpoint {} does not exist'.format(args.oracle_checkpoint))
     verify_agent_option(parser, args)
     return args
 

@@ -54,3 +54,34 @@ def compress_packed(data, offsets, tol_error=0.01, max_segment_length=10.0, devi
     new_offsets = torch.zeros((n + 1,), dtype=torch.int64, device=device)
     torch.cumsum(count, 0, out=new_offsets[1:])
     return d[keep.bool()], new_offsets
+
+
+def select_packed(data, offsets, keep=None, scores=None, threshold=0.0):
+    """Ordered selection of packed streamlines on their device (``ttl_select_streamlines`` +
+    ``ttl_gather_streamlines``): streamline i is kept when ``keep[i]`` (uint8 / bool, None = all) and
+    ``scores[i] >= threshold`` (float32, compared in float32; None = no score test; NaN is never kept).
+    Returns (data', offsets', index) as CUDA tensors: the kept points bit for bit, their offsets and the
+    int64 source row of every kept streamline.  One device-to-host copy of the two sizes."""
+    device = _dev(data.device)
+    lib = _lib.load()
+    data, offsets = _to_device(data, offsets, device)
+    n = int(offsets.shape[0]) - 1
+    sp = _lib.stream_ptr(device)
+    if keep is not None:
+        keep = keep.to(device, dtype=torch.uint8).contiguous()
+    if scores is not None:
+        scores = scores.to(device, dtype=torch.float32).contiguous()
+    nbytes = int(lib.ttl_select_workspace_bytes(max(n, 0)))
+    work = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=device)
+    out_off = torch.empty((max(n, 0) + 1,), dtype=torch.int64, device=device)
+    index = torch.empty((max(n, 0),), dtype=torch.int64, device=device)
+    result = torch.empty((2,), dtype=torch.int64, device=device)
+    with torch.cuda.device(device):
+        _lib.check(lib.ttl_select_streamlines(_lib.ptr(offsets), max(n, 0), _lib.ptr(keep), _lib.ptr(scores),
+                                              float(threshold), _lib.ptr(work), nbytes, _lib.ptr(out_off),
+                                              _lib.ptr(index), _lib.ptr(result), sp), 'ttl_select_streamlines')
+        m, total = (int(v) for v in result.cpu())
+        out = torch.empty((total, 3), dtype=torch.float32, device=device)
+        _lib.check(lib.ttl_gather_streamlines(_lib.ptr(data), _lib.ptr(offsets), _lib.ptr(index), _lib.ptr(out_off),
+                                              m, _lib.ptr(out), sp), 'ttl_gather_streamlines')
+    return out, out_off[:m + 1], index[:m]

@@ -148,17 +148,29 @@ class Tracker(object):
         d, o = compress_packed(data, offsets, tol_error=float(tol_vox), device=env.device)
         return d.cpu().numpy(), o.cpu().numpy()
 
-    def track_to_file(self, env, path, dims, voxel_sizes):
+    def track_to_file(self, env, path, dims, voxel_sizes, oracle=None, oracle_threshold=0.5, save_scores=False):
         """What ``ttl_track.py`` does with ``track`` + ``nib.streamlines.save`` (runners/ttl_track.py:
         172-186), on packed arrays and on the device: dipy ``length`` and the min/max filter
         (tracker.py:118-121), ``compress_streamlines`` (:123-125), voxel -> file space (:127-136);
         only the kept, transformed float32 points cross PCIe, into pinned memory, and go to a
-        streaming .trk / .tck writer.  Returns the number of streamlines kept."""
+        streaming .trk / .tck writer.  Returns the number of streamlines kept.
+
+        ``oracle`` (an ``OracleSingleton``): after the length filter, every streamline is scored by
+        TractOracle-Net on its voxel-space points -- the coordinates the in-step ORACLE criterion scores --
+        and kept when its score is >= ``oracle_threshold`` (the criterion stops below 0.5).  Scoring
+        comes before ``--compress``, so a score does not depend on it.  Each rank scores its own
+        streamlines: a streamline's score does not depend on the batch it is scored in, so the file is
+        the same for every GPU count.  ``save_scores`` (.trk only) writes the scores as the
+        per-streamline property ``oracle_score``."""
         from tracktolearn_b200.io.streamlines import TckWriter, TrkWriter, detect_format
-        from tracktolearn_b200.tracking.postprocess import compress_packed, lengths_packed
+        from tracktolearn_b200.tracking.postprocess import compress_packed, lengths_packed, select_packed
         import torch.distributed as dist
         from tracktolearn_b200 import parallel
         fmt = detect_format(path)
+        if save_scores and oracle is None:
+            raise ValueError('save_scores needs an oracle')
+        if save_scores and fmt != 'trk':
+            raise ValueError('.tck files cannot hold per-streamline data: save oracle scores to a .trk file')
         affine = np.asarray(env.affine_vox2rasmm, dtype=np.float64)
         np.random.shuffle(env.seeds)      # tracker.py:94
         # One process per GPU (torchrun): every rank shuffled the same seed list with the same RNG state;
@@ -176,8 +188,8 @@ class Tracker(object):
         lo, hi = self.min_length / vox_size, self.max_length / vox_size
         writer = None
         if rank == 0:
-            writer = (TrkWriter(path, dims, voxel_sizes, affine, self.save_seeds) if fmt == 'trk'
-                      else TckWriter(path))
+            writer = (TrkWriter(path, dims, voxel_sizes, affine, self.save_seeds, save_scores=save_scores)
+                      if fmt == 'trk' else TckWriter(path))
         self.alg.agent.eval()
         n_passes = len(list(self._passes(env)))
         if world > 1:       # ranks may differ by one seed: agree on the number of passes
@@ -190,15 +202,16 @@ class Tracker(object):
                 out = torch.zeros((0, 3), dtype=torch.float32, device=env.device)
                 new_off = torch.zeros((1,), dtype=torch.int64, device=env.device)
                 seeds_kept = np.zeros((0, 3))
+                scores_kept = torch.zeros((0,), dtype=torch.float32, device=env.device)
                 if ip < len(passes) and passes[ip][1] > passes[ip][0]:
                     self._run_pass(env, *passes[ip])
                     pts, offsets = env.get_streamlines_device()
                     lens = lengths_packed(pts, offsets)
-                    keep = (lens >= lo) & (lens <= hi)
-                    npts = offsets[1:] - offsets[:-1]
-                    data = pts[torch.repeat_interleave(keep, npts)]
-                    new_off = torch.zeros((int(keep.sum().item()) + 1,), dtype=torch.int64, device=pts.device)
-                    torch.cumsum(npts[keep], 0, out=new_off[1:])
+                    data, new_off, index = select_packed(pts, offsets, keep=(lens >= lo) & (lens <= hi))
+                    if oracle is not None:
+                        scores = oracle.predict_device(data, new_off, distributed=False)
+                        data, new_off, sel = select_packed(data, new_off, scores=scores, threshold=oracle_threshold)
+                        index, scores_kept = index[sel], scores[sel]
                     if self.compress:     # after the length filter, before the space change (tracker.py:120-129)
                         data, new_off = compress_packed(data, new_off, tol_error=float(self.compress) / float(vox_size))
                     d64 = data.to(torch.float64)
@@ -209,13 +222,15 @@ class Tracker(object):
                         cols = [d64[:, 0] * A[0, c] + d64[:, 1] * A[1, c] + d64[:, 2] * A[2, c] + A[c, 3]
                                 for c in range(3)]
                         out = torch.stack(cols, 1).to(torch.float32)
-                    seeds_kept = np.asarray(env.initial_points)[keep.cpu().numpy()] - 0.5
+                    seeds_kept = np.asarray(env.initial_points)[index.cpu().numpy()] - 0.5
                 if world > 1:
                     n_kept = int(new_off.shape[0]) - 1
                     merged = parallel.gather_packed(out, new_off[1:] - new_off[:-1], torch.as_tensor(seeds_kept),
-                                                    torch.zeros((n_kept,), dtype=torch.int64), copy=False)
+                                                    torch.zeros((n_kept,), dtype=torch.int64), copy=False,
+                                                    scores=scores_kept if save_scores else None)
                     if rank == 0 and len(merged) > 0:
-                        writer.write(merged.data, merged.offsets, merged.data_per_streamline['seeds'])
+                        writer.write(merged.data, merged.offsets, merged.data_per_streamline['seeds'],
+                                     merged.data_per_streamline.get('oracle_score'))
                     continue
                 if int(new_off.shape[0]) <= 1:
                     continue
@@ -224,7 +239,8 @@ class Tracker(object):
                 h_data.copy_(out.reshape(-1), non_blocking=True)
                 h_off.copy_(new_off, non_blocking=True)
                 torch.cuda.current_stream(env.device).synchronize()
-                writer.write(h_data.numpy().reshape(-1, 3), h_off.numpy(), seeds_kept)
+                writer.write(h_data.numpy().reshape(-1, 3), h_off.numpy(), seeds_kept,
+                             scores_kept.cpu().numpy() if save_scores else None)
         finally:
             if writer is not None:
                 writer.close()
