@@ -5,7 +5,7 @@ repeated:
 
     noise 0            the deterministic path bench.py times
     noise 0.1 host     rng.normal on the host every step + H2D copy; the fused head and graph replay are off
-    noise 0.1 device   drawn inside propagate_stop_kernel (ttl_env_step_head_rng): fused head stays on
+    noise 0.1 device   drawn inside propagate_stop_kernel (ttl_env_step with a ttl_noise): fused head stays on
 
     python benchmarks/noise_probe.py [--repeats 3] [--steps 200] [--out profiles/noise_probe.json]
 

@@ -6,7 +6,7 @@ repeated:
     prob 0             the deterministic path bench.py times (fused head)
     prob 1 torch eps   torch.randn per step, actor head_finish_kernel, then the env step: the route without a
                        policy seed, here streamed like the others so that the comparison is like for like
-    prob 1 device eps  eps drawn inside propagate_policy_kernel (ttl_env_step_head_policy): fused head stays on
+    prob 1 device eps  eps drawn inside propagate_policy_kernel (ttl_env_step with a ttl_policy): fused head stays on
 
     python benchmarks/policy_probe.py [--repeats 3] [--steps 200] [--burn-in 384] [--out profiles/policy_probe.json]
 

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define TTL_ABI_VERSION 4
+#define TTL_ABI_VERSION 5
 
 /* StoppingFlags, environments/stopping_criteria.py:10-20 */
 #define TTL_STOPPING_MASK 1
@@ -162,49 +162,6 @@ int ttl_peaks_from_sh(const float* sh, int64_t n_voxels, int32_t C, int32_t ld, 
 int ttl_env_reset(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b,
                   const double* seeds, void* stream);
 
-/* TrackingEnvironment.step (tracking_env.py:135-221; NoisyTrackingEnvironment.step when
- * prm->dir_f64): actions [n_alive][lda] fp32 for the alive rows of alive[cur], optional
- * `noise` [n_alive][3] f64 added first.  Normalise+scale (env.py:493-502), first-step flip,
- * grow, stopping flags (env.py:567-603, utils.py:127-173, stopping_criteria.py:38-82), reward,
- * ordered compaction into alive[cur^1] / ctrl[cur^1], new state rows into state[cur^1]
- * (survivors first, in order; then refilled rows if prm->refill, or stopped rows if
- * prm->state_stopped).
- * `n_upper` >= current alive count bounds the launch (the kernels read the true count from
- * ctrl[cur] on the device, so no host sync is needed between steps).
- * The caller flips cur afterwards: that flip is TrackingEnvironment.harvest (:223-245). */
-int ttl_env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                 const float* actions, int32_t lda, const double* noise, int32_t n_upper,
-                 void* stream);
-
-/* ttl_env_step with the actions taken straight from the actor's fused head (the pointers that
- * ttl_actor_head_partial returns after a forward with action == NULL): action = tanh(mu), the
- * deterministic policy that tracking uses (prob = 0: tracker.py:28, ttl_track.py:172-175;
- * offpolicy.py:126-128 with std * 0).  head_partial [n_alive][n_tiles][8] fp32 per-column-tile
- * partial sums of the 6-wide output layer (tiles_per_256 = 256 / tile width of the launch that wrote
- * them), head_bias [6].  The sums follow the same fixed tree as the actor's own finishing pass, so this
- * entry point and ttl_actor_forward* + ttl_env_step give the same bits whatever the tile width; it
- * saves one launch and the action round trip per step.  No noise array: the noisy
- * environment with host-drawn noise (sigma > 0) goes through ttl_env_step; device-drawn noise
- * through ttl_env_step_head_rng below. */
-int ttl_env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                      const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
-                      const float* head_bias, int32_t n_upper, void* stream);
-
-/* The same step split in two so that TractOracle-Net can be consulted in between
- * (OracleStoppingCriterion, stopping_criteria.py:113-154: stop where the score < 0.5 once the
- * streamline has more than min_pts_stop points; OracleReward, oracle_reward.py:45-93: `bonus` for
- * streamlines done this step with more than min_pts_reward points and score > 0.5):
- *   ttl_env_step_begin          propagate + LENGTH/CURVATURE/MASK + alignment reward
- *   ttl_oracle_features_rows    resample(128)+diff of the alive streamlines   \  caller, between
- *   ttl_oracle_forward          scores [n_alive]                              /  the two calls
- *   ttl_env_step_finish         ORACLE flag, bonus, compaction bookkeeping, state rows */
-int ttl_env_step_begin(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                       const float* actions, int32_t lda, const double* noise, int32_t n_upper,
-                       void* stream);
-int ttl_env_step_finish(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                        const float* scores, int32_t use_stop, int32_t min_pts_stop, int32_t min_pts_reward,
-                        float bonus, int32_t n_upper, void* stream);
-
 /* Tracking noise drawn inside the step kernel (NoisyTrackingEnvironment with noise_rng = 'device').
  * Row i of the batch, with g = row_base + i and L = its point count before the step (1 on the first
  * step), gets noise_c = sigma * z_c for c = 0, 1, 2, where
@@ -222,17 +179,6 @@ typedef struct ttl_noise {
   int64_t row_base;        /* global seed index of batch row 0 */
 } ttl_noise;
 
-/* ttl_env_step, ttl_env_step_head and ttl_env_step_begin with the noise drawn on the device as
- * described at ttl_noise: no host work, no copy and no extra launch per step.  prm->dir_f64 must be 1
- * (the noisy environment's float64 directions), else TTL_ERR_UNSUPPORTED. */
-int ttl_env_step_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                     const float* actions, int32_t lda, const ttl_noise* nz, int32_t n_upper, void* stream);
-int ttl_env_step_head_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                          const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
-                          const float* head_bias, const ttl_noise* nz, int32_t n_upper, void* stream);
-int ttl_env_step_begin_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                           const float* actions, int32_t lda, const ttl_noise* nz, int32_t n_upper,
-                           void* stream);
 /* The standard normals the step kernels use, for tests: out [n][3] f64, out[k][c] = z_c(nz->seed, g[k],
  * L[k]) for g [n] int64 and L [n] int32 (device arrays); nz->sigma and nz->row_base are ignored. */
 int ttl_noise_normals(const ttl_noise* nz, const int64_t* g, const int32_t* L, int32_t n, double* out,
@@ -242,16 +188,16 @@ int ttl_noise_normals(const ttl_noise* nz, const int64_t* g, const int32_t* L, i
  * Row i of the batch, with g = row_base + i (row_base as for ttl_noise: seed_offset + start after
  * reset / reset_streaming, 0 after nreset) and L = its point count before the step, takes for c = 0, 1, 2
  *   eps_c = fp32_rn(z(seed, g, L, 3 + c))        z = the ttl_noise normal above, counter words 3..5
- *   mu_c  = head output c     + bias[c]          the actor's fixed summation tree (ttl_env_step_head)
+ *   mu_c  = head output c     + bias[c]          the actor's fixed summation tree (ttl_step_action)
  *   ls_c  = head output 3 + c + bias[3 + c]
  *   std_c = expf(fminf(fmaxf(ls_c, -20.f), 2.f)) * prob
  *   a_c   = tanhf(fmaf(std_c, eps_c, mu_c))
  * which is the actor's own head arithmetic (MaxEntropyActor.forward, offpolicy.py:94-140) with eps_c in
- * place of torch.randn: the fused route (ttl_env_step_head_policy) and the actor-then-step route fed by
- * ttl_policy_eps give the same bits.  Counter words 3..5 keep eps independent of the tracking noise
- * (words 0..2) under one seed.  At prob = 0 the action is tanh(mu) bit for bit.  Each streamline's sample
- * depends only on (seed, g, L): not on the slot count, the alive-list order or the GPU count.  It is not
- * torch's random stream.  Host struct read at call time; a CUDA graph captures its values. */
+ * place of torch.randn: the fused route (ttl_env_step with head partials and `pol`) and the actor-then-step
+ * route fed by ttl_policy_eps give the same bits.  Counter words 3..5 keep eps independent of the tracking
+ * noise (words 0..2) under one seed.  At prob = 0 the action is tanh(mu) bit for bit.  Each streamline's
+ * sample depends only on (seed, g, L): not on the slot count, the alive-list order or the GPU count.  It is
+ * not torch's random stream.  Host struct read at call time; a CUDA graph captures its values. */
 typedef struct ttl_policy {
   uint64_t seed;           /* Philox key */
   int64_t row_base;        /* global seed index of batch row 0 */
@@ -259,13 +205,60 @@ typedef struct ttl_policy {
   int32_t pad;
 } ttl_policy;
 
-/* ttl_env_step_head with the policy sampled inside the propagate kernel: head_partial must hold all six
- * outputs (ttl_actor_forward*_policy_partial).  nz == NULL: no device noise; non-NULL: device-drawn
- * tracking noise added to a as ttl_env_step_head_rng does (prm->dir_f64 must be 1). */
-int ttl_env_step_head_policy(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                             const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
-                             const float* head_bias, const ttl_policy* pol, const ttl_noise* nz,
-                             int32_t n_upper, void* stream);
+/* Where the actions of a step come from: exactly one of `actions` and `head_partial`.  Host structure read
+ * at call time.
+ * head_partial: the actor's fused head, the pointers ttl_actor_head_partial returns after a forward with
+ * action == NULL -- [n_alive][n_tiles][8] fp32 per-column-tile partial sums of the 6-wide output layer
+ * (tiles_per_256 = 256 / tile width of the launch that wrote them), head_bias [6].  The sums follow the same
+ * fixed tree as the actor's own finishing pass, so this source and ttl_actor_forward* + an action buffer
+ * give the same bits whatever the tile width; it saves one launch and the action round trip per step. */
+typedef struct ttl_step_action {
+  const float* actions;       /* [n_alive][lda] fp32 action buffer, or NULL */
+  const float* head_partial;  /* or: fused head partial sums (ttl_actor_head_partial) */
+  const float* head_bias;     /* [6], with head_partial */
+  int32_t lda;                /* floats per action row, >= 3, with actions */
+  int32_t n_tiles, tiles_per_256;
+  int32_t pad;
+} ttl_step_action;
+
+/* TrackingEnvironment.step (tracking_env.py:135-221; NoisyTrackingEnvironment.step when
+ * prm->dir_f64) for the alive rows of alive[cur]: action from `act`, optional noise added first.
+ * Normalise+scale (env.py:493-502), first-step flip, grow, stopping flags (env.py:567-603,
+ * utils.py:127-173, stopping_criteria.py:38-82), reward, ordered compaction into alive[cur^1] /
+ * ctrl[cur^1], new state rows into state[cur^1] (survivors first, in order; then refilled rows if
+ * prm->refill, or stopped rows if prm->state_stopped).
+ *   noise   [n_alive][3] f64 drawn on the host, or NULL
+ *   nz      the noise drawn on the device as described at ttl_noise: no host work, no copy and no extra
+ *           launch per step.  prm->dir_f64 must be 1 (the noisy environment's float64 directions), else
+ *           TTL_ERR_UNSUPPORTED
+ *   pol     the stochastic policy sampled inside the propagate kernel (ttl_policy): head_partial must hold
+ *           all six outputs (ttl_actor_forward* with action == NULL and probabilistic != 0)
+ *   defer   1: stop before the state rows, so that TractOracle-Net can be consulted in between
+ *           (OracleStoppingCriterion, stopping_criteria.py:113-154: stop where the score < 0.5 once the
+ *           streamline has more than min_pts_stop points; OracleReward, oracle_reward.py:45-93: `bonus` for
+ *           streamlines done this step with more than min_pts_reward points and score > 0.5):
+ *             ttl_env_step, defer = 1     propagate + LENGTH/CURVATURE/MASK + alignment reward
+ *             ttl_oracle_features_rows    resample(128)+diff of the alive streamlines   \  caller, between
+ *             ttl_oracle_forward          scores [n_alive]                              /  the two calls
+ *             ttl_env_step_finish         ORACLE flag, bonus, compaction bookkeeping, state rows
+ * The combinations served (every other one is TTL_ERR_BAD_ARG):
+ *   action from      noise            pol      defer
+ *   actions          none / noise     -        0 or 1     the actor's head run on its own (with ttl_policy_eps
+ *                    / nz                                 at prob > 0 and a policy seed)
+ *   head_partial     none / nz        -        0          tanh(mu), the deterministic policy that tracking uses
+ *                                                         (prob = 0: tracker.py:28, ttl_track.py:172-175;
+ *                                                         offpolicy.py:126-128 with std * 0)
+ *   head_partial     none / nz        pol      0          the stochastic policy
+ * `n_upper` >= current alive count bounds the launch (the kernels read the true count from
+ * ctrl[cur] on the device, so no host sync is needed between steps).
+ * The caller flips cur afterwards: that flip is TrackingEnvironment.harvest (:223-245). */
+int ttl_env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                 const ttl_step_action* act, const double* noise, const ttl_noise* nz, const ttl_policy* pol,
+                 int32_t defer, int32_t n_upper, void* stream);
+int ttl_env_step_finish(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                        const float* scores, int32_t use_stop, int32_t min_pts_stop, int32_t min_pts_reward,
+                        float bonus, int32_t n_upper, void* stream);
+
 /* eps [rank][ld] fp32 (ld >= 3) for every rank of alive[cur], in rank order: the draws the fused route
  * makes, for the routes that run the actor's head on its own (ttl_actor_forward* with eps).  (row, L) come
  * from rank_rec[cur], the alive count from ctrl[cur]; ranks beyond it are not written. */
@@ -364,7 +357,9 @@ int ttl_actor_plan_refresh(ttl_actor_plan* plan, void* stream);
  * (may be NULL), pre [n][2*action] raw network output (may be NULL), in the plan's precision.
  * n is read from *n_rows_dev when that is non-NULL (no host sync), else n_rows_max.
  * eps [n][3] fp32 may be NULL when probabilistic == 0.  action == NULL (tensor-core tiers with the
- * output layer fused): stop after the last hidden layer, see ttl_actor_head_partial. */
+ * output layer fused; eps, logp and pre NULL): stop after the last hidden layer, see ttl_actor_head_partial;
+ * probabilistic != 0 then keeps the log_std partials too, for the policy ttl_env_step samples (the mu
+ * partials are the bits the deterministic call leaves). */
 int ttl_actor_forward(ttl_actor_plan* plan, const float* state, int32_t ld_state,
                       const int32_t* n_rows_dev, int32_t n_rows_max, float probabilistic,
                       const float* eps, float* action, float* logp, float* pre, void* stream);
@@ -379,20 +374,11 @@ int ttl_actor_forward_packed(ttl_actor_plan* plan, const void* state_op, int32_t
 /* With action == NULL (and logp == pre == NULL) ttl_actor_forward_packed stops after the last
  * tensor-core layer when the 6-wide output layer is fused into it: the per-tile partial sums of
  * mu / log_std stay in the plan's scratch and this call -- made AFTER the forward, the tile width is
- * chosen per launch -- returns where and in which geometry (see ttl_env_step_head):
+ * chosen per launch -- returns where and in which geometry (see ttl_step_action):
  * partial [rows][n_tiles][8] fp32, tiles_per_256 = 256 / tile width.
  * TTL_ERR_UNSUPPORTED when the plan's output layer is not fused. */
 int ttl_actor_head_partial(const ttl_actor_plan* plan, const float** partial, int32_t* n_tiles,
                            int32_t* tiles_per_256, const float** bias);
-/* ttl_actor_forward / ttl_actor_forward_packed with action == NULL for the stochastic policy: the
- * partial sums of all six outputs (mu and log_std) stay in the plan's scratch, for
- * ttl_env_step_head_policy.  The mu partials are the bits the deterministic call leaves.  Tensor-core
- * tiers with the output layer fused only (else TTL_ERR_BAD_ARG / TTL_ERR_UNSUPPORTED). */
-int ttl_actor_forward_policy_partial(ttl_actor_plan* plan, const float* state, int32_t ld_state,
-                                     const int32_t* n_rows_dev, int32_t n_rows_max, void* stream);
-int ttl_actor_forward_packed_policy_partial(ttl_actor_plan* plan, const void* state_op, int32_t ld,
-                                            int32_t rows_alloc, const int32_t* n_rows_dev, int32_t n_rows_max,
-                                            int32_t layout, void* stream);
 /* fp16 tier: 1 when a state or activation value was outside +-65504 and was saturated since the last
  * clearing call (synchronises `stream`).  The caller should then re-run in tf32. */
 int ttl_actor_overflow(ttl_actor_plan* plan, int32_t* out_host, int32_t clear, void* stream);

@@ -59,12 +59,12 @@ def test_philox_normals_shape_and_dependence():
     assert not np.array_equal(big, N.philox_normals(3, np.asarray([7]), 5))
 
 
-def test_noise_entry_points_are_exported_and_bound_in_abi_v4():
+def test_noise_entry_points_are_exported_and_bound_in_abi_v5():
     build.build()
     lib = _lib.load()
-    for name in ('ttl_env_step_rng', 'ttl_env_step_head_rng', 'ttl_env_step_begin_rng', 'ttl_noise_normals'):
+    for name in ('ttl_env_step', 'ttl_noise_normals'):
         assert hasattr(lib, name) and name in _lib.SIGNATURES, name
-    assert lib.ttl_abi_version() == _lib.ABI_VERSION == 4
+    assert lib.ttl_abi_version() == _lib.ABI_VERSION == 5
 
 
 def test_noise_struct_layout_matches_header():

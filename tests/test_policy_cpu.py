@@ -17,8 +17,7 @@ from tests import policy_oracle as PO
 from tracktolearn_b200 import _lib, build
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-NEW_SYMBOLS = ('ttl_env_step_head_policy', 'ttl_policy_eps', 'ttl_actor_forward_policy_partial',
-               'ttl_actor_forward_packed_policy_partial')
+NEW_SYMBOLS = ('ttl_env_step', 'ttl_policy_eps')
 
 
 def test_policy_eps_is_independent_of_the_noise_under_one_seed():
@@ -49,7 +48,7 @@ def test_policy_actions_at_prob_zero_are_tanh_mu():
     assert not np.array_equal(PO.policy_actions(pre, eps, 1.0), np.tanh(pre[:, :3]))
 
 
-def test_policy_entry_points_are_exported_and_bound():
+def test_policy_entry_points_are_exported_and_bound_in_abi_v5():
     build.build()
     lib = _lib.load()
     for name in NEW_SYMBOLS:

@@ -166,7 +166,7 @@ def test_seeded_policy_tractogram_does_not_depend_on_scheduling(sigma):
 
 
 def _policy_step_loop(env, alg, seed, prob, slots=256):
-    """ttl_env_step_head_policy driven by hand until every streamline stopped."""
+    """ttl_env_step with the head partials and the policy, driven by hand until every streamline stopped."""
     n = len(env.seeds)
     env.reset_streaming(0, n, slots, fp32_state=False, operand='fp16')
     actor = alg.agent.actor
@@ -177,7 +177,7 @@ def _policy_step_loop(env, alg, seed, prob, slots=256):
                                               n_rows_dev=env.alive_count_tensor(), layout=env.bf16_layout,
                                               state=env.current_state(), policy=True)
             assert head is not None
-            env.step_device_head_policy(head, pol)
+            env.step_device(head=head, policy=pol)
             env.harvest_device()
         if env.n_alive() == 0:
             break
@@ -185,7 +185,7 @@ def _policy_step_loop(env, alg, seed, prob, slots=256):
     return tr.data, np.asarray(tr.offsets), np.asarray(tr.data_per_streamline['flags'])
 
 
-def test_policy_step_at_prob_zero_is_the_deterministic_step():
+def test_single_step_entry_with_policy_at_prob_zero_is_the_deterministic_step():
     env, alg, seeds = _setup()
     n = len(seeds)
     det = _episode(env, alg, 0, n, slots=256, prob=0.0, seed=None)

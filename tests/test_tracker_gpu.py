@@ -164,7 +164,7 @@ def test_bf16_only_state_mode_tracks_the_same_streamlines(prec):
 @pytest.mark.parametrize('prec', TC)
 def test_fused_head_step_is_bit_identical_to_action_round_trip(prec):
     """Device loop with the env step reading tanh(mu) from the actor's fused output layer
-    (ttl_env_step_head) vs actor -> action buffer -> ttl_env_step: same streamlines, bit for bit,
+    (ttl_env_step with the head partials) vs actor -> action buffer -> ttl_env_step: same streamlines, bit for bit,
     in both state modes."""
     env, alg, sub, seeds, sd = _setup(precision=prec)
     n = len(seeds)

@@ -15,7 +15,7 @@ PRECISION_BF16, PRECISION_FP32, PRECISION_FP16, PRECISION_TF32 = 0, 1, 2, 3
 PRECISIONS = {'bf16': PRECISION_BF16, 'fp32': PRECISION_FP32, 'fp16': PRECISION_FP16, 'tf32': PRECISION_TF32}
 OPERAND_BF16, OPERAND_FP16, OPERAND_TF32 = 0, 1, 2
 OPERAND_OF_PRECISION = {'bf16': OPERAND_BF16, 'fp16': OPERAND_FP16, 'tf32': OPERAND_TF32}
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 
 class Volume(ctypes.Structure):
@@ -50,6 +50,13 @@ class Policy(ctypes.Structure):
     _fields_ = [('seed', ctypes.c_uint64), ('row_base', c_i64), ('prob', c_f32), ('pad', c_i32)]
 
 
+class StepAction(ctypes.Structure):
+    """ttl_step_action: where the actions of an env step come from -- an action buffer or the actor's fused
+    head partials (include/ttl_b200.h)."""
+    _fields_ = [('actions', c_vp), ('head_partial', c_vp), ('head_bias', c_vp), ('lda', c_i32), ('n_tiles', c_i32),
+                ('tiles_per_256', c_i32), ('pad', c_i32)]
+
+
 class ActorWeights(ctypes.Structure):
     _fields_ = [('n_layers', c_i32), ('in_dim', c_i32 * MAX_LAYERS), ('out_dim', c_i32 * MAX_LAYERS),
                 ('w', c_vp * MAX_LAYERS), ('b', c_vp * MAX_LAYERS)]
@@ -75,17 +82,10 @@ SIGNATURES = {
     'ttl_peaks_from_sh': (c_i32, [c_vp, c_i64, c_i32, c_i32, c_vp, c_vp, c_vp, c_i32, c_i32, c_f64, c_f64, c_f64,
                                   c_i32, c_vp, c_vp]),
     'ttl_env_reset': (c_i32, [P(Volume), P(Params), P(Batch), c_vp, c_vp]),
-    'ttl_env_step': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_vp, c_i32, c_vp]),
-    'ttl_env_step_head': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_i32, c_vp, c_i32, c_vp]),
-    'ttl_env_step_begin': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_vp, c_i32, c_vp]),
+    'ttl_env_step': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, P(StepAction), c_vp, P(Noise), P(Policy), c_i32,
+                             c_i32, c_vp]),
     'ttl_env_step_finish': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_i32, c_i32, c_f32, c_i32, c_vp]),
-    'ttl_env_step_rng': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, P(Noise), c_i32, c_vp]),
-    'ttl_env_step_head_rng': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_i32, c_vp, P(Noise), c_i32,
-                                      c_vp]),
-    'ttl_env_step_begin_rng': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, P(Noise), c_i32, c_vp]),
     'ttl_noise_normals': (c_i32, [P(Noise), c_vp, c_vp, c_i32, c_vp, c_vp]),
-    'ttl_env_step_head_policy': (c_i32, [P(Volume), P(Params), P(Batch), c_i32, c_vp, c_i32, c_i32, c_vp, P(Policy),
-                                         P(Noise), c_i32, c_vp]),
     'ttl_policy_eps': (c_i32, [P(Policy), P(Batch), c_i32, c_i32, c_vp, c_i32, c_vp]),
     'ttl_oracle_features_rows': (c_i32, [P(Batch), c_i32, c_i32, c_vp, c_vp]),
     'ttl_env_gather_step_state': (c_i32, [P(Batch), c_i32, c_i32, c_vp, c_i32, c_vp]),
@@ -107,8 +107,6 @@ SIGNATURES = {
     'ttl_actor_forward': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'ttl_actor_forward_packed': (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_i32, c_f32, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp]),
     'ttl_actor_head_partial': (c_i32, [c_vp, P(c_vp), P(c_i32), P(c_i32), P(c_vp)]),
-    'ttl_actor_forward_policy_partial': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_vp]),
-    'ttl_actor_forward_packed_policy_partial': (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_i32, c_i32, c_vp]),
     'ttl_actor_overflow': (c_i32, [c_vp, P(c_i32), c_i32, c_vp]),
     'ttl_actor_plan_set_layout': (c_i32, [c_vp, c_i32, c_i32, c_i32, c_vp]),
     'ttl_gemm_tc': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp, c_i32, c_i32, c_vp]),

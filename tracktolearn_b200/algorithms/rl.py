@@ -54,10 +54,7 @@ class StepRunner(object):
                                                    n_rows_dev=env.alive_count_tensor(), layout=env.bf16_layout,
                                                    state=env.current_state(), policy=sampled)
             if head is not None:
-                if sampled:
-                    env.step_device_head_policy(head, pol)
-                else:
-                    env.step_device_head(head)
+                env.step_device(head=head, policy=pol)
                 env.harvest_device()
                 return
             self.fuse_head = False

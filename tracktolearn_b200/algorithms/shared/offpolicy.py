@@ -189,18 +189,11 @@ class MaxEntropyActor(object):
             eps = torch.randn((rows, A), dtype=torch.float32, device=self.device)
         self._ensure_plan(rows)
         if self._operand_matches(state_bf16):
-            lay = 0
-            if layout is not None and layout[0] == 1:
-                lay = 1
-                if self._plan_layout != tuple(layout):
-                    _lib.check(self._lib.ttl_actor_plan_set_layout(
-                        self._plan, int(layout[1]), int(layout[2]), int(layout[3]),
-                        _lib.stream_ptr(self.device)), 'ttl_actor_plan_set_layout')
-                    self._plan_layout = tuple(layout)
             _lib.check(self._lib.ttl_actor_forward_packed(
                 self._plan, _lib.ptr(state_bf16), int(state_bf16.stride(0)), int(state_bf16.shape[0]),
                 _lib.ptr(n_rows_dev), rows, float(probabilistic), _lib.ptr(eps), _lib.ptr(action),
-                _lib.ptr(logp), _lib.ptr(pre), lay, _lib.stream_ptr(self.device)), 'ttl_actor_forward_packed')
+                _lib.ptr(logp), _lib.ptr(pre), self._set_layout(layout), _lib.stream_ptr(self.device)),
+                'ttl_actor_forward_packed')
             self._keep = (state_bf16, eps)
             return action, logp, pre
         if state is None:
@@ -214,14 +207,26 @@ class MaxEntropyActor(object):
         self._keep = (state, eps)
         return action, logp, pre
 
+    def _set_layout(self, layout):
+        """The plan's first-layer column layout for the env's operand rows (``env.bf16_layout``): 1 for the
+        channel-padded rows (their weight copy packed once per layout), else 0."""
+        if layout is None or layout[0] != 1:
+            return 0
+        if self._plan_layout != tuple(layout):
+            _lib.check(self._lib.ttl_actor_plan_set_layout(
+                self._plan, int(layout[1]), int(layout[2]), int(layout[3]),
+                _lib.stream_ptr(self.device)), 'ttl_actor_plan_set_layout')
+            self._plan_layout = tuple(layout)
+        return 1
+
     def forward_head_partial(self, state_bf16, n_rows, n_rows_dev=None, layout=None, state=None, policy=False):
         """Deterministic policy (prob = 0) for the device loop: runs the tensor-core layers over the
         env's operand rows (or, when their element type is not this actor's, over ``state``: the fp32 rows,
         packed first) and leaves the 6-wide output layer as per-tile partial sums in the plan's scratch.
-        Returns (partial_ptr, n_tiles, tiles_per_256, bias_ptr) for ``env.step_device_head``, or None when
+        Returns (partial_ptr, n_tiles, tiles_per_256, bias_ptr) for ``env.step_device(head=...)``, or None when
         this actor cannot do it (fp32 tier, output layer not fused, no usable rows).
         ``policy=True``: the partials of all six outputs (mu and log_std) for the stochastic policy that
-        ``env.step_device_head_policy`` samples; the mu partials are the same bits."""
+        ``env.step_device(head=..., policy=...)`` samples; the mu partials are the same bits."""
         packed = self._operand_matches(state_bf16)
         if self.precision not in self._OPERAND_DTYPES or (not packed and state is None):
             return None
@@ -234,36 +239,18 @@ class MaxEntropyActor(object):
                                                     ctypes.byref(per256), ctypes.byref(bias))
         if query() != 0:          # the output layer is not fused into the last hidden layer
             return None
+        probabilistic = 1.0 if policy else 0.0      # with no action buffer: keep the log_std partials too
         if rows > 0 and packed:
-            lay = 0
-            if layout is not None and layout[0] == 1:
-                lay = 1
-                if self._plan_layout != tuple(layout):
-                    _lib.check(self._lib.ttl_actor_plan_set_layout(
-                        self._plan, int(layout[1]), int(layout[2]), int(layout[3]),
-                        _lib.stream_ptr(self.device)), 'ttl_actor_plan_set_layout')
-                    self._plan_layout = tuple(layout)
-            if policy:
-                _lib.check(self._lib.ttl_actor_forward_packed_policy_partial(
-                    self._plan, _lib.ptr(state_bf16), int(state_bf16.stride(0)), int(state_bf16.shape[0]),
-                    _lib.ptr(n_rows_dev), rows, lay, _lib.stream_ptr(self.device)),
-                    'ttl_actor_forward_packed_policy_partial')
-            else:
-                _lib.check(self._lib.ttl_actor_forward_packed(
-                    self._plan, _lib.ptr(state_bf16), int(state_bf16.stride(0)), int(state_bf16.shape[0]),
-                    _lib.ptr(n_rows_dev), rows, 0.0, None, None, None, None, lay,
-                    _lib.stream_ptr(self.device)), 'ttl_actor_forward_packed')
+            _lib.check(self._lib.ttl_actor_forward_packed(
+                self._plan, _lib.ptr(state_bf16), int(state_bf16.stride(0)), int(state_bf16.shape[0]),
+                _lib.ptr(n_rows_dev), rows, probabilistic, None, None, None, None, self._set_layout(layout),
+                _lib.stream_ptr(self.device)), 'ttl_actor_forward_packed')
             self._keep = (state_bf16, None)
         elif rows > 0:
             ld = state.stride(0) if state.shape[0] > 1 else state.shape[1]
-            if policy:
-                _lib.check(self._lib.ttl_actor_forward_policy_partial(
-                    self._plan, _lib.ptr(state), int(ld), _lib.ptr(n_rows_dev), rows,
-                    _lib.stream_ptr(self.device)), 'ttl_actor_forward_policy_partial')
-            else:
-                _lib.check(self._lib.ttl_actor_forward(
-                    self._plan, _lib.ptr(state), int(ld), _lib.ptr(n_rows_dev), rows, 0.0, None, None, None, None,
-                    _lib.stream_ptr(self.device)), 'ttl_actor_forward')
+            _lib.check(self._lib.ttl_actor_forward(
+                self._plan, _lib.ptr(state), int(ld), _lib.ptr(n_rows_dev), rows, probabilistic, None, None, None,
+                None, _lib.stream_ptr(self.device)), 'ttl_actor_forward')
             self._keep = (state, None)
         query()                   # the geometry of the partials depends on the launch just made
         return partial.value, int(n_tiles.value), int(per256.value), bias.value

@@ -12,7 +12,7 @@
 //                through dependency flags; operands in bf16, fp16 or tf32 (TTL_PRECISION_*)
 //   head         the last (6-wide) layer is contracted in fp32 inside the last hidden layer's epilogue
 //                (per-tile partial sums); head_finish_kernel -- or the env step itself
-//                (ttl_env_step_head) -- sums them and applies clamp / exp / tanh / log-prob.
+//                (ttl_env_step, ttl_step_action) -- sums them and applies clamp / exp / tanh / log-prob.
 // A CUDA-core fp32 tier (TTL_PRECISION_FP32) reproduces the reference's fp32 arithmetic to ~1e-6 for
 // parity tests and users who want it.
 #include <cuda.h>
@@ -511,7 +511,7 @@ void pack_weights(ttl_actor_plan* p, cudaStream_t s) {
 // map_a0: TMA map of the first layer's operand rows [rows][k_pad[0]].
 int run_tc_layers(ttl_actor_plan* p, const CUtensorMap& map_a0, const int32_t* n_rows_dev, int32_t n_rows_max,
                   float probabilistic, const float* eps, float* action, float* logp, float* pre, cudaStream_t s,
-                  bool alt_w0 = false, bool policy_partial = false) {
+                  bool alt_w0 = false) {
   const ttl_actor_weights& w = p->w;
   const int nl = w.n_layers, nh = nl - 1;     // nh tensor-core layers
   const int n_out = w.out_dim[nl - 1], k_last = w.in_dim[nl - 1];
@@ -519,9 +519,9 @@ int run_tc_layers(ttl_actor_plan* p, const CUtensorMap& map_a0, const int32_t* n
   for (int i = 0; i < nh; ++i) max_np = p->n_pad[i] > max_np ? p->n_pad[i] : max_np;
   const int bn = choose_bn(n_rows_max, max_np);
   const int bi = bn_index(bn);
-  // only mu is needed when nothing reads log_std: deterministic policy, no log-prob, no raw output, no
-  // sampling in the env step (policy_partial)
-  const int head_n = (p->fuse_head && probabilistic == 0.f && !logp && !pre && !policy_partial) ? n_out / 2 : n_out;
+  // only mu is needed when nothing reads log_std: deterministic policy, no log-prob, no raw output (with
+  // action == NULL, probabilistic != 0 leaves the log_std partials for the policy the env step samples)
+  const int head_n = (p->fuse_head && probabilistic == 0.f && !logp && !pre) ? n_out / 2 : n_out;
 
   auto fill_layer = [&](MlpMaps& maps, MlpArgs& a, int slot, int i) {
     maps.a[slot] = i == 0 ? map_a0 : p->map_a[i];
@@ -713,7 +713,7 @@ int ttl_actor_forward(ttl_actor_plan* p, const float* state, int32_t ld_state, c
                       float* logp, float* pre, void* stream) {
   if (!p || !state || n_rows_max > p->max_rows) return TTL_ERR_BAD_ARG;
   if (!action && (logp || pre || eps || !p->fuse_head || p->kind < 0)) return TTL_ERR_BAD_ARG;
-  if (probabilistic != 0.f && !eps) return TTL_ERR_BAD_ARG;
+  if (probabilistic != 0.f && !eps && action) return TTL_ERR_BAD_ARG;
   if (n_rows_max <= 0) return 0;
   cudaStream_t s = (cudaStream_t)stream;
   const ttl_actor_weights& w = p->w;
@@ -770,39 +770,13 @@ int ttl_actor_forward_packed(ttl_actor_plan* p, const void* state_op, int32_t ld
   if (!action && (logp || pre || eps || !p->fuse_head)) return TTL_ERR_BAD_ARG;
   if (layout != 0 && !(layout == 1 && p->has_alt)) return TTL_ERR_BAD_ARG;
   if (ld != p->k_pad[0] || (reinterpret_cast<uintptr_t>(state_op) & 15)) return TTL_ERR_BAD_ARG;
-  if (probabilistic != 0.f && !eps) return TTL_ERR_BAD_ARG;
+  if (probabilistic != 0.f && !eps && action) return TTL_ERR_BAD_ARG;
   if (n_rows_max <= 0) return 0;
   const CUtensorMap* map = nullptr;
   int rc = ext_map(p, state_op, ld, rows_alloc, &map);
   if (rc) return rc;
   return run_tc_layers(p, *map, n_rows_dev, n_rows_max, probabilistic, eps, action, logp, pre,
                        (cudaStream_t)stream, layout == 1);
-}
-
-int ttl_actor_forward_policy_partial(ttl_actor_plan* p, const float* state, int32_t ld_state,
-                                     const int32_t* n_rows_dev, int32_t n_rows_max, void* stream) {
-  if (!p || !state || p->kind < 0 || n_rows_max > p->max_rows) return TTL_ERR_BAD_ARG;
-  if (!p->fuse_head) return TTL_ERR_UNSUPPORTED;
-  if (n_rows_max <= 0) return 0;
-  cudaStream_t s = (cudaStream_t)stream;
-  pack_state(p, state, ld_state, n_rows_dev, n_rows_max, s);
-  return run_tc_layers(p, p->map_a[0], n_rows_dev, n_rows_max, 0.f, nullptr, nullptr, nullptr, nullptr, s,
-                       false, true);
-}
-
-int ttl_actor_forward_packed_policy_partial(ttl_actor_plan* p, const void* state_op, int32_t ld,
-                                            int32_t rows_alloc, const int32_t* n_rows_dev, int32_t n_rows_max,
-                                            int32_t layout, void* stream) {
-  if (!p || !state_op || p->kind < 0 || n_rows_max > p->max_rows || n_rows_max > rows_alloc) return TTL_ERR_BAD_ARG;
-  if (!p->fuse_head) return TTL_ERR_UNSUPPORTED;
-  if (layout != 0 && !(layout == 1 && p->has_alt)) return TTL_ERR_BAD_ARG;
-  if (ld != p->k_pad[0] || (reinterpret_cast<uintptr_t>(state_op) & 15)) return TTL_ERR_BAD_ARG;
-  if (n_rows_max <= 0) return 0;
-  const CUtensorMap* map = nullptr;
-  int rc = ext_map(p, state_op, ld, rows_alloc, &map);
-  if (rc) return rc;
-  return run_tc_layers(p, *map, n_rows_dev, n_rows_max, 0.f, nullptr, nullptr, nullptr, nullptr,
-                       (cudaStream_t)stream, layout == 1, true);
 }
 
 int ttl_actor_head_partial(const ttl_actor_plan* p, const float** partial, int32_t* n_tiles,

@@ -532,7 +532,7 @@ __global__ void __launch_bounds__(kK1Threads, 6) propagate_stop_kernel(
   propagate_stop_body<RNG, false>(v, prm, b, cur, src, noise, defer, nz, ttl_policy{0, 0, 0.f, 0});
 }
 
-// The fused-head step with the stochastic policy sampled in the kernel (ttl_env_step_head_policy);
+// The fused-head step with the stochastic policy sampled in the kernel (ttl_env_step with `pol`);
 // NOISE: device-drawn tracking noise on top (dir_f64 only).  Never deferred: no oracle on this route.
 template <bool NOISE>
 __global__ void __launch_bounds__(kK1Threads, 6) propagate_policy_kernel(
@@ -1331,59 +1331,6 @@ int ttl_env_reset(const ttl_volume* vol, const ttl_params* prm, const ttl_batch*
   return 0;
 }
 
-// propagate_stop_kernel is latency-bound (a short dependent chain per streamline and ~90 registers
-// of fp64 spline state): how many 128-thread CTAs share an SM decides how many waves 50 000 rows
-// take.  It is built for 6 CTAs per SM (80 registers); 5 (94 registers, what ptxas picks
-// unconstrained) and 8 (64, a few spilled doubles) were measured and not adopted.
-extern "C++" {   // (inside the extern "C" block)
-template <bool RNG>
-static void launch_propagate_as(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
-                                const ActionSrc& src, const double* noise, int defer, const ttl_noise& nz,
-                                int grid, cudaStream_t s) {
-  TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<RNG>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, nz));
-}
-template <bool NOISE>
-static void launch_policy_as(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
-                             const ActionSrc& src, const ttl_noise& nz, const ttl_policy& pol, int grid,
-                             cudaStream_t s) {
-  TTL_LAUNCH("propagate_policy_kernel", s, ttl_launch_chain(propagate_policy_kernel<NOISE>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, nz, pol));
-}
-}  // extern "C++"
-
-// nz != NULL: the noise is drawn in the kernel (ttl_noise) and `noise` must be NULL
-static void launch_propagate(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
-                             const ActionSrc& src, const double* noise, int defer, int n_upper, cudaStream_t s,
-                             const ttl_noise* nz = nullptr) {
-  const int grid = ttl_div_up(n_upper, kGroup);
-  if (nz)
-    launch_propagate_as<true>(vol, prm, b, cur, src, nullptr, defer, *nz, grid, s);
-  else
-    launch_propagate_as<false>(vol, prm, b, cur, src, noise, defer, ttl_noise{0.0, 0, 0}, grid, s);
-}
-
-// nz != NULL: device-drawn noise on top of the sampled policy
-static void launch_propagate_policy(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
-                                    const ActionSrc& src, const ttl_policy& pol, const ttl_noise* nz,
-                                    int n_upper, cudaStream_t s) {
-  const int grid = ttl_div_up(n_upper, kGroup);
-  if (nz)
-    launch_policy_as<true>(vol, prm, b, cur, src, *nz, pol, grid, s);
-  else
-    launch_policy_as<false>(vol, prm, b, cur, src, ttl_noise{0.0, 0, 0}, pol, grid, s);
-}
-
-static int check_policy(const ttl_policy* pol) {
-  if (!pol || !(pol->prob >= 0.f) || isinf(pol->prob)) return TTL_ERR_BAD_ARG;
-  return 0;
-}
-
-// the device-noise entry points need the float64 direction arithmetic the noise is defined in
-static int check_noise(const ttl_params* prm, const ttl_noise* nz) {
-  if (!prm || !nz || !(nz->sigma >= 0.0) || isinf(nz->sigma)) return TTL_ERR_BAD_ARG;
-  if (!prm->dir_f64) return TTL_ERR_UNSUPPORTED;
-  return 0;
-}
-
 static int launch_build_state(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int cur,
                               int n_upper, cudaStream_t s) {
   int rc = state_kernels_ready();
@@ -1409,8 +1356,28 @@ static int launch_build_state(const ttl_volume* vol, const ttl_params* prm, cons
   return 0;
 }
 
-static int check_step_args(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                           int32_t* n_upper) {
+// The combinations ttl_env_step serves (include/ttl_b200.h), checked before any CUDA call: the noise and
+// policy values first, then -- when there is something to launch -- the action source and the batch.
+// Returns 0 with *n_upper <= 0 when nothing is alive.
+static int check_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                      const ttl_step_action* act, const double* noise, const ttl_noise* nz, const ttl_policy* pol,
+                      int32_t defer, int32_t* n_upper) {
+  if (!act || (act->actions && act->head_partial) || (noise && nz) || (pol && act->actions) ||
+      (act->head_partial && (noise || defer)) || (defer != 0 && defer != 1))
+    return TTL_ERR_BAD_ARG;
+  if (pol && (!(pol->prob >= 0.f) || isinf(pol->prob))) return TTL_ERR_BAD_ARG;
+  if (nz) {
+    if (!prm || !(nz->sigma >= 0.0) || isinf(nz->sigma)) return TTL_ERR_BAD_ARG;
+    if (!prm->dir_f64) return TTL_ERR_UNSUPPORTED;   // the device noise is defined in float64 directions
+  }
+  if (*n_upper <= 0) return 0;   // nothing alive: no launch (and no action source to look at)
+  if (act->head_partial) {
+    if (!act->head_bias || act->n_tiles < 1 || (reinterpret_cast<uintptr_t>(act->head_partial) & 15) ||
+        (act->tiles_per_256 != 1 && act->tiles_per_256 != 2 && act->tiles_per_256 != 4))
+      return TTL_ERR_BAD_ARG;
+  } else if (!act->actions || act->lda < 3) {
+    return TTL_ERR_BAD_ARG;
+  }
   int rc = check_common(vol, prm);
   if (rc) return rc;
   if (!b || (cur != 0 && cur != 1)) return TTL_ERR_BAD_ARG;
@@ -1425,99 +1392,34 @@ static int check_step_args(const ttl_volume* vol, const ttl_params* prm, const t
   return 0;
 }
 
-static int env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                    const float* actions, int32_t lda, const double* noise, const ttl_noise* nz, int defer,
-                    int32_t n_upper, cudaStream_t s) {
-  if (n_upper <= 0) return 0;   // nothing alive: no launch (and no action buffer to look at)
-  if (!actions || lda < 3) return TTL_ERR_BAD_ARG;
-  int rc = check_step_args(vol, prm, b, cur, &n_upper);
-  if (rc) return rc;
-  const ActionSrc src = {actions, lda, nullptr, 0, 1, nullptr, n_upper};
-  launch_propagate(vol, prm, b, cur, src, noise, defer, n_upper, s, nz);
+// propagate_stop_kernel is latency-bound (a short dependent chain per streamline and ~90 registers
+// of fp64 spline state): how many 128-thread CTAs share an SM decides how many waves 50 000 rows
+// take.  It is built for 6 CTAs per SM (80 registers); 5 (94 registers, what ptxas picks
+// unconstrained) and 8 (64, a few spilled doubles) were measured and not adopted.
+int ttl_env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
+                 const ttl_step_action* act, const double* noise, const ttl_noise* nz, const ttl_policy* pol,
+                 int32_t defer, int32_t n_upper, void* stream) {
+  int rc = check_step(vol, prm, b, cur, act, noise, nz, pol, defer, &n_upper);
+  if (rc || n_upper <= 0) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  const ActionSrc src = {act->actions, act->lda, act->head_partial, act->n_tiles, act->tiles_per_256,
+                         act->head_bias, n_upper};
+  const ttl_noise z = nz ? *nz : ttl_noise{0.0, 0, 0};
+  const int grid = ttl_div_up(n_upper, kGroup);
+  if (pol && nz)
+    TTL_LAUNCH("propagate_policy_kernel", s, ttl_launch_chain(propagate_policy_kernel<true>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, z, *pol));
+  else if (pol)
+    TTL_LAUNCH("propagate_policy_kernel", s, ttl_launch_chain(propagate_policy_kernel<false>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, z, *pol));
+  else if (nz)
+    TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<true>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, z));
+  else
+    TTL_LAUNCH("propagate_stop_kernel", s, ttl_launch_chain(propagate_stop_kernel<false>, grid, kK1Threads, 0, s, *vol, *prm, *b, cur, src, noise, defer, z));
   if (!defer) {
     rc = launch_build_state(vol, prm, b, cur, n_upper, s);
     if (rc) return rc;
   }
   TTL_CHECK_LAST();
   return 0;
-}
-
-// pol != NULL: the stochastic policy is sampled in the propagate kernel (propagate_policy_kernel)
-static int env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                         const float* head_partial, int32_t n_tiles, int32_t tiles_per_256, const float* head_bias,
-                         const ttl_noise* nz, int32_t n_upper, cudaStream_t s, const ttl_policy* pol = nullptr) {
-  if (n_upper <= 0) return 0;
-  if (!head_partial || !head_bias || n_tiles < 1 || (reinterpret_cast<uintptr_t>(head_partial) & 15) ||
-      (tiles_per_256 != 1 && tiles_per_256 != 2 && tiles_per_256 != 4))
-    return TTL_ERR_BAD_ARG;
-  int rc = check_step_args(vol, prm, b, cur, &n_upper);
-  if (rc) return rc;
-  const ActionSrc src = {nullptr, 0, head_partial, n_tiles, tiles_per_256, head_bias, n_upper};
-  if (pol)
-    launch_propagate_policy(vol, prm, b, cur, src, *pol, nz, n_upper, s);
-  else
-    launch_propagate(vol, prm, b, cur, src, nullptr, 0, n_upper, s, nz);
-  rc = launch_build_state(vol, prm, b, cur, n_upper, s);
-  if (rc) return rc;
-  TTL_CHECK_LAST();
-  return 0;
-}
-
-int ttl_env_step(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                 const float* actions, int32_t lda, const double* noise, int32_t n_upper,
-                 void* stream) {
-  return env_step(vol, prm, b, cur, actions, lda, noise, nullptr, 0, n_upper, (cudaStream_t)stream);
-}
-
-int ttl_env_step_head(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                      const float* head_partial, int32_t n_tiles, int32_t tiles_per_256, const float* head_bias,
-                      int32_t n_upper, void* stream) {
-  return env_step_head(vol, prm, b, cur, head_partial, n_tiles, tiles_per_256, head_bias, nullptr, n_upper,
-                       (cudaStream_t)stream);
-}
-
-int ttl_env_step_begin(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                       const float* actions, int32_t lda, const double* noise, int32_t n_upper,
-                       void* stream) {
-  return env_step(vol, prm, b, cur, actions, lda, noise, nullptr, 1, n_upper, (cudaStream_t)stream);
-}
-
-int ttl_env_step_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                     const float* actions, int32_t lda, const ttl_noise* nz, int32_t n_upper, void* stream) {
-  int rc = check_noise(prm, nz);
-  if (rc) return rc;
-  return env_step(vol, prm, b, cur, actions, lda, nullptr, nz, 0, n_upper, (cudaStream_t)stream);
-}
-
-int ttl_env_step_head_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                          const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
-                          const float* head_bias, const ttl_noise* nz, int32_t n_upper, void* stream) {
-  int rc = check_noise(prm, nz);
-  if (rc) return rc;
-  return env_step_head(vol, prm, b, cur, head_partial, n_tiles, tiles_per_256, head_bias, nz, n_upper,
-                       (cudaStream_t)stream);
-}
-
-int ttl_env_step_begin_rng(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                           const float* actions, int32_t lda, const ttl_noise* nz, int32_t n_upper,
-                           void* stream) {
-  int rc = check_noise(prm, nz);
-  if (rc) return rc;
-  return env_step(vol, prm, b, cur, actions, lda, nullptr, nz, 1, n_upper, (cudaStream_t)stream);
-}
-
-int ttl_env_step_head_policy(const ttl_volume* vol, const ttl_params* prm, const ttl_batch* b, int32_t cur,
-                             const float* head_partial, int32_t n_tiles, int32_t tiles_per_256,
-                             const float* head_bias, const ttl_policy* pol, const ttl_noise* nz, int32_t n_upper,
-                             void* stream) {
-  int rc = check_policy(pol);
-  if (rc) return rc;
-  if (nz) {
-    rc = check_noise(prm, nz);
-    if (rc) return rc;
-  }
-  return env_step_head(vol, prm, b, cur, head_partial, n_tiles, tiles_per_256, head_bias, nz, n_upper,
-                       (cudaStream_t)stream, pol);
 }
 
 int ttl_policy_eps(const ttl_policy* pol, const ttl_batch* b, int32_t cur, int32_t n_upper, float* eps, int32_t ld,

@@ -71,9 +71,7 @@ class NoisyTrackingEnvironment(TrackingEnvironment):
         actions = self._host_actions(actions)
         return self._step(actions, self._draw_noise((self._n_alive_host, 3)))
 
-    def step_device(self, actions, noise=None):
-        if noise is not None and self.noise_rng == 'device':
-            raise ValueError("noise_rng='device': the step kernel draws the noise; do not pass a noise array")
-        if noise is None:
+    def step_device(self, actions=None, noise=None, head=None, policy=None):
+        if noise is None and head is None:
             noise = self._draw_noise((self._n_alive_host, 3))
-        return super().step_device(actions, noise)
+        return super().step_device(actions, noise, head, policy)

@@ -236,97 +236,67 @@ class TrackingEnvironment(BaseEnv):
 
     # ------------------------------------------------------------------- device protocol
     def _device_noise(self):
-        """``_lib.Noise`` when the step kernels draw the noise themselves (ttl_env_step_rng), else None."""
+        """``_lib.Noise`` when the step kernels draw the noise themselves (ttl_noise), else None."""
         return None
-
-    def step_device(self, actions, noise=None):
-        """Enqueue one step for the alive rows.  ``actions``: CUDA float32 tensor
-        [>= n_alive, >= 3] (row stride taken from the tensor).  No host synchronisation."""
-        if self._pending_harvest:
-            raise RuntimeError('step() called twice without harvest()')
-        if actions.dtype != torch.float32 or actions.device != self.device or actions.stride(-1) != 1:
-            actions = actions.to(self.device, dtype=torch.float32).contiguous()
-        lda = actions.stride(0) if actions.dim() == 2 and actions.shape[0] > 1 else actions.shape[-1]
-        sp = _lib.stream_ptr(self.device)
-        n_up = int(self._n_alive_host)
-        nz = self._device_noise()
-        if nz is not None and noise is not None:
-            raise ValueError('the step kernels draw the noise of this environment; no noise array is taken')
-        args = (ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
-                _lib.ptr(actions), int(lda))
-        if self._oracle is None:
-            if nz is None:
-                _lib.check(self._lib.ttl_env_step(*args, _lib.ptr(noise), n_up, sp), 'ttl_env_step')
-            else:
-                _lib.check(self._lib.ttl_env_step_rng(*args, ctypes.byref(nz), n_up, sp), 'ttl_env_step_rng')
-        else:
-            # propagate + geometric criteria, then score every alive streamline, then ORACLE flag /
-            # bonus / compaction / state rows
-            if nz is None:
-                _lib.check(self._lib.ttl_env_step_begin(*args, _lib.ptr(noise), n_up, sp), 'ttl_env_step_begin')
-            else:
-                _lib.check(self._lib.ttl_env_step_begin_rng(*args, ctypes.byref(nz), n_up, sp),
-                           'ttl_env_step_begin_rng')
-            if n_up > 0:
-                slots = self._b.n_slots
-                if getattr(self, '_oracle_dirs', None) is None or self._oracle_dirs.shape[0] < slots:
-                    self._oracle_dirs = torch.empty((slots, 127, 3), dtype=torch.float32, device=self.device)
-                    self._oracle_scores = torch.zeros((slots,), dtype=torch.float32, device=self.device)
-                _lib.check(self._lib.ttl_oracle_features_rows(ctypes.byref(self._b), self._cur, n_up,
-                                                              _lib.ptr(self._oracle_dirs), sp),
-                           'ttl_oracle_features_rows')
-                self._oracle.forward_dirs(self._oracle_dirs, _lib.ptr(self._oracle_scores), n_up)
-                bonus = float(self.oracle_bonus) if self.compute_reward else 0.0
-                _lib.check(self._lib.ttl_env_step_finish(
-                    ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
-                    _lib.ptr(self._oracle_scores), int(bool(self.oracle_stopping_criterion)),
-                    int(self.min_nb_steps * 5), int(self.min_nb_steps), bonus, n_up, sp), 'ttl_env_step_finish')
-        self._keep = (actions, noise)
-        self.length += 1
-        self._pending_harvest = True
-
-    def step_device_head(self, head):
-        """``step_device`` with the actions read straight from the actor's fused output layer
-        (``head`` = what ``actor.forward_head_partial`` returned): tanh(mu), the deterministic policy.
-        One launch less per step; same bits as forward_device + step_device."""
-        if self._pending_harvest:
-            raise RuntimeError('step() called twice without harvest()')
-        if self._oracle is not None:
-            raise RuntimeError('step_device_head does not consult the oracle; use step_device')
-        partial, n_tiles, tiles_per_256, bias = head
-        args = (ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
-                partial, int(n_tiles), int(tiles_per_256), bias)
-        nz = self._device_noise()
-        if nz is None:
-            _lib.check(self._lib.ttl_env_step_head(*args, int(self._n_alive_host), _lib.stream_ptr(self.device)),
-                       'ttl_env_step_head')
-        else:
-            _lib.check(self._lib.ttl_env_step_head_rng(*args, ctypes.byref(nz), int(self._n_alive_host),
-                                                       _lib.stream_ptr(self.device)), 'ttl_env_step_head_rng')
-        self.length += 1
-        self._pending_harvest = True
 
     def policy(self, seed, prob):
         """``_lib.Policy`` for the current batch: the stochastic policy with std scaled by ``prob``, its eps
         drawn from ``seed`` at (row_base + batch row, point count) -- ttl_policy in include/ttl_b200.h."""
         return _lib.Policy(seed=int(seed), row_base=int(self._row_base), prob=float(prob))
 
-    def step_device_head_policy(self, head, policy):
-        """``step_device_head`` with the policy sampled inside the step kernel (ttl_env_step_head_policy):
-        ``head`` must hold all six outputs (``actor.forward_head_partial(..., policy=True)``); device-drawn
-        tracking noise, if any, is added on top.  Same bits as ``policy_eps`` + the actor's head + step."""
+    def step_device(self, actions=None, noise=None, head=None, policy=None):
+        """Enqueue one step for the alive rows (ttl_env_step).  No host synchronisation.  The actions come from
+        ``actions``: CUDA float32 tensor [>= n_alive, >= 3] (row stride taken from the tensor), with an
+        optional host-drawn ``noise`` array; or from ``head``, what ``actor.forward_head_partial`` returned:
+        tanh(mu) read straight from the actor's fused output layer, one launch less per step and the same
+        bits as forward_device + step_device.  ``policy`` (``self.policy(seed, prob)``, with ``head`` only):
+        the stochastic policy sampled inside the step kernel; ``head`` must then hold all six outputs
+        (``forward_head_partial(..., policy=True)``), and gives the same bits as ``policy_eps`` + the actor's
+        head + step.  Device-drawn tracking noise, if any, is added on top."""
         if self._pending_harvest:
             raise RuntimeError('step() called twice without harvest()')
-        if self._oracle is not None:
-            raise RuntimeError('step_device_head_policy does not consult the oracle; use step_device')
-        if getattr(self, 'noise', 0.0) > 0.0 and self._device_noise() is None:
-            raise RuntimeError('host-drawn noise arrives as an array: use policy_eps and step_device')
-        partial, n_tiles, tiles_per_256, bias = head
+        if (actions is None) == (head is None):
+            raise ValueError('step_device takes either actions or head')
         nz = self._device_noise()
-        _lib.check(self._lib.ttl_env_step_head_policy(
-            ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur, partial,
-            int(n_tiles), int(tiles_per_256), bias, ctypes.byref(policy), None if nz is None else ctypes.byref(nz),
-            int(self._n_alive_host), _lib.stream_ptr(self.device)), 'ttl_env_step_head_policy')
+        if nz is not None and noise is not None:
+            raise ValueError('the step kernels draw the noise of this environment; no noise array is taken')
+        if head is not None:
+            if self._oracle is not None:
+                raise RuntimeError('the fused-head step does not consult the oracle; pass actions')
+            if getattr(self, 'noise', 0.0) > 0.0 and nz is None:
+                raise RuntimeError('host-drawn noise arrives as an array: use policy_eps and actions')
+            partial, n_tiles, tiles_per_256, bias = head
+            act = _lib.StepAction(head_partial=partial, head_bias=bias, n_tiles=int(n_tiles),
+                                  tiles_per_256=int(tiles_per_256))
+        else:
+            if actions.dtype != torch.float32 or actions.device != self.device or actions.stride(-1) != 1:
+                actions = actions.to(self.device, dtype=torch.float32).contiguous()
+            lda = actions.stride(0) if actions.dim() == 2 and actions.shape[0] > 1 else actions.shape[-1]
+            act = _lib.StepAction(actions=actions.data_ptr(), lda=int(lda))
+        sp = _lib.stream_ptr(self.device)
+        n_up = int(self._n_alive_host)
+        # with the oracle: propagate + geometric criteria, then score every alive streamline, then ORACLE flag /
+        # bonus / compaction / state rows
+        defer = int(self._oracle is not None)
+        _lib.check(self._lib.ttl_env_step(
+            ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
+            ctypes.byref(act), _lib.ptr(noise), None if nz is None else ctypes.byref(nz),
+            None if policy is None else ctypes.byref(policy), defer, n_up, sp), 'ttl_env_step')
+        if defer and n_up > 0:
+            slots = self._b.n_slots
+            if getattr(self, '_oracle_dirs', None) is None or self._oracle_dirs.shape[0] < slots:
+                self._oracle_dirs = torch.empty((slots, 127, 3), dtype=torch.float32, device=self.device)
+                self._oracle_scores = torch.zeros((slots,), dtype=torch.float32, device=self.device)
+            _lib.check(self._lib.ttl_oracle_features_rows(ctypes.byref(self._b), self._cur, n_up,
+                                                          _lib.ptr(self._oracle_dirs), sp),
+                       'ttl_oracle_features_rows')
+            self._oracle.forward_dirs(self._oracle_dirs, _lib.ptr(self._oracle_scores), n_up)
+            bonus = float(self.oracle_bonus) if self.compute_reward else 0.0
+            _lib.check(self._lib.ttl_env_step_finish(
+                ctypes.byref(self._volume), ctypes.byref(self._params), ctypes.byref(self._b), self._cur,
+                _lib.ptr(self._oracle_scores), int(bool(self.oracle_stopping_criterion)),
+                int(self.min_nb_steps * 5), int(self.min_nb_steps), bonus, n_up, sp), 'ttl_env_step_finish')
+        self._keep = (actions, noise)
         self.length += 1
         self._pending_harvest = True
 
