@@ -312,6 +312,16 @@ int ttl_select_streamlines(const int64_t* offsets, int32_t n, const uint8_t* kee
  * ttl_select_streamlines: the points copied bit for bit, one warp per streamline. */
 int ttl_gather_streamlines(const float* points, const int64_t* offsets, const int64_t* index,
                            const int64_t* out_offsets, int32_t m, float* out_points, void* stream);
+/* Streamline density and endpoint maps of n packed voxel-space streamlines, ADDED into int32 maps
+ * [nx][ny][nz] (C order, z fastest) so that calls accumulate.  The voxel of a point p is
+ * c_k = floor((double)p_k + 0.5) per axis (dipy density_map's int(p + 0.5)); the point is in the grid when
+ * 0 <= c_k < dim_k on every axis (false for NaN and +-inf).  density[v] += 1 for every streamline with at
+ * least one in-grid point in v, however often it returns there; endpoints[v] += 1 for the voxel of the first
+ * point and 1 for the voxel of the last point (a one-point streamline adds 2), when in the grid.  Either map
+ * may be NULL, not both.  *skipped (device) += the number of points outside the grid.  TTL_ERR_BAD_ARG
+ * before any CUDA call for n < 0, a non-positive dimension, nx*ny*nz >= 2^31, both maps NULL or no skipped. */
+int ttl_tract_maps(const float* points, const int64_t* offsets, int32_t n, int32_t nx, int32_t ny, int32_t nz,
+                   int32_t* density, int32_t* endpoints, int64_t* skipped, void* stream);
 
 /* ---- SAC actor (algorithms/shared/offpolicy.py:61-140, shared/utils.py:41-51) -------------- */
 

@@ -2,7 +2,8 @@
 // per streamline in Python after tracking (tracking/tracker.py:118-125) -- dipy `length` for the
 // min/max length filter and dipy `compress_streamlines` for --compress -- on packed ragged arrays
 // [total][3] fp32 + int64 offsets [n+1], one warp per streamline -- and the ordered selection that
-// keeps the streamlines passing the length filter and, optionally, the TractOracle-Net score threshold.
+// keeps the streamlines passing the length filter and, optionally, the TractOracle-Net score threshold --
+// and the streamline density and endpoint maps of the streamlines kept.
 #include <math.h>
 
 #include <cub/device/device_scan.cuh>
@@ -146,6 +147,82 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) gather_streamlines_kernel
   for (long long j = lane; j < cnt; j += 32) dst[j] = src[j];
 }
 
+// Streamline maps (DESIGN.md section 2, "Streamline maps").  The voxel of a point p is c_k = floor(p_k + 0.5)
+// per axis, computed in double where the addition is exact (dipy density_map's int(p + 0.5) without the
+// rounding a float sum would add); the point is in the grid when 0 <= c_k < dim_k on every axis, a test NaN
+// and +-inf fail.  Returns the linear index (x * ny + y) * nz + z, or -1 outside the grid.
+__device__ __forceinline__ int map_voxel(const float* p, int nx, int ny, int nz) {
+  const double cx = floor(__dadd_rn((double)p[0], 0.5));
+  const double cy = floor(__dadd_rn((double)p[1], 0.5));
+  const double cz = floor(__dadd_rn((double)p[2], 0.5));
+  if (!(cx >= 0.0 && cx < (double)nx && cy >= 0.0 && cy < (double)ny && cz >= 0.0 && cz < (double)nz)) return -1;
+  return ((int)cx * ny + (int)cy) * nz + (int)cz;
+}
+
+// Distinct voxels of one streamline kept in shared memory, per warp: 16 KB a block.  A streamline that
+// touches more distinct voxels stays exact through the rescan below, only slower.
+constexpr int kMapSeen = 512;
+
+// One warp per streamline, its points in chunks of 32.  density[v] += 1 once for every distinct in-grid voxel
+// of the streamline: in a chunk the lowest lane of each voxel (__match_any_sync) is a candidate, and a
+// candidate counts unless the voxel is already in the warp's set of the streamline's earlier voxels.  Once that
+// set has overflowed it no longer holds every earlier voxel, and a candidate it misses is compared with every
+// earlier point instead.  endpoints[v] += 1 for the first and for the last point.  Out-of-grid points are
+// summed per warp into *skipped.  Counts are integer atomics: the maps do not depend on launch order.
+__global__ void __launch_bounds__(kWarpsPerBlock * 32) tract_maps_kernel(
+    const float* __restrict__ points, const long long* __restrict__ offsets, int n, int nx, int ny, int nz,
+    int* __restrict__ density, int* __restrict__ endpoints, unsigned long long* __restrict__ skipped) {
+  __shared__ int seen_block[kWarpsPerBlock][kMapSeen];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int i = blockIdx.x * kWarpsPerBlock + warp;
+  if (i >= n) return;
+  int* seen = seen_block[warp];
+  const long long beg = offsets[i];
+  const int N = (int)(offsets[i + 1] - beg);
+  const float* P = points + beg * 3;
+  if (endpoints != nullptr && lane < 2 && N > 0) {
+    const int v = map_voxel(P + 3 * (lane == 0 ? 0 : N - 1), nx, ny, nz);
+    if (v >= 0) atomicAdd(endpoints + v, 1);
+  }
+  unsigned outside = 0;
+  int n_seen = 0;
+  bool complete = true;      // seen[] holds every in-grid voxel of the points before `base`
+  for (int base = 0; base < N; base += 32) {
+    const int j = base + lane;
+    const int v = j < N ? map_voxel(P + 3 * j, nx, ny, nz) : -1;
+    outside += (j < N && v < 0) ? 1u : 0u;
+    if (density == nullptr) continue;
+    const unsigned same = __match_any_sync(0xffffffffu, v);
+    bool cand = v >= 0 && __ffs(same) - 1 == lane;
+    for (unsigned todo = __ballot_sync(0xffffffffu, cand); todo != 0; todo &= todo - 1) {
+      const int src = __ffs(todo) - 1;
+      const int w = __shfl_sync(0xffffffffu, v, src);
+      bool hit = false;
+      for (int k = lane; k < n_seen; k += 32) hit |= seen[k] == w;
+      if (__any_sync(0xffffffffu, hit) && lane == src) cand = false;
+    }
+    if (!complete && __any_sync(0xffffffffu, cand)) {
+      bool found = false;
+      for (int b = 0; b < base; b += 32) {       // b + lane < base: base is a multiple of 32
+        const int e = map_voxel(P + 3 * (b + lane), nx, ny, nz);
+#pragma unroll
+        for (int k = 0; k < 32; ++k) found |= __shfl_sync(0xffffffffu, e, k) == v;
+      }
+      cand = cand && !found;
+    }
+    if (cand) atomicAdd(density + v, 1);
+    const unsigned add = __ballot_sync(0xffffffffu, cand);
+    const int pos = n_seen + __popc(add & ((1u << lane) - 1u));
+    if (cand && pos < kMapSeen) seen[pos] = v;
+    if (n_seen + __popc(add) > kMapSeen) complete = false;
+    n_seen = min(n_seen + __popc(add), kMapSeen);
+    __syncwarp();
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) outside += __shfl_xor_sync(0xffffffffu, outside, off);
+  if (lane == 0 && outside != 0) atomicAdd(skipped, (unsigned long long)outside);
+}
+
 size_t select_pairs_bytes(int n) { return ((size_t)n * sizeof(longlong2) + 255) / 256 * 256; }
 
 size_t select_scan_bytes(int n) {
@@ -231,6 +308,22 @@ int ttl_gather_streamlines(const float* points, const int64_t* offsets, const in
              gather_streamlines_kernel<<<ttl_div_up(m, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
                  points, (const long long*)offsets, (const long long*)index, (const long long*)out_offsets, m,
                  out_points));
+  TTL_CHECK_LAST();
+  return 0;
+}
+
+int ttl_tract_maps(const float* points, const int64_t* offsets, int32_t n, int32_t nx, int32_t ny, int32_t nz,
+                   int32_t* density, int32_t* endpoints, int64_t* skipped, void* stream) {
+  if (n < 0 || nx <= 0 || ny <= 0 || nz <= 0 || (int64_t)nx * ny * nz >= ((int64_t)1 << 31) ||
+      (!density && !endpoints) || !skipped)
+    return TTL_ERR_BAD_ARG;
+  if (n == 0) return 0;
+  if (!points || !offsets) return TTL_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  TTL_LAUNCH("tract_maps_kernel", s,
+             tract_maps_kernel<<<ttl_div_up(n, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
+                 points, (const long long*)offsets, n, nx, ny, nz, density, endpoints,
+                 (unsigned long long*)skipped));
   TTL_CHECK_LAST();
   return 0;
 }

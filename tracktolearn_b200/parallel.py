@@ -4,7 +4,7 @@ The path shards by seed (SURVEY.md section 8(e)): every rank holds a replica of 
 mask and actor, tracks its own contiguous slice of the (globally shuffled) seeds and there is
 no collective on the data path.  The only exchange is at the end: ranks send their packed
 streamlines to rank 0, which concatenates them in rank order -- the same order a single GPU
-would have produced.  Works with any ``torch.distributed`` backend (NCCL on GPUs, gloo in the
+would have produced -- and per-rank streamline maps are summed onto rank 0.  Works with any ``torch.distributed`` backend (NCCL on GPUs, gloo in the
 CPU tests): only host logic lives here.
 """
 import numpy as np
@@ -304,6 +304,22 @@ def _packed_tractogram(arrs):
     if len(arrs) > 4:
         per['oracle_score'] = arrs[4][:, 0]
     return Tractogram(data=data, offsets=offsets, data_per_streamline=per)
+
+
+def reduce_maps(maps, skipped, dst=0):
+    """Sum per-rank streamline maps onto rank `dst`: one ``dist.reduce`` (SUM) per int32 map in ``maps`` (a
+    list; None entries are passed over), in place, and one for the ``skipped`` point count.  The maps are
+    integer counts, so the sum is exact and the same for every GPU count.  Tensors live on this rank's device
+    for the backend (CUDA under NCCL, CPU under gloo).  Returns the total skipped count on `dst`, this rank's
+    count elsewhere; without torch.distributed, ``skipped`` unchanged."""
+    if not dist.is_available() or not dist.is_initialized() or dist.get_world_size() == 1:
+        return int(skipped)
+    for m in maps:
+        if m is not None:
+            dist.reduce(m, dst, op=dist.ReduceOp.SUM)
+    t = torch.tensor([int(skipped)], dtype=torch.int64, device=_device_for_backend())
+    dist.reduce(t, dst, op=dist.ReduceOp.SUM)
+    return int(t.item())
 
 
 def gather_tractogram(local, dst=0, copy=True, via='auto'):

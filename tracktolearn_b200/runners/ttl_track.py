@@ -53,6 +53,8 @@ class TrackToLearnTrack(object):
         self.oracle_threshold = float(track_dto.get('oracle_threshold', 0.5))
         self.oracle_precision = track_dto.get('oracle_precision', 'fp16')
         self.save_oracle_scores = bool(track_dto.get('save_oracle_scores', False))
+        self.out_density = track_dto.get('out_density')
+        self.out_endpoints = track_dto.get('out_endpoints')
         self.compute_reward = False
         if not torch.cuda.is_available():
             raise SystemExit('ttl_track (tracktolearn_b200) needs a CUDA device; there is no CPU path')
@@ -130,9 +132,16 @@ class TrackToLearnTrack(object):
             OracleSingleton.clear()
             oracle = OracleSingleton(self.oracle_checkpoint, self.device, precision=self.oracle_precision)
         n = tracker.track_to_file(env, self.out_tractogram, ref_img.shape[:3], ref_img.zooms[:3], oracle=oracle,
-                                  oracle_threshold=self.oracle_threshold, save_scores=self.save_oracle_scores)
+                                  oracle_threshold=self.oracle_threshold, save_scores=self.save_oracle_scores,
+                                  density_path=self.out_density, endpoints_path=self.out_endpoints)
         if int(os.environ.get('RANK', '0')) == 0:
             print('Wrote {} streamlines to {}.'.format(n, self.out_tractogram))
+            for what, path in (('density', self.out_density), ('endpoint', self.out_endpoints)):
+                if path is not None:
+                    print('Wrote the streamline {} map to {}.'.format(what, path))
+            if tracker.maps_skipped:
+                print('{} points lie outside the volume\'s grid and are not counted in the maps.'.format(
+                    tracker.maps_skipped))
         return n
 
 
@@ -224,6 +233,34 @@ def add_track_args(parser):
     oracle_g.add_argument('--save_oracle_scores', action='store_true',
                           help='Save each kept streamline\'s score as the per-streamline\nproperty '
                                '"oracle_score" (.trk only).')
+    add_map_args(parser)
+
+
+def add_map_args(p):
+    maps_g = p.add_argument_group('Maps')
+    maps_g.add_argument('--out_density', metavar='FILE', default=None,
+                        help='Streamline density map (.nii or .nii.gz, int32): for every voxel of the\n'
+                             'tracking volume, the number of streamlines with a point in it.')
+    maps_g.add_argument('--out_endpoints', metavar='FILE', default=None,
+                        help='Endpoint map (.nii or .nii.gz, int32): for every voxel, the number of\n'
+                             'streamline first and last points in it.')
+    return maps_g
+
+
+def check_map_args(parser, args, other_outputs):
+    """--out_density / --out_endpoints: NIfTI names, not existing files without -f, distinct from each other
+    and from `other_outputs`."""
+    taken = [os.path.abspath(f) for f in other_outputs]
+    for opt, path in (('--out_density', args.out_density), ('--out_endpoints', args.out_endpoints)):
+        if path is None:
+            continue
+        if not path.endswith(('.nii', '.nii.gz')):
+            parser.error('{} must be a .nii or .nii.gz file, not {}'.format(opt, path))
+        if os.path.isfile(path) and not args.overwrite:
+            parser.error('Output file {} exists. Use -f to force overwriting'.format(path))
+        if os.path.abspath(path) in taken:
+            parser.error('{} {} is also another output'.format(opt, path))
+        taken.append(os.path.abspath(path))
 
 
 def verify_agent_option(parser, args):
@@ -266,6 +303,7 @@ def parse_args(argv=None):
         parser.error('--save_oracle_scores needs a .trk output: .tck files cannot hold per-streamline data')
     if args.oracle_checkpoint and not os.path.isfile(args.oracle_checkpoint):
         parser.error('Oracle checkpoint {} does not exist'.format(args.oracle_checkpoint))
+    check_map_args(parser, args, [args.out_tractogram])
     verify_agent_option(parser, args)
     return args
 

@@ -85,3 +85,28 @@ def select_packed(data, offsets, keep=None, scores=None, threshold=0.0):
         _lib.check(lib.ttl_gather_streamlines(_lib.ptr(data), _lib.ptr(offsets), _lib.ptr(index), _lib.ptr(out_off),
                                               m, _lib.ptr(out), sp), 'ttl_gather_streamlines')
     return out, out_off[:m + 1], index[:m]
+
+
+def tract_maps_packed(data, offsets, dims, density=None, endpoints=None):
+    """Streamline density and endpoint maps of packed voxel-space streamlines (``ttl_tract_maps``), added in
+    place into int32 CUDA tensors of shape ``dims`` (X, Y, Z) on the points' device; either may be None, not
+    both.  The voxel of a point is ``floor(p + 0.5)`` per axis; ``density[v]`` counts the streamlines with a
+    point in v, ``endpoints[v]`` their first and last points in v.  Returns the number of points outside the
+    grid (one small device-to-host copy)."""
+    device = _dev(data.device)
+    lib = _lib.load()
+    data, offsets = _to_device(data, offsets, device)
+    dims = tuple(int(d) for d in dims)
+    if density is None and endpoints is None:
+        raise ValueError('tract_maps_packed needs a density map, an endpoint map or both')
+    for m in (density, endpoints):
+        if m is not None and (m.device != device or m.dtype != torch.int32 or tuple(m.shape) != dims
+                              or not m.is_contiguous()):
+            raise ValueError('maps must be contiguous int32 tensors of shape %r on %s' % (dims, device))
+    n = int(offsets.shape[0]) - 1
+    skipped = torch.zeros((1,), dtype=torch.int64, device=device)
+    with torch.cuda.device(device):
+        _lib.check(lib.ttl_tract_maps(_lib.ptr(data), _lib.ptr(offsets), max(n, 0), *dims, _lib.ptr(density),
+                                      _lib.ptr(endpoints), _lib.ptr(skipped), _lib.stream_ptr(device)),
+                   'ttl_tract_maps')
+        return int(skipped.item())

@@ -45,6 +45,7 @@ class Tracker(object):
         self.save_seeds = save_seeds
         self.streaming = streaming
         self.rows_per_pass = rows_per_pass
+        self.maps_skipped = 0       # points outside the grid in the maps of the last track_to_file
 
     # ----------------------------------------------------------------------------------
     def _passes(self, env):
@@ -148,7 +149,8 @@ class Tracker(object):
         d, o = compress_packed(data, offsets, tol_error=float(tol_vox), device=env.device)
         return d.cpu().numpy(), o.cpu().numpy()
 
-    def track_to_file(self, env, path, dims, voxel_sizes, oracle=None, oracle_threshold=0.5, save_scores=False):
+    def track_to_file(self, env, path, dims, voxel_sizes, oracle=None, oracle_threshold=0.5, save_scores=False,
+                      density_path=None, endpoints_path=None):
         """What ``ttl_track.py`` does with ``track`` + ``nib.streamlines.save`` (runners/ttl_track.py:
         172-186), on packed arrays and on the device: dipy ``length`` and the min/max filter
         (tracker.py:118-121), ``compress_streamlines`` (:123-125), voxel -> file space (:127-136);
@@ -161,9 +163,16 @@ class Tracker(object):
         comes before ``--compress``, so a score does not depend on it.  Each rank scores its own
         streamlines: a streamline's score does not depend on the batch it is scored in, so the file is
         the same for every GPU count.  ``save_scores`` (.trk only) writes the scores as the
-        per-streamline property ``oracle_score``."""
+        per-streamline property ``oracle_score``.
+
+        ``density_path`` / ``endpoints_path`` (.nii / .nii.gz): the streamline density and endpoint maps of the
+        streamlines written, on the env's voxel grid (``postprocess.tract_maps_packed``), taken from their
+        voxel-space points after the length and oracle filters and before ``--compress``; summed over the
+        ranks onto rank 0, which writes them as int32 NIfTI with ``env.affine_vox2rasmm``.  The number of
+        points outside the grid is kept in ``self.maps_skipped``."""
         from tracktolearn_b200.io.streamlines import TckWriter, TrkWriter, detect_format
-        from tracktolearn_b200.tracking.postprocess import compress_packed, lengths_packed, select_packed
+        from tracktolearn_b200.tracking.postprocess import (compress_packed, lengths_packed, select_packed,
+                                                            tract_maps_packed)
         import torch.distributed as dist
         from tracktolearn_b200 import parallel
         fmt = detect_format(path)
@@ -197,6 +206,13 @@ class Tracker(object):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             n_passes = int(t.item())
         passes = list(self._passes(env))
+        grid = (env._volume.X, env._volume.Y, env._volume.Z)
+        density = endpoints = None
+        if density_path is not None:
+            density = torch.zeros(grid, dtype=torch.int32, device=env.device)
+        if endpoints_path is not None:
+            endpoints = torch.zeros(grid, dtype=torch.int32, device=env.device)
+        skipped = 0
         try:
             for ip in range(n_passes):
                 out = torch.zeros((0, 3), dtype=torch.float32, device=env.device)
@@ -212,6 +228,8 @@ class Tracker(object):
                         scores = oracle.predict_device(data, new_off, distributed=False)
                         data, new_off, sel = select_packed(data, new_off, scores=scores, threshold=oracle_threshold)
                         index, scores_kept = index[sel], scores[sel]
+                    if density is not None or endpoints is not None:
+                        skipped += tract_maps_packed(data, new_off, grid, density, endpoints)
                     if self.compress:     # after the length filter, before the space change (tracker.py:120-129)
                         data, new_off = compress_packed(data, new_off, tol_error=float(self.compress) / float(vox_size))
                     d64 = data.to(torch.float64)
@@ -244,6 +262,14 @@ class Tracker(object):
         finally:
             if writer is not None:
                 writer.close()
+        if density is not None or endpoints is not None:
+            skipped = parallel.reduce_maps([density, endpoints], skipped)
+            if rank == 0:
+                from tracktolearn_b200.io import nifti
+                for p, m in ((density_path, density), (endpoints_path, endpoints)):
+                    if m is not None:
+                        nifti.save(p, m.cpu().numpy(), env.affine_vox2rasmm)
+        self.maps_skipped = skipped
         n = writer.n if writer is not None else 0
         if world > 1:
             t = torch.tensor([n], device=env.device)
