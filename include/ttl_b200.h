@@ -322,6 +322,27 @@ int ttl_gather_streamlines(const float* points, const int64_t* offsets, const in
  * before any CUDA call for n < 0, a non-positive dimension, nx*ny*nz >= 2^31, both maps NULL or no skipped. */
 int ttl_tract_maps(const float* points, const int64_t* offsets, int32_t n, int32_t nx, int32_t ny, int32_t nz,
                    int32_t* density, int32_t* endpoints, int64_t* skipped, void* stream);
+/* Structural connectivity matrix of n packed voxel-space streamlines over an int32 label volume
+ * labels [nx][ny][nz] (C order, z fastest; 0 = no region, a value outside [0, K) reads as 0).  The label of an
+ * endpoint p (first or last point, float32):
+ *   1. its own voxel c_k = floor((double)p_k + 0.5) (ttl_tract_maps' rule), when in the grid and labelled > 0;
+ *   2. else, over the in-grid voxels c with ceil(p_k - r) <= c_k <= floor(p_k + r) (p_k - r, p_k + r in fp64),
+ *      d2 = ((dx*dx) + (dy*dy)) + (dz*dz), dx = (double)c_x - (double)p_x, ..., every operation fp64
+ *      round-to-nearest without contraction: the label of the labelled voxel with the smallest d2 <= r*r, ties
+ *      to the smallest linear index (x*ny + y)*nz + z;
+ *   3. 0 when no voxel qualifies or a coordinate of p is NaN or +-inf.
+ * r = radius_vox; at 0 this is dipy's end-voxel rule (with 0 off the grid).  A streamline with end labels
+ * (a, b) ADDS 1 to matrix[a][a] when a == b, else 1 to matrix[a][b] and 1 to matrix[b][a] (int32 [K][K], calls
+ * accumulate; dipy connectivity_matrix(symmetric=True)); an empty streamline adds nothing.  pairs [n][2] =
+ * (a, b), unsorted; (0, 0) for an empty streamline.  Either output may be NULL, not both.  TTL_ERR_BAD_ARG
+ * before any CUDA call for n < 0, a non-positive dimension, nx*ny*nz >= 2^31, K outside
+ * [1, TTL_CONNECTOME_MAX_LABELS], radius_vox not finite or outside [0, TTL_CONNECTOME_MAX_RADIUS], both
+ * outputs NULL, no labels, or no points / offsets with n > 0. */
+#define TTL_CONNECTOME_MAX_LABELS 16384
+#define TTL_CONNECTOME_MAX_RADIUS 8.0
+int ttl_connectome(const float* points, const int64_t* offsets, int32_t n, const int32_t* labels, int32_t nx,
+                   int32_t ny, int32_t nz, int32_t K, double radius_vox, int32_t* matrix, int32_t* pairs,
+                   void* stream);
 
 /* ---- SAC actor (algorithms/shared/offpolicy.py:61-140, shared/utils.py:41-51) -------------- */
 

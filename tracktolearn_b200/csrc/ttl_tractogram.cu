@@ -3,7 +3,8 @@
 // min/max length filter and dipy `compress_streamlines` for --compress -- on packed ragged arrays
 // [total][3] fp32 + int64 offsets [n+1], one warp per streamline -- and the ordered selection that
 // keeps the streamlines passing the length filter and, optionally, the TractOracle-Net score threshold --
-// and the streamline density and endpoint maps of the streamlines kept.
+// the streamline density and endpoint maps of the streamlines kept -- and their connectivity matrix over a
+// label volume.
 #include <math.h>
 
 #include <cub/device/device_scan.cuh>
@@ -223,6 +224,95 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) tract_maps_kernel(
   if (lane == 0 && outside != 0) atomicAdd(skipped, (unsigned long long)outside);
 }
 
+// Connectivity matrix (DESIGN.md section 2, "Connectivity matrix").  A label value outside [0, K) reads as 0,
+// so no value a caller leaves in the volume can index past the matrix.
+__device__ __forceinline__ int conn_label(const int* labels, int v, int K) {
+  const int l = labels[v];
+  return (l > 0 && l < K) ? l : 0;
+}
+
+// Label of the endpoint p, computed by the whole warp (every lane returns it).  Its own voxel
+// floor((double)p + 0.5) when in the grid and labelled; otherwise the labelled voxel c of the box
+// ceil(p - r) <= c <= floor(p + r) (fp64 bounds, clamped to the grid) with the smallest
+// d2 = ((dx*dx) + (dy*dy)) + (dz*dz) <= r2, dx = (double)c - (double)p, every operation rounded to nearest with
+// no contraction; ties go to the smaller linear index.  0 when there is none or p is not finite.  Lanes take
+// the box's voxels round-robin and read a label only inside the sphere; a shuffle tree finds the minimum of
+// (d2, index).
+__device__ __forceinline__ int conn_end_label(const float* p, const int* __restrict__ labels, int nx, int ny,
+                                              int nz, int K, double r, double r2, int lane) {
+  const double px = (double)p[0], py = (double)p[1], pz = (double)p[2];
+  const int own = map_voxel(p, nx, ny, nz);
+  if (own >= 0) {
+    const int l = conn_label(labels, own, K);
+    if (l > 0) return l;
+  }
+  if (!(isfinite(px) && isfinite(py) && isfinite(pz))) return 0;
+  const double lx = fmax(ceil(__dsub_rn(px, r)), 0.0), hx = fmin(floor(__dadd_rn(px, r)), (double)(nx - 1));
+  const double ly = fmax(ceil(__dsub_rn(py, r)), 0.0), hy = fmin(floor(__dadd_rn(py, r)), (double)(ny - 1));
+  const double lz = fmax(ceil(__dsub_rn(pz, r)), 0.0), hz = fmin(floor(__dadd_rn(pz, r)), (double)(nz - 1));
+  if (!(lx <= hx && ly <= hy && lz <= hz)) return 0;
+  const int x0 = (int)lx, y0 = (int)ly, z0 = (int)lz;
+  const int by = (int)hy - y0 + 1, bz = (int)hz - z0 + 1;
+  const int plane = by * bz, count = ((int)hx - x0 + 1) * plane;
+  double best = r2;
+  int best_v = 0x7fffffff, best_l = 0;
+  for (int t = lane; t < count; t += 32) {
+    const int ix = t / plane, rem = t - ix * plane;
+    const int iy = rem / bz, iz = rem - iy * bz;
+    const int cx = x0 + ix, cy = y0 + iy, cz = z0 + iz;
+    const double d2 = sumsq3(__dsub_rn((double)cx, px), __dsub_rn((double)cy, py), __dsub_rn((double)cz, pz));
+    if (d2 <= best) {
+      const int v = (cx * ny + cy) * nz + cz;
+      const int l = conn_label(labels, v, K);
+      if (l > 0 && (d2 < best || v < best_v)) {
+        best = d2;
+        best_v = v;
+        best_l = l;
+      }
+    }
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    const double od = __shfl_xor_sync(0xffffffffu, best, off);
+    const int ov = __shfl_xor_sync(0xffffffffu, best_v, off);
+    const int ol = __shfl_xor_sync(0xffffffffu, best_l, off);
+    if (ol > 0 && (best_l == 0 || od < best || (od == best && ov < best_v))) {
+      best = od;
+      best_v = ov;
+      best_l = ol;
+    }
+  }
+  return best_l;
+}
+
+// One warp per streamline: the labels (a, b) of its first and last points.  matrix[a][a] += 1 when a == b,
+// else matrix[a][b] += 1 and matrix[b][a] += 1 (integer atomics: the matrix does not depend on launch order);
+// an empty streamline adds nothing and gets the pair (0, 0).
+__global__ void __launch_bounds__(kWarpsPerBlock * 32) connectome_kernel(
+    const float* __restrict__ points, const long long* __restrict__ offsets, int n, const int* __restrict__ labels,
+    int nx, int ny, int nz, int K, double r, int* __restrict__ matrix, int* __restrict__ pairs) {
+  const int lane = threadIdx.x & 31;
+  const int i = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
+  if (i >= n) return;
+  const long long beg = offsets[i];
+  const long long N = offsets[i + 1] - beg;
+  int a = 0, b = 0;
+  if (N > 0) {
+    const double r2 = __dmul_rn(r, r);
+    a = conn_end_label(points + beg * 3, labels, nx, ny, nz, K, r, r2, lane);
+    b = conn_end_label(points + (beg + N - 1) * 3, labels, nx, ny, nz, K, r, r2, lane);
+  }
+  if (lane != 0) return;
+  if (pairs != nullptr) {
+    pairs[2 * (long long)i] = a;
+    pairs[2 * (long long)i + 1] = b;
+  }
+  if (matrix != nullptr && N > 0) {
+    atomicAdd(matrix + a * K + b, 1);
+    if (a != b) atomicAdd(matrix + b * K + a, 1);
+  }
+}
+
 size_t select_pairs_bytes(int n) { return ((size_t)n * sizeof(longlong2) + 255) / 256 * 256; }
 
 size_t select_scan_bytes(int n) {
@@ -324,6 +414,24 @@ int ttl_tract_maps(const float* points, const int64_t* offsets, int32_t n, int32
              tract_maps_kernel<<<ttl_div_up(n, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
                  points, (const long long*)offsets, n, nx, ny, nz, density, endpoints,
                  (unsigned long long*)skipped));
+  TTL_CHECK_LAST();
+  return 0;
+}
+
+int ttl_connectome(const float* points, const int64_t* offsets, int32_t n, const int32_t* labels, int32_t nx,
+                   int32_t ny, int32_t nz, int32_t K, double radius_vox, int32_t* matrix, int32_t* pairs,
+                   void* stream) {
+  if (n < 0 || nx <= 0 || ny <= 0 || nz <= 0 || (int64_t)nx * ny * nz >= ((int64_t)1 << 31) || K < 1 ||
+      K > TTL_CONNECTOME_MAX_LABELS ||
+      !(radius_vox >= 0.0 && radius_vox <= TTL_CONNECTOME_MAX_RADIUS) ||
+      (!matrix && !pairs) || !labels)
+    return TTL_ERR_BAD_ARG;
+  if (n == 0) return 0;
+  if (!points || !offsets) return TTL_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  TTL_LAUNCH("connectome_kernel", s,
+             connectome_kernel<<<ttl_div_up(n, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
+                 points, (const long long*)offsets, n, labels, nx, ny, nz, K, radius_vox, matrix, pairs));
   TTL_CHECK_LAST();
   return 0;
 }

@@ -32,14 +32,17 @@ def _voxel_order(affine):
 
 class TrkWriter(object):
     """Streams (data, offsets) batches to a .trk file; the streamline count is patched on close.
-    Per-streamline properties: ``seeds_x/y/z`` (``save_seeds``), then ``oracle_score`` (``save_scores``)."""
+    Per-streamline properties: ``seeds_x/y/z`` (``save_seeds``), then ``oracle_score`` (``save_scores``), then
+    ``start_label`` and ``end_label`` (``save_labels``: connectivity labels, integers held exactly in float32)."""
 
-    def __init__(self, path, dims, voxel_sizes, affine, save_seeds=False, save_scores=False):
+    def __init__(self, path, dims, voxel_sizes, affine, save_seeds=False, save_scores=False, save_labels=False):
         self.f = open(path, 'wb')
         self.n = 0
         self.save_seeds = save_seeds
         self.save_scores = save_scores
-        names = ((b'seeds_x', b'seeds_y', b'seeds_z') if save_seeds else ()) + ((b'oracle_score',) if save_scores else ())
+        self.save_labels = save_labels
+        names = (((b'seeds_x', b'seeds_y', b'seeds_z') if save_seeds else ()) + ((b'oracle_score',) if save_scores else ())
+                 + ((b'start_label', b'end_label') if save_labels else ()))
         hdr = bytearray(1000)
         hdr[0:6] = b'TRACK\x00'
         struct.pack_into('<3h', hdr, 6, *[int(d) for d in dims])
@@ -57,12 +60,12 @@ class TrkWriter(object):
         struct.pack_into('<i', hdr, 996, 1000)                               # hdr_size
         self.f.write(bytes(hdr))
 
-    def write(self, data, offsets, seeds=None, scores=None):
+    def write(self, data, offsets, seeds=None, scores=None, labels=None):
         n = len(offsets) - 1
         if n <= 0:
             return
         lens = np.diff(offsets).astype(np.int64)
-        n_prop = (3 if self.save_seeds else 0) + (1 if self.save_scores else 0)
+        n_prop = (3 if self.save_seeds else 0) + (1 if self.save_scores else 0) + (2 if self.save_labels else 0)
         total = int(lens.sum()) * 3 + n * (1 + n_prop)
         out = np.empty(total, dtype='<f4')
         # positions of the int32 counts inside the float buffer
@@ -75,7 +78,11 @@ class TrkWriter(object):
             for c in range(3):
                 out[ps + c] = np.asarray(seeds, dtype=np.float32)[:, c]
         if self.save_scores:
-            out[starts + lens * 3 + n_prop] = np.asarray(scores, dtype=np.float32).reshape(-1)
+            out[starts + lens * 3 + 1 + (3 if self.save_seeds else 0)] = np.asarray(scores, dtype=np.float32).reshape(-1)
+        if self.save_labels:
+            lab = np.asarray(labels).reshape(-1, 2).astype(np.float32)
+            out[starts + lens * 3 + n_prop - 1] = lab[:, 0]
+            out[starts + lens * 3 + n_prop] = lab[:, 1]
         self.f.write(out.tobytes())
         self.n += n
 
@@ -101,8 +108,9 @@ class TckWriter(object):
         self.f.write(text.encode())
         self.offset = offset
 
-    def write(self, data, offsets, seeds=None, scores=None):
-        """``seeds`` and ``scores`` are accepted for TrkWriter's signature: .tck has no per-streamline data."""
+    def write(self, data, offsets, seeds=None, scores=None, labels=None):
+        """``seeds``, ``scores`` and ``labels`` are accepted for TrkWriter's signature: .tck has no per-streamline
+        data."""
         n = len(offsets) - 1
         if n <= 0:
             return

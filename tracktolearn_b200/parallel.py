@@ -212,7 +212,7 @@ def _gather_via_arena(parts, dst, copy):
     return out
 
 
-def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', scores=None):
+def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', scores=None, labels=None):
     """Gather packed streamlines on rank `dst` in rank order.
 
     ``via``: 'nccl' -- the data travels through NCCL to `dst`'s GPU and over its PCIe link (below);
@@ -227,8 +227,10 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', s
     point-to-point: device-to-device over NVLink under NCCL) and `dst` makes one D2H copy per array
     into grow-only pinned memory.  With ``copy=False`` the returned arrays are views of that pinned
     memory, valid until the next gather.  ``scores`` [n] float32 (optional): per-streamline oracle scores,
-    carried along and returned as ``data_per_streamline['oracle_score']``.  Returns a Tractogram on `dst`,
-    None elsewhere."""
+    carried along and returned as ``data_per_streamline['oracle_score']``.  ``labels`` [n, 2] int32 (optional):
+    the connectivity labels of every streamline's first and last points, returned as
+    ``data_per_streamline['start_label']`` and ``['end_label']``.  Returns a Tractogram on `dst`, None
+    elsewhere."""
     world, rank = dist.get_world_size(), dist.get_rank()
     dev = _device_for_backend()
     if via == 'auto':
@@ -243,11 +245,13 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', s
                  (flags.to(dtype=torch.int64).reshape(-1, 1), 1, torch.int64, 'flags')]
         if scores is not None:
             parts.append((scores.to(dtype=torch.float32).reshape(-1, 1), 1, torch.float32, 'scores'))
+        if labels is not None:
+            parts.append((labels.to(dtype=torch.int32).reshape(-1, 2), 2, torch.int32, 'labels'))
         arrs = _gather_via_arena(parts, dst, copy)
         if arrs is None:
             return None
         if not isinstance(arrs, str):
-            return _packed_tractogram(arrs)
+            return _packed_tractogram(arrs, [p[3] for p in parts])
         # the arena could not be set up on some rank (every rank knows): the NCCL route below
     parts = [(points.to(dev, dtype=torch.float32).reshape(-1, 3).contiguous(), 3, torch.float32, 'pts'),
              (lengths.to(dev, dtype=torch.int64).reshape(-1, 1).contiguous(), 1, torch.int64, 'len'),
@@ -255,6 +259,8 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', s
              (flags.to(dev, dtype=torch.int64).reshape(-1, 1).contiguous(), 1, torch.int64, 'flags')]
     if scores is not None:
         parts.append((scores.to(dev, dtype=torch.float32).reshape(-1, 1).contiguous(), 1, torch.float32, 'scores'))
+    if labels is not None:
+        parts.append((labels.to(dev, dtype=torch.int32).reshape(-1, 2).contiguous(), 2, torch.int32, 'labels'))
     n_sl, n_pts = int(parts[1][0].shape[0]), int(parts[0][0].shape[0])
     sizes = torch.tensor([n_sl, n_pts], dtype=torch.int64, device=dev)
     all_sizes = [torch.zeros_like(sizes) for _ in range(world)]
@@ -293,16 +299,20 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', s
             host.append(buf)
     if bufs and bufs[0].is_cuda:
         torch.cuda.current_stream(bufs[0].device).synchronize()
-    return _packed_tractogram([h.numpy().copy() if copy else h.numpy() for h in host])
+    return _packed_tractogram([h.numpy().copy() if copy else h.numpy() for h in host], [p[3] for p in parts])
 
 
-def _packed_tractogram(arrs):
-    """[points, lengths, seeds, flags(, scores)] host arrays in gather_packed's part order -> Tractogram."""
+def _packed_tractogram(arrs, names):
+    """[points, lengths, seeds, flags(, scores)(, labels)] host arrays in gather_packed's part order, with the
+    parts' names -> Tractogram."""
     data, lens, gseeds, gflags = arrs[:4]
     offsets = np.concatenate(([0], np.cumsum(lens[:, 0]))).astype(np.int64)
     per = {'seeds': gseeds, 'flags': gflags[:, 0]}
-    if len(arrs) > 4:
-        per['oracle_score'] = arrs[4][:, 0]
+    extra = dict(zip(names[4:], arrs[4:]))
+    if 'scores' in extra:
+        per['oracle_score'] = extra['scores'][:, 0]
+    if 'labels' in extra:
+        per['start_label'], per['end_label'] = extra['labels'][:, 0], extra['labels'][:, 1]
     return Tractogram(data=data, offsets=offsets, data_per_streamline=per)
 
 

@@ -55,6 +55,10 @@ class TrackToLearnTrack(object):
         self.save_oracle_scores = bool(track_dto.get('save_oracle_scores', False))
         self.out_density = track_dto.get('out_density')
         self.out_endpoints = track_dto.get('out_endpoints')
+        self.in_labels = track_dto.get('in_labels')
+        self.out_connectivity = track_dto.get('out_connectivity')
+        self.connectivity_radius = float(track_dto.get('connectivity_radius') or 0.0)
+        self.save_connectivity_labels = bool(track_dto.get('save_connectivity_labels', False))
         self.compute_reward = False
         if not torch.cuda.is_available():
             raise SystemExit('ttl_track (tracktolearn_b200) needs a CUDA device; there is no CPU path')
@@ -115,6 +119,16 @@ class TrackToLearnTrack(object):
             print("Subject has a voxel size of {}mm, setting step size to "
                   "{}mm.".format(tracking_voxel_size, step_size_mm))
         env = self.get_tracking_env(step_size_mm)
+        labels = None
+        if self.in_labels is not None:      # checked before tracking starts
+            from tracktolearn_b200.runners.ttl_connectivity import load_labels
+            from tracktolearn_b200.tracking.postprocess import radius_voxels
+            try:
+                labels, _ = load_labels(self.in_labels, (env._volume.X, env._volume.Y, env._volume.Z),
+                                        env.affine_vox2rasmm, self.device)
+                radius_voxels(self.connectivity_radius, env.affine_vox2rasmm)
+            except ValueError as e:
+                raise SystemExit(str(e))
         self.input_size = env.get_state_size()
         self.action_size = env.get_action_size()
         algs = {'SACAuto': SACAuto}
@@ -133,7 +147,10 @@ class TrackToLearnTrack(object):
             oracle = OracleSingleton(self.oracle_checkpoint, self.device, precision=self.oracle_precision)
         n = tracker.track_to_file(env, self.out_tractogram, ref_img.shape[:3], ref_img.zooms[:3], oracle=oracle,
                                   oracle_threshold=self.oracle_threshold, save_scores=self.save_oracle_scores,
-                                  density_path=self.out_density, endpoints_path=self.out_endpoints)
+                                  density_path=self.out_density, endpoints_path=self.out_endpoints,
+                                  labels=labels, connectivity_path=self.out_connectivity,
+                                  connectivity_radius=self.connectivity_radius,
+                                  save_labels=self.save_connectivity_labels)
         if int(os.environ.get('RANK', '0')) == 0:
             print('Wrote {} streamlines to {}.'.format(n, self.out_tractogram))
             for what, path in (('density', self.out_density), ('endpoint', self.out_endpoints)):
@@ -142,6 +159,9 @@ class TrackToLearnTrack(object):
             if tracker.maps_skipped:
                 print('{} points lie outside the volume\'s grid and are not counted in the maps.'.format(
                     tracker.maps_skipped))
+            if self.out_connectivity is not None:
+                print('Wrote the connectivity matrix to {}; {} streamline endpoints have no label.'.format(
+                    self.out_connectivity, tracker.connectome_unlabelled))
         return n
 
 
@@ -234,6 +254,19 @@ def add_track_args(parser):
                           help='Save each kept streamline\'s score as the per-streamline\nproperty '
                                '"oracle_score" (.trk only).')
     add_map_args(parser)
+    conn_g = parser.add_argument_group('Connectivity')
+    conn_g.add_argument('--in_labels', metavar='FILE', default=None,
+                        help='Label volume (.nii / .nii.gz) on the tracking volume\'s grid: integers in\n'
+                             '[0, 16383], 0 = no region.  Labels both ends of every streamline written.')
+    conn_g.add_argument('--out_connectivity', metavar='FILE', default=None,
+                        help='Connectivity matrix (.npy, int32 [K, K], K = max label + 1): the number\n'
+                             'of streamlines between each pair of labels, symmetric.')
+    conn_g.add_argument('--connectivity_radius', type=float, default=0.0, metavar='MM',
+                        help='An endpoint whose own voxel is unlabelled takes the label of the nearest\n'
+                             'labelled voxel within MM (at most 8 voxels). 0: its own voxel only. [%(default)s]')
+    conn_g.add_argument('--save_connectivity_labels', action='store_true',
+                        help='Save the labels of each streamline\'s ends as the per-streamline\n'
+                             'properties "start_label" and "end_label" (.trk only).')
 
 
 def add_map_args(p):
@@ -248,14 +281,18 @@ def add_map_args(p):
 
 
 def check_map_args(parser, args, other_outputs):
-    """--out_density / --out_endpoints: NIfTI names, not existing files without -f, distinct from each other
-    and from `other_outputs`."""
+    """--out_density / --out_endpoints (NIfTI names) and, where the parser has it, --out_connectivity (.npy):
+    not existing files without -f, distinct from each other and from `other_outputs`."""
     taken = [os.path.abspath(f) for f in other_outputs]
-    for opt, path in (('--out_density', args.out_density), ('--out_endpoints', args.out_endpoints)):
+    outs = [('--out_density', args.out_density, ('.nii', '.nii.gz')),
+            ('--out_endpoints', args.out_endpoints, ('.nii', '.nii.gz'))]
+    if hasattr(args, 'out_connectivity'):
+        outs.append(('--out_connectivity', args.out_connectivity, ('.npy',)))
+    for opt, path, exts in outs:
         if path is None:
             continue
-        if not path.endswith(('.nii', '.nii.gz')):
-            parser.error('{} must be a .nii or .nii.gz file, not {}'.format(opt, path))
+        if not path.endswith(exts):
+            parser.error('{} must be a {} file, not {}'.format(opt, ' or '.join(exts), path))
         if os.path.isfile(path) and not args.overwrite:
             parser.error('Output file {} exists. Use -f to force overwriting'.format(path))
         if os.path.abspath(path) in taken:
@@ -304,6 +341,16 @@ def parse_args(argv=None):
     if args.oracle_checkpoint and not os.path.isfile(args.oracle_checkpoint):
         parser.error('Oracle checkpoint {} does not exist'.format(args.oracle_checkpoint))
     check_map_args(parser, args, [args.out_tractogram])
+    if args.in_labels is not None and args.out_connectivity is None and not args.save_connectivity_labels:
+        parser.error('--in_labels needs --out_connectivity or --save_connectivity_labels')
+    if args.in_labels is None and (args.out_connectivity is not None or args.save_connectivity_labels):
+        parser.error('--out_connectivity and --save_connectivity_labels need --in_labels')
+    if args.in_labels is not None and not os.path.isfile(args.in_labels):
+        parser.error('Input file {} does not exist'.format(args.in_labels))
+    if not 0.0 <= args.connectivity_radius < float('inf'):
+        parser.error('--connectivity_radius must be a finite number of mm >= 0, not %r' % args.connectivity_radius)
+    if args.save_connectivity_labels and detect_format(args.out_tractogram) != 'trk':
+        parser.error('--save_connectivity_labels needs a .trk output: .tck files cannot hold per-streamline data')
     verify_agent_option(parser, args)
     return args
 

@@ -110,3 +110,61 @@ def tract_maps_packed(data, offsets, dims, density=None, endpoints=None):
                                       _lib.ptr(endpoints), _lib.ptr(skipped), _lib.stream_ptr(device)),
                    'ttl_tract_maps')
         return int(skipped.item())
+
+
+CONNECTOME_MAX_LABEL = 16383       # K <= TTL_CONNECTOME_MAX_LABELS (include/ttl_b200.h)
+CONNECTOME_MAX_RADIUS_VOX = 8.0    # TTL_CONNECTOME_MAX_RADIUS
+
+
+def radius_voxels(radius_mm, affine):
+    """A connectivity search radius in mm -> voxels of the grid of ``affine``, the voxel size taken as
+    ``track_to_file`` takes it (the mean of |diagonal| of the vox -> RAS mm affine).  Raises ValueError for a
+    negative or non-finite radius, or one of more than 8 voxels."""
+    radius_mm = float(radius_mm)
+    if not 0.0 <= radius_mm < float('inf'):
+        raise ValueError('the connectivity radius must be a finite number of mm >= 0, not %r' % radius_mm)
+    vox_size = float(np.mean(np.abs(np.asarray(affine, dtype=np.float64))[np.diag_indices(4)][:3]))
+    r = radius_mm / vox_size
+    if not r <= CONNECTOME_MAX_RADIUS_VOX:
+        raise ValueError('a connectivity radius of %g mm is %g voxels of %g mm: at most %g voxels are searched'
+                         % (radius_mm, r, vox_size, CONNECTOME_MAX_RADIUS_VOX))
+    return r
+
+
+def unlabelled_endpoints(matrix):
+    """The number of endpoints given label 0 in a connectivity matrix (numpy): one count in row 0 each, two
+    for a streamline with both ends at 0."""
+    m = np.asarray(matrix)
+    return 2 * int(m[0, 0]) + int(m[0, 1:].sum(dtype=np.int64))
+
+
+def connectome_packed(data, offsets, labels, matrix=None, radius_vox=0.0, pairs=False):
+    """Structural connectivity of packed voxel-space streamlines over ``labels``, an int32 CUDA volume
+    (X, Y, Z) on the points' device (``ttl_connectome``).  An endpoint's label is that of its own voxel
+    ``floor(p + 0.5)`` when labelled, else that of the nearest labelled voxel within ``radius_vox`` voxels
+    (ties to the smaller linear index), else 0.  A streamline with end labels (a, b) is added in place into
+    ``matrix`` (int32 CUDA [K, K], K = max label + 1): 1 at [a, a] when a == b, else 1 at [a, b] and at [b, a].
+    With ``pairs``, returns the int32 [n, 2] CUDA tensor of the labels of every streamline's first and last
+    points, else None.  ``matrix`` may be None when ``pairs`` is set (K is then ``labels.max() + 1``)."""
+    device = _dev(data.device)
+    lib = _lib.load()
+    data, offsets = _to_device(data, offsets, device)
+    if matrix is None and not pairs:
+        raise ValueError('connectome_packed needs a matrix, pairs or both')
+    if (not isinstance(labels, torch.Tensor) or labels.device != device or labels.dtype != torch.int32
+            or labels.dim() != 3 or not labels.is_contiguous()):
+        raise ValueError('labels must be a contiguous int32 tensor (X, Y, Z) on %s' % device)
+    if matrix is not None:
+        if (matrix.device != device or matrix.dtype != torch.int32 or matrix.dim() != 2
+                or matrix.shape[0] != matrix.shape[1] or not matrix.is_contiguous()):
+            raise ValueError('matrix must be a contiguous square int32 tensor on %s' % device)
+        K = int(matrix.shape[0])
+    else:
+        K = int(labels.max().item()) + 1 if labels.numel() else 1
+    n = max(int(offsets.shape[0]) - 1, 0)
+    out = torch.zeros((n, 2), dtype=torch.int32, device=device) if pairs else None
+    with torch.cuda.device(device):
+        _lib.check(lib.ttl_connectome(_lib.ptr(data), _lib.ptr(offsets), n, _lib.ptr(labels), *labels.shape, K,
+                                      float(radius_vox), _lib.ptr(matrix), _lib.ptr(out), _lib.stream_ptr(device)),
+                   'ttl_connectome')
+    return out

@@ -46,6 +46,7 @@ class Tracker(object):
         self.streaming = streaming
         self.rows_per_pass = rows_per_pass
         self.maps_skipped = 0       # points outside the grid in the maps of the last track_to_file
+        self.connectome_unlabelled = 0      # endpoints given label 0 in the matrix of the last track_to_file
 
     # ----------------------------------------------------------------------------------
     def _passes(self, env):
@@ -150,7 +151,8 @@ class Tracker(object):
         return d.cpu().numpy(), o.cpu().numpy()
 
     def track_to_file(self, env, path, dims, voxel_sizes, oracle=None, oracle_threshold=0.5, save_scores=False,
-                      density_path=None, endpoints_path=None):
+                      density_path=None, endpoints_path=None, labels=None, connectivity_path=None,
+                      connectivity_radius=0.0, save_labels=False):
         """What ``ttl_track.py`` does with ``track`` + ``nib.streamlines.save`` (runners/ttl_track.py:
         172-186), on packed arrays and on the device: dipy ``length`` and the min/max filter
         (tracker.py:118-121), ``compress_streamlines`` (:123-125), voxel -> file space (:127-136);
@@ -169,10 +171,19 @@ class Tracker(object):
         streamlines written, on the env's voxel grid (``postprocess.tract_maps_packed``), taken from their
         voxel-space points after the length and oracle filters and before ``--compress``; summed over the
         ranks onto rank 0, which writes them as int32 NIfTI with ``env.affine_vox2rasmm``.  The number of
-        points outside the grid is kept in ``self.maps_skipped``."""
+        points outside the grid is kept in ``self.maps_skipped``.
+
+        ``labels`` (an int32 volume of the env's grid on its device, ``ttl_connectivity.load_labels``): the
+        structural connectivity of the streamlines written (``postprocess.connectome_packed``), from the same
+        points as the maps, each endpoint labelled from its own voxel or the nearest labelled voxel within
+        ``connectivity_radius`` mm.  ``connectivity_path`` (.npy): the int32 matrix [K, K], K = max label + 1,
+        summed over the ranks onto rank 0, which writes it with ``np.save``; the number of endpoints given label
+        0 is kept in ``self.connectome_unlabelled``.  ``save_labels`` (.trk only) writes every streamline's end
+        labels as the per-streamline properties ``start_label`` and ``end_label``, after ``oracle_score``."""
         from tracktolearn_b200.io.streamlines import TckWriter, TrkWriter, detect_format
-        from tracktolearn_b200.tracking.postprocess import (compress_packed, lengths_packed, select_packed,
-                                                            tract_maps_packed)
+        from tracktolearn_b200.tracking.postprocess import (compress_packed, connectome_packed, lengths_packed,
+                                                            radius_voxels, select_packed, tract_maps_packed,
+                                                            unlabelled_endpoints)
         import torch.distributed as dist
         from tracktolearn_b200 import parallel
         fmt = detect_format(path)
@@ -180,6 +191,15 @@ class Tracker(object):
             raise ValueError('save_scores needs an oracle')
         if save_scores and fmt != 'trk':
             raise ValueError('.tck files cannot hold per-streamline data: save oracle scores to a .trk file')
+        grid = (env._volume.X, env._volume.Y, env._volume.Z)
+        if (connectivity_path is not None or save_labels) != (labels is not None):
+            raise ValueError('a connectivity output needs labels, and labels need a connectivity output')
+        if save_labels and fmt != 'trk':
+            raise ValueError('.tck files cannot hold per-streamline data: save connectivity labels to a .trk file')
+        if labels is not None:
+            if tuple(labels.shape) != grid or labels.dtype != torch.int32:
+                raise ValueError('labels must be an int32 volume of shape %r' % (grid,))
+            radius_vox = radius_voxels(connectivity_radius, env.affine_vox2rasmm)
         affine = np.asarray(env.affine_vox2rasmm, dtype=np.float64)
         np.random.shuffle(env.seeds)      # tracker.py:94
         # One process per GPU (torchrun): every rank shuffled the same seed list with the same RNG state;
@@ -197,7 +217,8 @@ class Tracker(object):
         lo, hi = self.min_length / vox_size, self.max_length / vox_size
         writer = None
         if rank == 0:
-            writer = (TrkWriter(path, dims, voxel_sizes, affine, self.save_seeds, save_scores=save_scores)
+            writer = (TrkWriter(path, dims, voxel_sizes, affine, self.save_seeds, save_scores=save_scores,
+                                save_labels=save_labels)
                       if fmt == 'trk' else TckWriter(path))
         self.alg.agent.eval()
         n_passes = len(list(self._passes(env)))
@@ -206,19 +227,23 @@ class Tracker(object):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             n_passes = int(t.item())
         passes = list(self._passes(env))
-        grid = (env._volume.X, env._volume.Y, env._volume.Z)
         density = endpoints = None
         if density_path is not None:
             density = torch.zeros(grid, dtype=torch.int32, device=env.device)
         if endpoints_path is not None:
             endpoints = torch.zeros(grid, dtype=torch.int32, device=env.device)
         skipped = 0
+        matrix = None
+        if connectivity_path is not None:
+            K = int(labels.max().item()) + 1
+            matrix = torch.zeros((K, K), dtype=torch.int32, device=env.device)
         try:
             for ip in range(n_passes):
                 out = torch.zeros((0, 3), dtype=torch.float32, device=env.device)
                 new_off = torch.zeros((1,), dtype=torch.int64, device=env.device)
                 seeds_kept = np.zeros((0, 3))
                 scores_kept = torch.zeros((0,), dtype=torch.float32, device=env.device)
+                pairs = torch.zeros((0, 2), dtype=torch.int32, device=env.device)
                 if ip < len(passes) and passes[ip][1] > passes[ip][0]:
                     self._run_pass(env, *passes[ip])
                     pts, offsets = env.get_streamlines_device()
@@ -230,6 +255,8 @@ class Tracker(object):
                         index, scores_kept = index[sel], scores[sel]
                     if density is not None or endpoints is not None:
                         skipped += tract_maps_packed(data, new_off, grid, density, endpoints)
+                    if labels is not None:
+                        pairs = connectome_packed(data, new_off, labels, matrix, radius_vox, pairs=save_labels)
                     if self.compress:     # after the length filter, before the space change (tracker.py:120-129)
                         data, new_off = compress_packed(data, new_off, tol_error=float(self.compress) / float(vox_size))
                     d64 = data.to(torch.float64)
@@ -245,10 +272,12 @@ class Tracker(object):
                     n_kept = int(new_off.shape[0]) - 1
                     merged = parallel.gather_packed(out, new_off[1:] - new_off[:-1], torch.as_tensor(seeds_kept),
                                                     torch.zeros((n_kept,), dtype=torch.int64), copy=False,
-                                                    scores=scores_kept if save_scores else None)
+                                                    scores=scores_kept if save_scores else None,
+                                                    labels=pairs if save_labels else None)
                     if rank == 0 and len(merged) > 0:
-                        writer.write(merged.data, merged.offsets, merged.data_per_streamline['seeds'],
-                                     merged.data_per_streamline.get('oracle_score'))
+                        per = merged.data_per_streamline
+                        writer.write(merged.data, merged.offsets, per['seeds'], per.get('oracle_score'),
+                                     np.stack((per['start_label'], per['end_label']), 1) if save_labels else None)
                     continue
                 if int(new_off.shape[0]) <= 1:
                     continue
@@ -258,17 +287,23 @@ class Tracker(object):
                 h_off.copy_(new_off, non_blocking=True)
                 torch.cuda.current_stream(env.device).synchronize()
                 writer.write(h_data.numpy().reshape(-1, 3), h_off.numpy(), seeds_kept,
-                             scores_kept.cpu().numpy() if save_scores else None)
+                             scores_kept.cpu().numpy() if save_scores else None,
+                             pairs.cpu().numpy() if save_labels else None)
         finally:
             if writer is not None:
                 writer.close()
-        if density is not None or endpoints is not None:
-            skipped = parallel.reduce_maps([density, endpoints], skipped)
+        self.connectome_unlabelled = 0
+        if density is not None or endpoints is not None or matrix is not None:
+            skipped = parallel.reduce_maps([density, endpoints, matrix], skipped)
             if rank == 0:
                 from tracktolearn_b200.io import nifti
                 for p, m in ((density_path, density), (endpoints_path, endpoints)):
                     if m is not None:
                         nifti.save(p, m.cpu().numpy(), env.affine_vox2rasmm)
+                if matrix is not None:
+                    m = matrix.cpu().numpy()
+                    np.save(connectivity_path, m)
+                    self.connectome_unlabelled = unlabelled_endpoints(m)
         self.maps_skipped = skipped
         n = writer.n if writer is not None else 0
         if world > 1:
