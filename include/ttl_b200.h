@@ -343,6 +343,35 @@ int ttl_tract_maps(const float* points, const int64_t* offsets, int32_t n, int32
 int ttl_connectome(const float* points, const int64_t* offsets, int32_t n, const int32_t* labels, int32_t nx,
                    int32_t ny, int32_t nz, int32_t K, double radius_vox, int32_t* matrix, int32_t* pairs,
                    void* stream);
+/* Tractometry: per-streamline means of C scalar maps.  volumes: float32 [nx][ny][nz][C] (C order, the C values
+ * of a voxel contiguous; 16-byte aligned for C = 4 / 8, 8-byte for C = 2).  A point p is sampled when
+ * ttl_tract_maps counts it (its voxel floor((double)p_k + 0.5) is in the grid, so p is finite).  Its value is
+ * the fp64 trilinear interpolation: per axis c = (double)p_k, i = floor(c), d = c - i, corners clamp(i, 0, n-1)
+ * and clamp(i+1, 0, n-1) with weights 1-d and d (scipy map_coordinates(order=1) inside [0, n-1], edge
+ * replication in the outer half-voxel rim); the value is the sum over the 8 corners, x then y then z lower
+ * before upper, of ((wx*wy)*wz)*v, every operation fp64 round-to-nearest without contraction.
+ * means [n][C] = (float)(fp64 sum of the sampled values / their number), NaN when no point is sampled (an empty
+ * streamline too).  Lane l of the streamline's warp sums points l, l+32, ... in order and a fixed xor-shuffle
+ * tree adds the 32 lanes, so a mean depends on the streamline's points alone, not on its batch or position.
+ * *skipped (device) += the number of points not sampled (ttl_tract_maps' count on the same input).
+ * TTL_ERR_BAD_ARG before any CUDA call for n < 0, C outside [1, TTL_SAMPLE_MAX_METRICS], a non-positive
+ * dimension, nx*ny*nz*C >= 2^31, no volumes, means or skipped, or no points / offsets with n > 0. */
+#define TTL_SAMPLE_MAX_METRICS 8
+int ttl_sample_metrics(const float* points, const int64_t* offsets, int32_t n, const float* volumes, int32_t C,
+                       int32_t nx, int32_t ny, int32_t nz, float* means, int64_t* skipped, void* stream);
+/* Metric-weighted connectivity: ADDS per-streamline values into caller-owned planes, exactly and in any order.
+ * pairs [n][2] int32 are ttl_connectome's end labels (a value outside [0, K) reads as 0); values [n][C] float32.
+ * A finite value v of column c with labels (a, b) adds q = __double2ll_rn(ldexp((double)v, shifts[c])) to
+ * sums[c][a][b] (int64) and 1 to counts[c][a][b] (int32), and the same at [b][a] when a != b; a NaN or +-inf
+ * value adds nothing.  With shifts[c] = clamp(31 - e, 0, 62) where every |v| < 2^e, |q| <= 2^31 and any 2^31
+ * streamlines sum within +-2^62.  The mean of a cell is (sums * 2^-shift) / counts.  shifts is HOST memory.
+ * TTL_ERR_BAD_ARG before any CUDA call for n < 0, C outside [1, TTL_CONNECTOME_SUMS_MAX_COLUMNS], K outside
+ * [1, TTL_CONNECTOME_MAX_LABELS], a shift outside [0, TTL_CONNECTOME_SUMS_MAX_SHIFT], no shifts, sums or
+ * counts, or no pairs / values with n > 0. */
+#define TTL_CONNECTOME_SUMS_MAX_COLUMNS (TTL_SAMPLE_MAX_METRICS + 1)   /* the metrics and the length */
+#define TTL_CONNECTOME_SUMS_MAX_SHIFT 62
+int ttl_connectome_sums(const int32_t* pairs, int32_t n, const float* values, int32_t C, int32_t K,
+                        const int32_t* shifts, int64_t* sums, int32_t* counts, void* stream);
 
 /* ---- SAC actor (algorithms/shared/offpolicy.py:61-140, shared/utils.py:41-51) -------------- */
 

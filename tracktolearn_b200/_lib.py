@@ -99,6 +99,8 @@ SIGNATURES = {
     'ttl_gather_streamlines': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_vp]),
     'ttl_tract_maps': (c_i32, [c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp]),
     'ttl_connectome': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_i32, c_i32, c_i32, c_f64, c_vp, c_vp, c_vp]),
+    'ttl_sample_metrics': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp]),
+    'ttl_connectome_sums': (c_i32, [c_vp, c_i32, c_vp, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp]),
     'ttl_pack_streamlines': (c_i32, [P(Batch), c_vp, c_vp, c_vp]),
     'ttl_actor_workspace_bytes': (c_i64, [P(ActorWeights), c_i32, c_i32]),
     'ttl_actor_plan_create': (c_i32, [P(c_vp), P(ActorWeights), c_i32, c_i32, c_vp, c_i64, c_vp]),

@@ -3,8 +3,8 @@
 // min/max length filter and dipy `compress_streamlines` for --compress -- on packed ragged arrays
 // [total][3] fp32 + int64 offsets [n+1], one warp per streamline -- and the ordered selection that
 // keeps the streamlines passing the length filter and, optionally, the TractOracle-Net score threshold --
-// the streamline density and endpoint maps of the streamlines kept -- and their connectivity matrix over a
-// label volume.
+// the streamline density and endpoint maps of the streamlines kept -- their connectivity matrix over a
+// label volume -- and their tractometry: per-streamline means of scalar maps and metric-weighted matrices.
 #include <math.h>
 
 #include <cub/device/device_scan.cuh>
@@ -313,6 +313,156 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) connectome_kernel(
   }
 }
 
+// Tractometry (DESIGN.md section 2, "Tractometry").  The C metrics of voxel v are vol[v*C .. v*C+C-1]: one
+// read-only vector load per corner where C allows it (float4 for C = 4 / 8, float2 for C = 2).
+template <int C>
+__device__ __forceinline__ void metric_corner(const float* __restrict__ vol, int v, float (&m)[C]) {
+  const float* p = vol + (long long)v * C;
+  if constexpr (C % 4 == 0) {
+#pragma unroll
+    for (int c = 0; c < C; c += 4) {
+      const float4 q = __ldg(reinterpret_cast<const float4*>(p + c));
+      m[c] = q.x; m[c + 1] = q.y; m[c + 2] = q.z; m[c + 3] = q.w;
+    }
+  } else if constexpr (C % 2 == 0) {
+#pragma unroll
+    for (int c = 0; c < C; c += 2) {
+      const float2 q = __ldg(reinterpret_cast<const float2*>(p + c));
+      m[c] = q.x; m[c + 1] = q.y;
+    }
+  } else {
+#pragma unroll
+    for (int c = 0; c < C; ++c) m[c] = __ldg(p + c);
+  }
+}
+
+// Lower corner index, upper corner index and upper weight of one axis: i = floor(c), d = c - i, corners
+// clamp(i, 0, n-1) and clamp(i+1, 0, n-1).  Only called for points map_voxel puts in the grid, so
+// -1 <= i <= n-1 and the casts are exact.
+__device__ __forceinline__ void metric_axis(float p, int n, int& i0, int& i1, double& d) {
+  const double c = (double)p;
+  const double f = floor(c);
+  d = __dsub_rn(c, f);
+  const int i = (int)f;
+  i0 = max(i, 0);
+  i1 = min(i + 1, n - 1);
+}
+
+// One warp per streamline.  Lane l takes points l, l+32, ... in order; a point that map_voxel puts in the
+// grid adds its trilinear value, sum over the 8 corners (x, y, z lower before upper, z fastest) of
+// ((wx * wy) * wz) * value, every operation fp64 round-to-nearest without contraction, to the lane's fp64
+// partial sum of each metric.  A fixed xor-shuffle tree then adds the 32 partial sums, so the order of the
+// sum depends on the point count alone.  means[i][c] = (float)(sum / count), NaN without a sampled point.
+// Out-of-grid points are summed per warp into *skipped.
+template <int C>
+__global__ void __launch_bounds__(kWarpsPerBlock * 32) sample_metrics_kernel(
+    const float* __restrict__ points, const long long* __restrict__ offsets, int n, const float* __restrict__ vol,
+    int nx, int ny, int nz, float* __restrict__ means, unsigned long long* __restrict__ skipped) {
+  const int lane = threadIdx.x & 31;
+  const int i = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
+  if (i >= n) return;
+  const long long beg = offsets[i];
+  const int N = (int)(offsets[i + 1] - beg);
+  const float* P = points + beg * 3;
+  double acc[C];
+#pragma unroll
+  for (int c = 0; c < C; ++c) acc[c] = 0.0;
+  int count = 0;
+  unsigned outside = 0;
+  for (int j = lane; j < N; j += 32) {
+    const float* p = P + 3 * j;
+    if (map_voxel(p, nx, ny, nz) < 0) {
+      ++outside;
+      continue;
+    }
+    int x0, x1, y0, y1, z0, z1;
+    double dx, dy, dz;
+    metric_axis(p[0], nx, x0, x1, dx);
+    metric_axis(p[1], ny, y0, y1, dy);
+    metric_axis(p[2], nz, z0, z1, dz);
+    const double wx[2] = {__dsub_rn(1.0, dx), dx}, wy[2] = {__dsub_rn(1.0, dy), dy}, wz[2] = {__dsub_rn(1.0, dz), dz};
+    const int xs[2] = {x0, x1}, ys[2] = {y0, y1}, zs[2] = {z0, z1};
+    double val[C];
+#pragma unroll
+    for (int c = 0; c < C; ++c) val[c] = 0.0;
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+#pragma unroll
+      for (int b = 0; b < 2; ++b) {
+        const double wxy = __dmul_rn(wx[a], wy[b]);
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const double w = __dmul_rn(wxy, wz[e]);
+          float m[C];
+          metric_corner<C>(vol, (xs[a] * ny + ys[b]) * nz + zs[e], m);
+#pragma unroll
+          for (int c = 0; c < C; ++c) val[c] = __dadd_rn(val[c], __dmul_rn(w, (double)m[c]));
+        }
+      }
+    }
+#pragma unroll
+    for (int c = 0; c < C; ++c) acc[c] = __dadd_rn(acc[c], val[c]);
+    ++count;
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+#pragma unroll
+    for (int c = 0; c < C; ++c) acc[c] = __dadd_rn(acc[c], __shfl_xor_sync(0xffffffffu, acc[c], off));
+    count += __shfl_xor_sync(0xffffffffu, count, off);
+    outside += __shfl_xor_sync(0xffffffffu, outside, off);
+  }
+  if (lane != 0) return;
+#pragma unroll
+  for (int c = 0; c < C; ++c)
+    means[(long long)i * C + c] = count > 0 ? __double2float_rn(__ddiv_rn(acc[c], (double)count)) : __int_as_float(0x7fc00000);
+  if (outside != 0) atomicAdd(skipped, (unsigned long long)outside);
+}
+
+// The fixed-point shift of every column, passed by value: the host checks them before the launch.
+struct SumShifts {
+  int s[TTL_CONNECTOME_SUMS_MAX_COLUMNS];
+};
+
+// One thread per (streamline, column): a finite value v with end labels (a, b) adds
+// q = __double2ll_rn(ldexp((double)v, shift)) to sums[c][a][b] and 1 to counts[c][a][b], and the same at [b][a]
+// when a != b.  Integer atomics: the planes do not depend on launch order.  A label outside [0, K) reads as 0.
+__global__ void __launch_bounds__(256) connectome_sums_kernel(
+    const int* __restrict__ pairs, int n, const float* __restrict__ values, int C, int K, const SumShifts shifts,
+    long long* __restrict__ sums, int* __restrict__ counts) {
+  const long long t = (long long)blockIdx.x * 256 + threadIdx.x;
+  if (t >= (long long)n * C) return;
+  const int i = (int)(t / C), c = (int)(t - (long long)i * C);
+  const float v = values[t];
+  if (!isfinite(v)) return;
+  int a = pairs[2 * (long long)i], b = pairs[2 * (long long)i + 1];
+  a = (a > 0 && a < K) ? a : 0;
+  b = (b > 0 && b < K) ? b : 0;
+  int shift = 0;      // selected with constant indices: a dynamic index would copy the array to the stack
+#pragma unroll
+  for (int k = 0; k < TTL_CONNECTOME_SUMS_MAX_COLUMNS; ++k) shift = k == c ? shifts.s[k] : shift;
+  const long long q = __double2ll_rn(ldexp((double)v, shift));
+  const long long base = (long long)c * K * K;
+  atomicAdd((unsigned long long*)(sums + base + (long long)a * K + b), (unsigned long long)q);
+  atomicAdd(counts + base + (long long)a * K + b, 1);
+  if (a != b) {
+    atomicAdd((unsigned long long*)(sums + base + (long long)b * K + a), (unsigned long long)q);
+    atomicAdd(counts + base + (long long)b * K + a, 1);
+  }
+}
+
+template <int C>
+void launch_sample_metrics(const float* points, const long long* offsets, int n, const float* vol, int nx, int ny,
+                           int nz, float* means, unsigned long long* skipped, cudaStream_t s) {
+  sample_metrics_kernel<C><<<ttl_div_up(n, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
+      points, offsets, n, vol, nx, ny, nz, means, skipped);
+}
+
+typedef void (*sample_metrics_launcher)(const float*, const long long*, int, const float*, int, int, int, float*,
+                                        unsigned long long*, cudaStream_t);
+const sample_metrics_launcher kSampleMetrics[TTL_SAMPLE_MAX_METRICS] = {
+    launch_sample_metrics<1>, launch_sample_metrics<2>, launch_sample_metrics<3>, launch_sample_metrics<4>,
+    launch_sample_metrics<5>, launch_sample_metrics<6>, launch_sample_metrics<7>, launch_sample_metrics<8>};
+
 size_t select_pairs_bytes(int n) { return ((size_t)n * sizeof(longlong2) + 255) / 256 * 256; }
 
 size_t select_scan_bytes(int n) {
@@ -432,6 +582,41 @@ int ttl_connectome(const float* points, const int64_t* offsets, int32_t n, const
   TTL_LAUNCH("connectome_kernel", s,
              connectome_kernel<<<ttl_div_up(n, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
                  points, (const long long*)offsets, n, labels, nx, ny, nz, K, radius_vox, matrix, pairs));
+  TTL_CHECK_LAST();
+  return 0;
+}
+
+int ttl_sample_metrics(const float* points, const int64_t* offsets, int32_t n, const float* volumes, int32_t C,
+                       int32_t nx, int32_t ny, int32_t nz, float* means, int64_t* skipped, void* stream) {
+  if (n < 0 || C < 1 || C > TTL_SAMPLE_MAX_METRICS || nx <= 0 || ny <= 0 || nz <= 0 ||
+      (int64_t)nx * ny * nz * C >= ((int64_t)1 << 31) || !volumes || !means || !skipped)
+    return TTL_ERR_BAD_ARG;
+  if (n == 0) return 0;
+  if (!points || !offsets) return TTL_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  TTL_LAUNCH("sample_metrics_kernel", s,
+             kSampleMetrics[C - 1](points, (const long long*)offsets, n, volumes, nx, ny, nz, means,
+                                   (unsigned long long*)skipped, s));
+  TTL_CHECK_LAST();
+  return 0;
+}
+
+int ttl_connectome_sums(const int32_t* pairs, int32_t n, const float* values, int32_t C, int32_t K,
+                        const int32_t* shifts, int64_t* sums, int32_t* counts, void* stream) {
+  if (n < 0 || C < 1 || C > TTL_CONNECTOME_SUMS_MAX_COLUMNS || K < 1 || K > TTL_CONNECTOME_MAX_LABELS || !shifts ||
+      !sums || !counts)
+    return TTL_ERR_BAD_ARG;
+  SumShifts sh;
+  for (int c = 0; c < C; ++c) {
+    if (shifts[c] < 0 || shifts[c] > TTL_CONNECTOME_SUMS_MAX_SHIFT) return TTL_ERR_BAD_ARG;
+    sh.s[c] = shifts[c];
+  }
+  if (n == 0) return 0;
+  if (!pairs || !values) return TTL_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  TTL_LAUNCH("connectome_sums_kernel", s,
+             connectome_sums_kernel<<<ttl_div_up((long long)n * C, 256), 256, 0, s>>>(
+                 pairs, n, values, C, K, sh, (long long*)sums, counts));
   TTL_CHECK_LAST();
   return 0;
 }

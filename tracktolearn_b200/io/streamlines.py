@@ -33,16 +33,28 @@ def _voxel_order(affine):
 class TrkWriter(object):
     """Streams (data, offsets) batches to a .trk file; the streamline count is patched on close.
     Per-streamline properties: ``seeds_x/y/z`` (``save_seeds``), then ``oracle_score`` (``save_scores``), then
-    ``start_label`` and ``end_label`` (``save_labels``: connectivity labels, integers held exactly in float32)."""
+    ``start_label`` and ``end_label`` (``save_labels``: connectivity labels, integers held exactly in float32), then
+    ``mean_NAME`` for every name of ``metric_names`` (per-streamline metric means).  The header has room for 10
+    properties: more raise ValueError."""
 
-    def __init__(self, path, dims, voxel_sizes, affine, save_seeds=False, save_scores=False, save_labels=False):
+    MAX_PROPERTIES = 10
+
+    def __init__(self, path, dims, voxel_sizes, affine, save_seeds=False, save_scores=False, save_labels=False,
+                 metric_names=()):
+        names = (((b'seeds_x', b'seeds_y', b'seeds_z') if save_seeds else ()) + ((b'oracle_score',) if save_scores else ())
+                 + ((b'start_label', b'end_label') if save_labels else ())
+                 + tuple(b'mean_' + str(m).encode() for m in metric_names))
+        if len(names) > self.MAX_PROPERTIES:
+            raise ValueError('a .trk file holds at most %d per-streamline properties, not %d'
+                             % (self.MAX_PROPERTIES, len(names)))
+        if any(len(name) > 19 for name in names):
+            raise ValueError('a .trk property name has at most 19 bytes: %r' % [n for n in names if len(n) > 19])
         self.f = open(path, 'wb')
         self.n = 0
         self.save_seeds = save_seeds
         self.save_scores = save_scores
         self.save_labels = save_labels
-        names = (((b'seeds_x', b'seeds_y', b'seeds_z') if save_seeds else ()) + ((b'oracle_score',) if save_scores else ())
-                 + ((b'start_label', b'end_label') if save_labels else ()))
+        self.n_metrics = len(metric_names)
         hdr = bytearray(1000)
         hdr[0:6] = b'TRACK\x00'
         struct.pack_into('<3h', hdr, 6, *[int(d) for d in dims])
@@ -60,12 +72,13 @@ class TrkWriter(object):
         struct.pack_into('<i', hdr, 996, 1000)                               # hdr_size
         self.f.write(bytes(hdr))
 
-    def write(self, data, offsets, seeds=None, scores=None, labels=None):
+    def write(self, data, offsets, seeds=None, scores=None, labels=None, means=None):
         n = len(offsets) - 1
         if n <= 0:
             return
         lens = np.diff(offsets).astype(np.int64)
-        n_prop = (3 if self.save_seeds else 0) + (1 if self.save_scores else 0) + (2 if self.save_labels else 0)
+        n_prop = ((3 if self.save_seeds else 0) + (1 if self.save_scores else 0) + (2 if self.save_labels else 0)
+                  + self.n_metrics)
         total = int(lens.sum()) * 3 + n * (1 + n_prop)
         out = np.empty(total, dtype='<f4')
         # positions of the int32 counts inside the float buffer
@@ -81,8 +94,12 @@ class TrkWriter(object):
             out[starts + lens * 3 + 1 + (3 if self.save_seeds else 0)] = np.asarray(scores, dtype=np.float32).reshape(-1)
         if self.save_labels:
             lab = np.asarray(labels).reshape(-1, 2).astype(np.float32)
-            out[starts + lens * 3 + n_prop - 1] = lab[:, 0]
-            out[starts + lens * 3 + n_prop] = lab[:, 1]
+            out[starts + lens * 3 + n_prop - 1 - self.n_metrics] = lab[:, 0]
+            out[starts + lens * 3 + n_prop - self.n_metrics] = lab[:, 1]
+        if self.n_metrics:
+            m = np.asarray(means, dtype=np.float32).reshape(n, self.n_metrics)
+            for c in range(self.n_metrics):
+                out[starts + lens * 3 + n_prop - self.n_metrics + 1 + c] = m[:, c]
         self.f.write(out.tobytes())
         self.n += n
 
@@ -108,9 +125,9 @@ class TckWriter(object):
         self.f.write(text.encode())
         self.offset = offset
 
-    def write(self, data, offsets, seeds=None, scores=None, labels=None):
-        """``seeds``, ``scores`` and ``labels`` are accepted for TrkWriter's signature: .tck has no per-streamline
-        data."""
+    def write(self, data, offsets, seeds=None, scores=None, labels=None, means=None):
+        """``seeds``, ``scores``, ``labels`` and ``means`` are accepted for TrkWriter's signature: .tck has no
+        per-streamline data."""
         n = len(offsets) - 1
         if n <= 0:
             return

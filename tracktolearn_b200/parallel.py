@@ -212,7 +212,8 @@ def _gather_via_arena(parts, dst, copy):
     return out
 
 
-def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', scores=None, labels=None):
+def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', scores=None, labels=None,
+                  means=None):
     """Gather packed streamlines on rank `dst` in rank order.
 
     ``via``: 'nccl' -- the data travels through NCCL to `dst`'s GPU and over its PCIe link (below);
@@ -229,8 +230,9 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', s
     memory, valid until the next gather.  ``scores`` [n] float32 (optional): per-streamline oracle scores,
     carried along and returned as ``data_per_streamline['oracle_score']``.  ``labels`` [n, 2] int32 (optional):
     the connectivity labels of every streamline's first and last points, returned as
-    ``data_per_streamline['start_label']`` and ``['end_label']``.  Returns a Tractogram on `dst`, None
-    elsewhere."""
+    ``data_per_streamline['start_label']`` and ``['end_label']``.  ``means`` [n, C] float32 (optional): the
+    per-streamline metric means, returned as ``data_per_streamline['metric_means']``.  Returns a Tractogram on
+    `dst`, None elsewhere."""
     world, rank = dist.get_world_size(), dist.get_rank()
     dev = _device_for_backend()
     if via == 'auto':
@@ -247,6 +249,8 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', s
             parts.append((scores.to(dtype=torch.float32).reshape(-1, 1), 1, torch.float32, 'scores'))
         if labels is not None:
             parts.append((labels.to(dtype=torch.int32).reshape(-1, 2), 2, torch.int32, 'labels'))
+        if means is not None:
+            parts.append((means.to(dtype=torch.float32), int(means.shape[1]), torch.float32, 'means'))
         arrs = _gather_via_arena(parts, dst, copy)
         if arrs is None:
             return None
@@ -261,6 +265,8 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', s
         parts.append((scores.to(dev, dtype=torch.float32).reshape(-1, 1).contiguous(), 1, torch.float32, 'scores'))
     if labels is not None:
         parts.append((labels.to(dev, dtype=torch.int32).reshape(-1, 2).contiguous(), 2, torch.int32, 'labels'))
+    if means is not None:
+        parts.append((means.to(dev, dtype=torch.float32).contiguous(), int(means.shape[1]), torch.float32, 'means'))
     n_sl, n_pts = int(parts[1][0].shape[0]), int(parts[0][0].shape[0])
     sizes = torch.tensor([n_sl, n_pts], dtype=torch.int64, device=dev)
     all_sizes = [torch.zeros_like(sizes) for _ in range(world)]
@@ -303,8 +309,8 @@ def gather_packed(points, lengths, seeds, flags, dst=0, copy=True, via='auto', s
 
 
 def _packed_tractogram(arrs, names):
-    """[points, lengths, seeds, flags(, scores)(, labels)] host arrays in gather_packed's part order, with the
-    parts' names -> Tractogram."""
+    """[points, lengths, seeds, flags(, scores)(, labels)(, means)] host arrays in gather_packed's part order,
+    with the parts' names -> Tractogram."""
     data, lens, gseeds, gflags = arrs[:4]
     offsets = np.concatenate(([0], np.cumsum(lens[:, 0]))).astype(np.int64)
     per = {'seeds': gseeds, 'flags': gflags[:, 0]}
@@ -313,13 +319,16 @@ def _packed_tractogram(arrs, names):
         per['oracle_score'] = extra['scores'][:, 0]
     if 'labels' in extra:
         per['start_label'], per['end_label'] = extra['labels'][:, 0], extra['labels'][:, 1]
+    if 'means' in extra:
+        per['metric_means'] = extra['means']
     return Tractogram(data=data, offsets=offsets, data_per_streamline=per)
 
 
 def reduce_maps(maps, skipped, dst=0):
-    """Sum per-rank streamline maps onto rank `dst`: one ``dist.reduce`` (SUM) per int32 map in ``maps`` (a
-    list; None entries are passed over), in place, and one for the ``skipped`` point count.  The maps are
-    integer counts, so the sum is exact and the same for every GPU count.  Tensors live on this rank's device
+    """Sum per-rank streamline maps onto rank `dst`: one ``dist.reduce`` (SUM) per int32 or int64 map in ``maps``
+    (a list; None entries are passed over), in place, and one for the ``skipped`` point count.  The maps are
+    integers -- counts, or the int64 fixed-point sums of metric-weighted matrices -- so the sum is exact and the
+    same for every GPU count.  Tensors live on this rank's device
     for the backend (CUDA under NCCL, CPU under gloo).  Returns the total skipped count on `dst`, this rank's
     count elsewhere; without torch.distributed, ``skipped`` unchanged."""
     if not dist.is_available() or not dist.is_initialized() or dist.get_world_size() == 1:

@@ -59,6 +59,10 @@ class TrackToLearnTrack(object):
         self.out_connectivity = track_dto.get('out_connectivity')
         self.connectivity_radius = float(track_dto.get('connectivity_radius') or 0.0)
         self.save_connectivity_labels = bool(track_dto.get('save_connectivity_labels', False))
+        self.in_metric = [tuple(m) for m in (track_dto.get('in_metric') or [])]
+        self.save_metric_means = bool(track_dto.get('save_metric_means', False))
+        self.out_connectivity_metrics = track_dto.get('out_connectivity_metrics')
+        self.out_connectivity_length = track_dto.get('out_connectivity_length')
         self.compute_reward = False
         if not torch.cuda.is_available():
             raise SystemExit('ttl_track (tracktolearn_b200) needs a CUDA device; there is no CPU path')
@@ -129,6 +133,14 @@ class TrackToLearnTrack(object):
                 radius_voxels(self.connectivity_radius, env.affine_vox2rasmm)
             except ValueError as e:
                 raise SystemExit(str(e))
+        metrics, metric_names = None, ()
+        if self.in_metric:                  # checked before tracking starts
+            from tracktolearn_b200.runners.ttl_connectivity import load_metrics
+            try:
+                metrics, metric_names, _ = load_metrics(self.in_metric, (env._volume.X, env._volume.Y, env._volume.Z),
+                                                        env.affine_vox2rasmm, self.device)
+            except ValueError as e:
+                raise SystemExit(str(e))
         self.input_size = env.get_state_size()
         self.action_size = env.get_action_size()
         algs = {'SACAuto': SACAuto}
@@ -150,7 +162,10 @@ class TrackToLearnTrack(object):
                                   density_path=self.out_density, endpoints_path=self.out_endpoints,
                                   labels=labels, connectivity_path=self.out_connectivity,
                                   connectivity_radius=self.connectivity_radius,
-                                  save_labels=self.save_connectivity_labels)
+                                  save_labels=self.save_connectivity_labels, metrics=metrics,
+                                  metric_names=metric_names, save_metric_means=self.save_metric_means,
+                                  metric_connectivity_prefix=self.out_connectivity_metrics,
+                                  length_connectivity_path=self.out_connectivity_length)
         if int(os.environ.get('RANK', '0')) == 0:
             print('Wrote {} streamlines to {}.'.format(n, self.out_tractogram))
             for what, path in (('density', self.out_density), ('endpoint', self.out_endpoints)):
@@ -162,6 +177,15 @@ class TrackToLearnTrack(object):
             if self.out_connectivity is not None:
                 print('Wrote the connectivity matrix to {}; {} streamline endpoints have no label.'.format(
                     self.out_connectivity, tracker.connectome_unlabelled))
+            from tracktolearn_b200.runners.ttl_connectivity import metric_outputs
+            for path in metric_outputs(self.out_connectivity_metrics, metric_names):
+                print('Wrote the mean {} connectivity matrix to {}.'.format(path[len(self.out_connectivity_metrics):-4],
+                                                                           path))
+            if self.out_connectivity_length is not None:
+                print('Wrote the mean length connectivity matrix to {}.'.format(self.out_connectivity_length))
+            if tracker.metrics_unsampled:
+                print('{} streamlines have no point inside the grid: their metric means are NaN.'.format(
+                    tracker.metrics_unsampled))
         return n
 
 
@@ -267,6 +291,19 @@ def add_track_args(parser):
     conn_g.add_argument('--save_connectivity_labels', action='store_true',
                         help='Save the labels of each streamline\'s ends as the per-streamline\n'
                              'properties "start_label" and "end_label" (.trk only).')
+    from tracktolearn_b200.runners.ttl_connectivity import add_metric_arg
+    tm_g = parser.add_argument_group('Tractometry')
+    add_metric_arg(tm_g)
+    tm_g.add_argument('--save_metric_means', action='store_true',
+                      help='Save each streamline\'s mean of every --in_metric over its points as the\n'
+                           'per-streamline property "mean_NAME" (.trk only; at most 10 properties in all).')
+    tm_g.add_argument('--out_connectivity_metrics', metavar='PREFIX', default=None,
+                      help='Write the mean of each --in_metric over the streamlines of every edge of\n'
+                           'the connectivity matrix to PREFIX + NAME + ".npy" (float64 [K, K], NaN where\n'
+                           'no streamline).  Needs --in_labels.')
+    tm_g.add_argument('--out_connectivity_length', metavar='FILE', default=None,
+                      help='Mean length in mm of the streamlines of every edge (.npy, float64 [K, K]).\n'
+                           'Needs --in_labels.')
 
 
 def add_map_args(p):
@@ -281,13 +318,20 @@ def add_map_args(p):
 
 
 def check_map_args(parser, args, other_outputs):
-    """--out_density / --out_endpoints (NIfTI names) and, where the parser has it, --out_connectivity (.npy):
-    not existing files without -f, distinct from each other and from `other_outputs`."""
+    """--out_density / --out_endpoints (NIfTI names) and, where the parser has them, --out_connectivity,
+    --out_connectivity_length and the files of --out_connectivity_metrics (.npy): not existing files without -f,
+    distinct from each other and from `other_outputs`."""
     taken = [os.path.abspath(f) for f in other_outputs]
     outs = [('--out_density', args.out_density, ('.nii', '.nii.gz')),
             ('--out_endpoints', args.out_endpoints, ('.nii', '.nii.gz'))]
     if hasattr(args, 'out_connectivity'):
         outs.append(('--out_connectivity', args.out_connectivity, ('.npy',)))
+    if hasattr(args, 'out_connectivity_metrics'):
+        from tracktolearn_b200.runners.ttl_connectivity import metric_outputs
+        names = [n for n, _ in args.in_metric or []]
+        outs += [('--out_connectivity_metrics', f, ('.npy',))
+                 for f in metric_outputs(args.out_connectivity_metrics, names)]
+        outs.append(('--out_connectivity_length', args.out_connectivity_length, ('.npy',)))
     for opt, path, exts in outs:
         if path is None:
             continue
@@ -298,6 +342,36 @@ def check_map_args(parser, args, other_outputs):
         if os.path.abspath(path) in taken:
             parser.error('{} {} is also another output'.format(opt, path))
         taken.append(os.path.abspath(path))
+
+
+def check_metric_args(parser, args):
+    """The Tractometry options: names and files of --in_metric, what each output needs, and the number of .trk
+    properties.  The volumes themselves are checked before tracking starts."""
+    from tracktolearn_b200.io.streamlines import TrkWriter
+    from tracktolearn_b200.runners.ttl_connectivity import check_metric_names
+    metrics = args.in_metric or []
+    metric_outputs = args.save_metric_means or args.out_connectivity_metrics is not None
+    if metrics and not metric_outputs:
+        parser.error('--in_metric needs --save_metric_means or --out_connectivity_metrics')
+    if metric_outputs and not metrics:
+        parser.error('--save_metric_means and --out_connectivity_metrics need --in_metric')
+    if metrics:
+        try:
+            check_metric_names([n for n, _ in metrics])
+        except ValueError as e:
+            parser.error('--in_metric: {}'.format(e))
+    for _, path in metrics:
+        if not os.path.isfile(path):
+            parser.error('Input file {} does not exist'.format(path))
+    if args.save_metric_means:
+        if detect_format(args.out_tractogram) != 'trk':
+            parser.error('--save_metric_means needs a .trk output: .tck files cannot hold per-streamline data')
+        n_prop = (3 * bool(args.save_seeds) + bool(args.save_oracle_scores) + 2 * bool(args.save_connectivity_labels)
+                  + len(metrics))
+        if n_prop > TrkWriter.MAX_PROPERTIES:
+            parser.error('{} per-streamline properties requested (--save_seeds 3, --save_oracle_scores 1, '
+                         '--save_connectivity_labels 2, --save_metric_means 1 per metric): a .trk file holds at '
+                         'most {}'.format(n_prop, TrkWriter.MAX_PROPERTIES))
 
 
 def verify_agent_option(parser, args):
@@ -340,11 +414,16 @@ def parse_args(argv=None):
         parser.error('--save_oracle_scores needs a .trk output: .tck files cannot hold per-streamline data')
     if args.oracle_checkpoint and not os.path.isfile(args.oracle_checkpoint):
         parser.error('Oracle checkpoint {} does not exist'.format(args.oracle_checkpoint))
+    check_metric_args(parser, args)
     check_map_args(parser, args, [args.out_tractogram])
-    if args.in_labels is not None and args.out_connectivity is None and not args.save_connectivity_labels:
-        parser.error('--in_labels needs --out_connectivity or --save_connectivity_labels')
-    if args.in_labels is None and (args.out_connectivity is not None or args.save_connectivity_labels):
-        parser.error('--out_connectivity and --save_connectivity_labels need --in_labels')
+    conn_outputs = (args.out_connectivity is not None or args.save_connectivity_labels
+                    or args.out_connectivity_metrics is not None or args.out_connectivity_length is not None)
+    if args.in_labels is not None and not conn_outputs:
+        parser.error('--in_labels needs --out_connectivity, --save_connectivity_labels, --out_connectivity_metrics '
+                     'or --out_connectivity_length')
+    if args.in_labels is None and conn_outputs:
+        parser.error('--out_connectivity, --save_connectivity_labels, --out_connectivity_metrics and '
+                     '--out_connectivity_length need --in_labels')
     if args.in_labels is not None and not os.path.isfile(args.in_labels):
         parser.error('Input file {} does not exist'.format(args.in_labels))
     if not 0.0 <= args.connectivity_radius < float('inf'):

@@ -2,6 +2,8 @@
 tracking/tracker.py:118-125): dipy ``length`` for the min/max length filter and dipy
 ``compress_streamlines`` for ``--compress``.  Packed layout: ``data`` [total, 3] float32 and
 ``offsets`` [n + 1] int64 (streamline i = data[offsets[i]:offsets[i+1]])."""
+import math
+
 import numpy as np
 import torch
 
@@ -167,4 +169,89 @@ def connectome_packed(data, offsets, labels, matrix=None, radius_vox=0.0, pairs=
         _lib.check(lib.ttl_connectome(_lib.ptr(data), _lib.ptr(offsets), n, _lib.ptr(labels), *labels.shape, K,
                                       float(radius_vox), _lib.ptr(matrix), _lib.ptr(out), _lib.stream_ptr(device)),
                    'ttl_connectome')
+    return out
+
+
+SAMPLE_MAX_METRICS = 8             # TTL_SAMPLE_MAX_METRICS (include/ttl_b200.h)
+SUMS_MAX_SHIFT = 62                # TTL_CONNECTOME_SUMS_MAX_SHIFT
+
+
+def sample_metrics_packed(data, offsets, volumes):
+    """Per-streamline means of scalar maps along packed voxel-space streamlines (``ttl_sample_metrics``).
+    ``volumes``: a contiguous float32 CUDA tensor (X, Y, Z, C), C in [1, 8], on the points' device.  A point is
+    sampled when ``tract_maps_packed`` counts it (its voxel ``floor(p + 0.5)`` is in the grid); its value is the
+    fp64 trilinear interpolation with the corner indices clamped to the grid (scipy ``map_coordinates(order=1)``
+    inside [0, n-1]).  Returns (means, skipped): float32 CUDA [n, C], the fp64 mean of the sampled values rounded
+    once to float32 (NaN when no point is sampled), and the number of points not sampled (one small
+    device-to-host copy).  A streamline's means do not depend on its batch or its position in it."""
+    device = _dev(data.device)
+    lib = _lib.load()
+    data, offsets = _to_device(data, offsets, device)
+    if (not isinstance(volumes, torch.Tensor) or volumes.device != device or volumes.dtype != torch.float32
+            or volumes.dim() != 4 or not volumes.is_contiguous()
+            or not 1 <= int(volumes.shape[3]) <= SAMPLE_MAX_METRICS):
+        raise ValueError('volumes must be a contiguous float32 tensor (X, Y, Z, C), C in [1, %d], on %s'
+                         % (SAMPLE_MAX_METRICS, device))
+    n = max(int(offsets.shape[0]) - 1, 0)
+    C = int(volumes.shape[3])
+    means = torch.empty((n, C), dtype=torch.float32, device=device)
+    skipped = torch.zeros((1,), dtype=torch.int64, device=device)
+    with torch.cuda.device(device):
+        _lib.check(lib.ttl_sample_metrics(_lib.ptr(data), _lib.ptr(offsets), n, _lib.ptr(volumes), C,
+                                          *volumes.shape[:3], _lib.ptr(means), _lib.ptr(skipped),
+                                          _lib.stream_ptr(device)), 'ttl_sample_metrics')
+        return means, int(skipped.item())
+
+
+def metric_shift(bound):
+    """The fixed-point shift S of edge sums for values with |v| <= ``bound``: S = clamp(31 - e, 0, 62) where
+    bound < 2^e, so that every |round(v * 2^S)| <= 2^31 and any 2^31 streamlines sum within +-2^62 in int64.
+    Raises ValueError for a negative or non-finite bound, or one >= 2^31."""
+    bound = float(bound)
+    if not 0.0 <= bound < 2.0 ** 31:
+        raise ValueError('edge values bounded by %r cannot be summed exactly in int64: the largest |value| must be '
+                         'finite and below 2^31' % bound)
+    return min(max(31 - math.frexp(bound)[1], 0), SUMS_MAX_SHIFT)
+
+
+def connectome_sums_packed(pairs, values, shifts, sums, counts):
+    """Metric-weighted connectivity (``ttl_connectome_sums``), added in place.  ``pairs``: int32 CUDA [n, 2], the
+    end labels of ``connectome_packed(pairs=True)``; ``values``: float32 CUDA [n, C]; ``shifts``: C ints
+    (``metric_shift``).  A finite value v of column c adds round(v * 2^shifts[c]) to ``sums[c, a, b]`` (int64 CUDA
+    [C, K, K]) and 1 to ``counts[c, a, b]`` (int32 CUDA [C, K, K]), and the same at [b, a] when a != b; NaN adds
+    nothing.  The planes are exact integer sums: they do not depend on the order of streamlines or calls."""
+    device = _dev(values.device if isinstance(values, torch.Tensor) else None)
+    lib = _lib.load()
+    if (not isinstance(values, torch.Tensor) or values.device != device or values.dtype != torch.float32 or values.dim() != 2
+            or not values.is_contiguous()):
+        raise ValueError('values must be a contiguous float32 tensor [n, C] on %s' % device)
+    n, C = (int(s) for s in values.shape)
+    if (not isinstance(pairs, torch.Tensor) or pairs.device != device or pairs.dtype != torch.int32
+            or tuple(pairs.shape) != (n, 2) or not pairs.is_contiguous()):
+        raise ValueError('pairs must be a contiguous int32 tensor [%d, 2] on %s' % (n, device))
+    for name, t, dtype in (('sums', sums, torch.int64), ('counts', counts, torch.int32)):
+        if (not isinstance(t, torch.Tensor) or t.device != device or t.dtype != dtype or t.dim() != 3
+                or t.shape[0] != C or t.shape[1] != t.shape[2] or not t.is_contiguous()):
+            raise ValueError('%s must be a contiguous %s tensor [%d, K, K] on %s' % (name, dtype, C, device))
+    if sums.shape != counts.shape:
+        raise ValueError('sums and counts must have the same shape')
+    sh = np.ascontiguousarray(np.asarray(shifts, dtype=np.int64).reshape(-1))
+    if sh.shape != (C,) or sh.min(initial=0) < 0 or sh.max(initial=0) > SUMS_MAX_SHIFT:
+        raise ValueError('shifts must be %d integers in [0, %d]' % (C, SUMS_MAX_SHIFT))
+    sh = sh.astype(np.int32)
+    with torch.cuda.device(device):
+        _lib.check(lib.ttl_connectome_sums(_lib.ptr(pairs), n, _lib.ptr(values), C, int(sums.shape[1]),
+                                           sh.ctypes.data, _lib.ptr(sums), _lib.ptr(counts),
+                                           _lib.stream_ptr(device)), 'ttl_connectome_sums')
+
+
+def edge_means(sums, counts, shifts):
+    """The mean value of every edge from ``connectome_sums_packed``'s planes: float64 numpy [C, K, K],
+    (sums * 2^-shift) / counts, NaN where the count is 0."""
+    s = np.asarray(sums.cpu() if isinstance(sums, torch.Tensor) else sums, dtype=np.int64)
+    c = np.asarray(counts.cpu() if isinstance(counts, torch.Tensor) else counts, dtype=np.int64)
+    sh = np.asarray(shifts, dtype=np.int32).reshape(-1, 1, 1)
+    with np.errstate(invalid='ignore', divide='ignore'):
+        out = np.ldexp(s.astype(np.float64), -sh) / c
+    out[c == 0] = np.nan
     return out

@@ -47,6 +47,7 @@ class Tracker(object):
         self.rows_per_pass = rows_per_pass
         self.maps_skipped = 0       # points outside the grid in the maps of the last track_to_file
         self.connectome_unlabelled = 0      # endpoints given label 0 in the matrix of the last track_to_file
+        self.metrics_unsampled = 0          # streamlines with no sampled point in the last track_to_file
 
     # ----------------------------------------------------------------------------------
     def _passes(self, env):
@@ -152,7 +153,8 @@ class Tracker(object):
 
     def track_to_file(self, env, path, dims, voxel_sizes, oracle=None, oracle_threshold=0.5, save_scores=False,
                       density_path=None, endpoints_path=None, labels=None, connectivity_path=None,
-                      connectivity_radius=0.0, save_labels=False):
+                      connectivity_radius=0.0, save_labels=False, metrics=None, metric_names=(),
+                      save_metric_means=False, metric_connectivity_prefix=None, length_connectivity_path=None):
         """What ``ttl_track.py`` does with ``track`` + ``nib.streamlines.save`` (runners/ttl_track.py:
         172-186), on packed arrays and on the device: dipy ``length`` and the min/max filter
         (tracker.py:118-121), ``compress_streamlines`` (:123-125), voxel -> file space (:127-136);
@@ -179,10 +181,22 @@ class Tracker(object):
         ``connectivity_radius`` mm.  ``connectivity_path`` (.npy): the int32 matrix [K, K], K = max label + 1,
         summed over the ranks onto rank 0, which writes it with ``np.save``; the number of endpoints given label
         0 is kept in ``self.connectome_unlabelled``.  ``save_labels`` (.trk only) writes every streamline's end
-        labels as the per-streamline properties ``start_label`` and ``end_label``, after ``oracle_score``."""
+        labels as the per-streamline properties ``start_label`` and ``end_label``, after ``oracle_score``.
+
+        ``metrics`` (a float32 volume (X, Y, Z, C) of the env's grid on its device, ``ttl_connectivity.load_metrics``)
+        with ``metric_names`` (C names): tractometry of the streamlines written, from the same points as the maps
+        (``postprocess.sample_metrics_packed``): every streamline's mean of each metric over its sampled points.
+        ``save_metric_means`` (.trk only) writes them as the per-streamline properties ``mean_NAME``, after the
+        labels.  With ``labels``, ``metric_connectivity_prefix`` writes PREFIX + NAME + '.npy' per metric and
+        ``length_connectivity_path`` one .npy: the mean metric / mean length in mm of the streamlines of every edge,
+        float64 [K, K], NaN where the count matrix is 0.  They are summed exactly (``postprocess.metric_shift``,
+        ``connectome_sums_packed``) over the ranks onto rank 0, so they do not depend on batch order, passes,
+        ``n_actor`` or GPU count.  The number of streamlines with no sampled point is kept in
+        ``self.metrics_unsampled``."""
         from tracktolearn_b200.io.streamlines import TckWriter, TrkWriter, detect_format
-        from tracktolearn_b200.tracking.postprocess import (compress_packed, connectome_packed, lengths_packed,
-                                                            radius_voxels, select_packed, tract_maps_packed,
+        from tracktolearn_b200.tracking.postprocess import (compress_packed, connectome_packed, connectome_sums_packed,
+                                                            edge_means, lengths_packed, metric_shift, radius_voxels,
+                                                            sample_metrics_packed, select_packed, tract_maps_packed,
                                                             unlabelled_endpoints)
         import torch.distributed as dist
         from tracktolearn_b200 import parallel
@@ -192,7 +206,8 @@ class Tracker(object):
         if save_scores and fmt != 'trk':
             raise ValueError('.tck files cannot hold per-streamline data: save oracle scores to a .trk file')
         grid = (env._volume.X, env._volume.Y, env._volume.Z)
-        if (connectivity_path is not None or save_labels) != (labels is not None):
+        weighted = metric_connectivity_prefix is not None or length_connectivity_path is not None
+        if (connectivity_path is not None or save_labels or weighted) != (labels is not None):
             raise ValueError('a connectivity output needs labels, and labels need a connectivity output')
         if save_labels and fmt != 'trk':
             raise ValueError('.tck files cannot hold per-streamline data: save connectivity labels to a .trk file')
@@ -200,6 +215,20 @@ class Tracker(object):
             if tuple(labels.shape) != grid or labels.dtype != torch.int32:
                 raise ValueError('labels must be an int32 volume of shape %r' % (grid,))
             radius_vox = radius_voxels(connectivity_radius, env.affine_vox2rasmm)
+        if (save_metric_means or metric_connectivity_prefix is not None) != (metrics is not None):
+            raise ValueError('a metric output needs metrics, and metrics need a metric output')
+        if save_metric_means and fmt != 'trk':
+            raise ValueError('.tck files cannot hold per-streamline data: save metric means to a .trk file')
+        shifts = []
+        if metrics is not None:
+            metric_names = [str(m) for m in metric_names]
+            if (metrics.dim() != 4 or tuple(metrics.shape[:3]) != grid or metrics.dtype != torch.float32
+                    or int(metrics.shape[3]) != len(metric_names)):
+                raise ValueError('metrics must be a float32 volume of shape %r + (%d,)' % (grid, len(metric_names)))
+            if metric_connectivity_prefix is not None:
+                shifts += [metric_shift(b) for b in metrics.abs().amax(dim=(0, 1, 2)).cpu().tolist()]
+        if length_connectivity_path is not None:      # kept lengths are <= max_length, up to float32 rounding
+            shifts.append(metric_shift(float(self.max_length) * 1.001))
         affine = np.asarray(env.affine_vox2rasmm, dtype=np.float64)
         np.random.shuffle(env.seeds)      # tracker.py:94
         # One process per GPU (torchrun): every rank shuffled the same seed list with the same RNG state;
@@ -218,7 +247,7 @@ class Tracker(object):
         writer = None
         if rank == 0:
             writer = (TrkWriter(path, dims, voxel_sizes, affine, self.save_seeds, save_scores=save_scores,
-                                save_labels=save_labels)
+                                save_labels=save_labels, metric_names=metric_names if save_metric_means else ())
                       if fmt == 'trk' else TckWriter(path))
         self.alg.agent.eval()
         n_passes = len(list(self._passes(env)))
@@ -234,9 +263,16 @@ class Tracker(object):
             endpoints = torch.zeros(grid, dtype=torch.int32, device=env.device)
         skipped = 0
         matrix = None
-        if connectivity_path is not None:
+        if connectivity_path is not None or weighted:
             K = int(labels.max().item()) + 1
+        if connectivity_path is not None:
             matrix = torch.zeros((K, K), dtype=torch.int32, device=env.device)
+        sums = counts = unsampled = None
+        if weighted:
+            sums = torch.zeros((len(shifts), K, K), dtype=torch.int64, device=env.device)
+            counts = torch.zeros((len(shifts), K, K), dtype=torch.int32, device=env.device)
+        if metrics is not None:
+            unsampled = torch.zeros((1,), dtype=torch.int64, device=env.device)
         try:
             for ip in range(n_passes):
                 out = torch.zeros((0, 3), dtype=torch.float32, device=env.device)
@@ -244,6 +280,7 @@ class Tracker(object):
                 seeds_kept = np.zeros((0, 3))
                 scores_kept = torch.zeros((0,), dtype=torch.float32, device=env.device)
                 pairs = torch.zeros((0, 2), dtype=torch.int32, device=env.device)
+                means = torch.zeros((0, len(metric_names)), dtype=torch.float32, device=env.device)
                 if ip < len(passes) and passes[ip][1] > passes[ip][0]:
                     self._run_pass(env, *passes[ip])
                     pts, offsets = env.get_streamlines_device()
@@ -256,7 +293,16 @@ class Tracker(object):
                     if density is not None or endpoints is not None:
                         skipped += tract_maps_packed(data, new_off, grid, density, endpoints)
                     if labels is not None:
-                        pairs = connectome_packed(data, new_off, labels, matrix, radius_vox, pairs=save_labels)
+                        pairs = connectome_packed(data, new_off, labels, matrix, radius_vox,
+                                                  pairs=save_labels or weighted)
+                    if metrics is not None:
+                        means, _ = sample_metrics_packed(data, new_off, metrics)
+                        unsampled += torch.isnan(means[:, 0]).sum()
+                    if weighted:
+                        cols = [means] if metric_connectivity_prefix is not None else []
+                        if length_connectivity_path is not None:
+                            cols.append((lens[index] * float(vox_size)).to(torch.float32).reshape(-1, 1))
+                        connectome_sums_packed(pairs, torch.cat(cols, 1).contiguous(), shifts, sums, counts)
                     if self.compress:     # after the length filter, before the space change (tracker.py:120-129)
                         data, new_off = compress_packed(data, new_off, tol_error=float(self.compress) / float(vox_size))
                     d64 = data.to(torch.float64)
@@ -273,11 +319,13 @@ class Tracker(object):
                     merged = parallel.gather_packed(out, new_off[1:] - new_off[:-1], torch.as_tensor(seeds_kept),
                                                     torch.zeros((n_kept,), dtype=torch.int64), copy=False,
                                                     scores=scores_kept if save_scores else None,
-                                                    labels=pairs if save_labels else None)
+                                                    labels=pairs if save_labels else None,
+                                                    means=means if save_metric_means else None)
                     if rank == 0 and len(merged) > 0:
                         per = merged.data_per_streamline
                         writer.write(merged.data, merged.offsets, per['seeds'], per.get('oracle_score'),
-                                     np.stack((per['start_label'], per['end_label']), 1) if save_labels else None)
+                                     np.stack((per['start_label'], per['end_label']), 1) if save_labels else None,
+                                     per.get('metric_means'))
                     continue
                 if int(new_off.shape[0]) <= 1:
                     continue
@@ -288,13 +336,14 @@ class Tracker(object):
                 torch.cuda.current_stream(env.device).synchronize()
                 writer.write(h_data.numpy().reshape(-1, 3), h_off.numpy(), seeds_kept,
                              scores_kept.cpu().numpy() if save_scores else None,
-                             pairs.cpu().numpy() if save_labels else None)
+                             pairs.cpu().numpy() if save_labels else None,
+                             means.cpu().numpy() if save_metric_means else None)
         finally:
             if writer is not None:
                 writer.close()
-        self.connectome_unlabelled = 0
-        if density is not None or endpoints is not None or matrix is not None:
-            skipped = parallel.reduce_maps([density, endpoints, matrix], skipped)
+        self.connectome_unlabelled = self.metrics_unsampled = 0
+        if any(m is not None for m in (density, endpoints, matrix, sums, unsampled)):
+            skipped = parallel.reduce_maps([density, endpoints, matrix, sums, counts, unsampled], skipped)
             if rank == 0:
                 from tracktolearn_b200.io import nifti
                 for p, m in ((density_path, density), (endpoints_path, endpoints)):
@@ -304,6 +353,15 @@ class Tracker(object):
                     m = matrix.cpu().numpy()
                     np.save(connectivity_path, m)
                     self.connectome_unlabelled = unlabelled_endpoints(m)
+                if sums is not None:
+                    mean = edge_means(sums, counts, shifts)
+                    if metric_connectivity_prefix is not None:
+                        for c, name in enumerate(metric_names):
+                            np.save(metric_connectivity_prefix + name + '.npy', mean[c])
+                    if length_connectivity_path is not None:
+                        np.save(length_connectivity_path, mean[-1])
+                if unsampled is not None:
+                    self.metrics_unsampled = int(unsampled.item())
         self.maps_skipped = skipped
         n = writer.n if writer is not None else 0
         if world > 1:
